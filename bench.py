@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the path-join + permutation-scoring hot path (BASELINE.json metric: path-pair*perm scores / s).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (config.workload): BASELINE config 3 - synthetic cohort of 10,000 patients (5,000 cases), 15,000 genes, path
@@ -17,6 +17,10 @@ in the checkout; sizes generated are reported in `config`).  One step = the whol
              for the dense kernel; the SURVEY 8d algorithmic bytes / word-ops are kept as `algorithmic` (speed-ups, not fractions)
   cpu_baseline  the reference's own join (oracle/_ref, built from the unmodified reference sources with
              g++ -O3 -march=<host level> -mpopcnt) on all host cores over a bounded sample of the same level-4 join
+
+--steps K sets the timed steps of every timed leg (resident, e2e, strong).  --dump-outputs DIR writes what the last timed
+resident step returned to its caller (see dump_outputs); the inputs depend only on the workload arguments and the seed, so
+two builds run with the same arguments can be compared output for output.
 
 Multi-GPU (N > 1), one process per GPU:
   --shard perms (default)  every GPU scores ALL pairs against its own block of n_perms permutations (the decomposition of
@@ -48,7 +52,8 @@ WORKLOAD = dict(n_cases=5000, n_ctrls=5000, n_genes=15000, n_edges=150000, n_per
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5,
+                    help="timed steps of every timed leg; the e2e leg needs about 30 for a stable figure (host contention comes in bursts)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--kernel", default="auto", choices=["auto", "dense", "sparse"])
@@ -71,11 +76,19 @@ def parse_args():
                          "the benchmarked network up to 20,000 patients, n_edges / 20 above - the reference replays levels 1-3 on the host first "
                          "and keeps an (n+1)^2 table per method-2 thread, SURVEY App. D)")
     ap.add_argument("--cpu-perms", type=int, default=1000, help="permutations the CPU baseline / parity leg scores (the reference's cost per pair*perm does not depend on the count)")
-    ap.add_argument("--e2e-steps", type=int, default=0, help="timed end-to-end steps (default: max(30, --steps))")
+    ap.add_argument("--e2e-steps", type=int, default=0, help="timed end-to-end steps (default: --steps)")
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="target CPU work per method for the baseline sample")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the results of the last timed step (per method and level: permutation maxima and top-K) "
+                         "as DIR/<name>.npy")
     for k, v in WORKLOAD.items():
         ap.add_argument("--" + k.replace("_", "-"), type=type(v), default=v)
-    return ap.parse_args()
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's results: not with --impl reference")
+    return a
 
 
 def make_workload(a):
@@ -504,6 +517,42 @@ def check_parity(ref_out, last_out, state, lv4, w, api, cpu_perms, reset_masks):
     return out
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def device_perm_max(perm_all, world, n_batches, ip, batch_perms, n_perms):
+    """The device vector of last-level maxima, laid out [rank][batch][ip], -> float64 [world * n_perms]: the real permutations of
+    every block, in order.  ip is the batch padded to the kernels' tile, and the slots of a short last batch past its real
+    permutations are scored on copies of real ones: neither is part of the result."""
+    v = np.asarray(perm_all, dtype=np.float64).reshape(world, n_batches, ip)
+    return np.concatenate([v[r, b, : min(batch_perms, n_perms - b * batch_perms)] for r in range(world) for b in range(n_batches)])
+
+
+def dump_outputs(d, last_out, names, last_perm, n_perms, limit=DUMP_LIMIT_BYTES):
+    """What one step returns to its caller, for each method and each level whose result the step keeps (1b and up):
+    <method>_level<k>_perm_max.npy (float64 [n_perms]: the f32 permutation maxima of all batches, widened as the API returns
+    them) and <method>_level<k>_topk.npy (float64 [rows, 5]: score, src, trg, cases, ctrls in the API's ascending order, -inf
+    sentinel row included).  `last_perm[method]` replaces the last level's maxima with the merged [world * n_perms] vector
+    of a perm-sharded run.  Should the maxima exceed half of `limit`, the same fixed, seeded sample of permutation indices is
+    kept from every block of n_perms and the indices are written as perm_sample_index.npy."""
+    os.makedirs(d, exist_ok=True)
+    out, perms = {}, {}
+    for method, step in last_out.items():
+        res, parts = step[1], step[3]
+        for k in [k for k in names if k in res]:
+            v = last_perm[method] if k == names[-1] and method in last_perm else np.concatenate(parts[k])
+            perms[f"{method}_level{k}_perm_max"] = np.asarray(v, dtype=np.float64).reshape(-1, n_perms)
+            out[f"{method}_level{k}_topk"] = np.array([[s.score, s.src, s.trg, s.cases, s.ctrls] for s in res[k].scores], dtype=np.float64).reshape(-1, 5)
+    total = sum(v.nbytes for v in perms.values())
+    if total > limit // 2:
+        keep = np.sort(np.random.default_rng(0).choice(n_perms, size=max(1, int(n_perms * (limit // 2) // total)), replace=False))
+        perms = {k: v[:, keep] for k, v in perms.items()}
+        out["perm_sample_index"] = keep.astype(np.float64)
+    out.update({k: v.reshape(-1) for k, v in perms.items()})
+    for k, v in out.items():
+        np.save(os.path.join(d, k + ".npy"), v)
+
+
 def rerun_level4_prefix(st, lv4, w, x, api):
     """Levels 1-3 again (resident inputs) and the level-4 join over the first x upstream rows."""
     ex, d1, d2 = st["ex"], st["d1"], st["d2"]
@@ -646,6 +695,9 @@ def main():
     # permutations beyond --perm-batch are scored as sequential batches through the same exec (masks of every batch resident)
     batch_perms = int(min(w.n_perms, max(a.perm_batch, 1)))
     n_batches = (w.n_perms + batch_perms - 1) // batch_perms
+    if a.dump_outputs and world > 1 and not shard_perms and n_batches > 1:
+        # each batch's row shards are merged on their own and only the last batch's merged maxima reach the host
+        raise SystemExit("bench.py: --dump-outputs with --shard rows needs n_perms <= --perm-batch")
     W1m = (n + 63) // 64
     masks_dev = torch.from_numpy(np.ascontiguousarray(w.perm_masks).view(np.int64)).cuda() if n_batches > 1 else None
     state = {}
@@ -734,13 +786,13 @@ def main():
 
     def run_batches(st, collective=True, single=False):
         """All permutation batches of one method; returns (per-level info with kernel times summed over the batches, results of the
-        last batch, results of batch 0)."""
-        info_sum, res_last, res_first = None, None, None
+        last batch, results of batch 0, per level the list of every batch's permutation maxima)."""
+        info_sum, res_last, res_first, perms = None, None, None, {}
         for b in range(n_batches):
             ex = st["ex"]
             st["batch"] = b
+            nb = min(batch_perms, w.n_perms - b * batch_perms)
             if n_batches > 1:
-                nb = min(batch_perms, w.n_perms - b * batch_perms)
                 ex.setPermutedMasksDevice(masks_dev.data_ptr() + 8 * b * batch_perms * W1m, nb)
             res = {}
             info = schedule_resident(st, res, collective=collective, single=single)
@@ -748,6 +800,8 @@ def main():
                 export_block(st, b)
             for k in [k for k in res if k.startswith("_")]:
                 del res[k]  # kept path sets go back to the block cache now, not when the next step overwrites `last_out`
+            for k, r in res.items():
+                perms.setdefault(k, []).append(r.permuted_scores[:nb])  # a short last batch is padded with copies of real permutations
             if info_sum is None:
                 info_sum, res_first = info, res
             else:
@@ -756,7 +810,7 @@ def main():
                     info_sum[k]["exact_pairs"] += info[k].get("exact_pairs", 0)
             res_last = res
         st["batch"] = 0
-        return info_sum, res_last, res_first
+        return info_sum, res_last, res_first, perms
 
     def step_resident():
         out = {}
@@ -803,6 +857,11 @@ def main():
     ev1.record(stream)
     sync_all()
     ms_total = ev0.elapsed_time(ev1)
+    if a.dump_outputs and rank == 0:
+        # perm-sharded, the last level's merged maxima of every rank are only in perm_all (which later legs overwrite)
+        last_perm = {m: device_perm_max(state[m]["perm_all"].cpu().numpy(), world, n_batches, state[m]["ex"].iterations, batch_perms, w.n_perms)
+                     for m in state} if shard_perms else {}
+        dump_outputs(a.dump_outputs, last_out, names, last_perm, w.n_perms)
     n_launch = launches() - l0
     clocks = sampler.stop() if rank == 0 else None
     gc.enable()
@@ -884,7 +943,7 @@ def main():
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             return float(t.item())
 
-        k_steps = max(3, min(a.steps, 10))
+        k_steps = a.steps
         ms_one = timed("single", k_steps)
         ms_rows = timed("rows", k_steps)
         strong = {"job": f"the N=1 job ({batch_perms} permutations, all pairs, methods 1+2) done once by the {world} GPUs together",
@@ -1078,7 +1137,7 @@ def main():
         gc.collect()
         gc.freeze()
         gc.disable()  # as in the resident region: a cyclic GC pass costs 100+ ms with torch imported
-        e2e_steps = max(30, a.steps) if a.e2e_steps <= 0 else a.e2e_steps  # ~2 s: bursts of host contention last ~0.5 s
+        e2e_steps = a.steps if a.e2e_steps <= 0 else a.e2e_steps  # host contention comes in ~0.5 s bursts: a stable e2e figure needs ~30 steps
         per_step = []
         for i in range(e2e_steps):
             sync_all()  # every rank starts the step together; the step's own time is host wall clock, result read-back included

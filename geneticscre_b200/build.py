@@ -2,8 +2,9 @@
 
 A build happens only when a source is newer than the library.  Concurrent starters (the N ranks of a torchrun launch, pytest
 workers) serialise on a lock file: one of them compiles into a temporary name and renames it over the library, the others
-find it fresh when they get the lock - nobody ever dlopens a half-written file.  The ptxas resource table of the last build
-is kept in profiles/ptxas_sm100a.log (tracked: registers, spills and shared memory of every kernel).
+find it fresh when they get the lock - nobody ever dlopens a half-written file.  Run as a script
+(``python geneticscre_b200/build.py [--force]``), a build also writes the ptxas resource table of the build (registers, spills and shared memory of every kernel) to the tracked
+profiles/ptxas_sm100a.log; an ordinary build leaves the tracked files alone.
 """
 from __future__ import annotations
 
@@ -36,7 +37,7 @@ def _stale() -> bool:
     return any(os.path.getmtime(d) > t for d in dependencies())
 
 
-def build(force: bool = False, verbose: bool = False) -> str:
+def build(force: bool = False, verbose: bool = False, ptxas_log: bool = False) -> str:
     if not force and not _stale():
         return LIB
     with open(os.path.join(PKG, ".build.lock"), "w") as lock:
@@ -55,16 +56,13 @@ def build(force: bool = False, verbose: bool = False) -> str:
                     os.unlink(tmp)
                 raise RuntimeError("nvcc failed building libgcre_b200.so")
             os.replace(tmp, LIB)  # atomic: a process that already mapped the old file keeps its inode
-            try:
-                os.makedirs(os.path.dirname(PTXAS_LOG), exist_ok=True)
+            if ptxas_log:
                 with open(PTXAS_LOG, "w") as f:
                     f.write(res.stderr)
-            except OSError:
-                pass
         finally:
             fcntl.flock(lock, fcntl.LOCK_UN)
     return LIB
 
 
 if __name__ == "__main__":
-    print(build(force="--force" in sys.argv, verbose=True))
+    print(build(force="--force" in sys.argv, verbose=True, ptxas_log=True))
