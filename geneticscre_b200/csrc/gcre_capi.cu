@@ -362,10 +362,28 @@ struct gcre_exec {
   mutable std::set<gcre_uidset*> uidsets;
 };
 
+// Where the rows of a path set came from: what the tail form of the pre-counted sparse kernel (join_sparse.cuh) needs to know
+// that a level-4 partner's first gene is its upstream row's last gene.  Entries name rows of a base set (base row << 1 |
+// halves swapped, setup_kernels.cuh).  They hold while neither this set nor the base set has been written since: every write
+// drops them (rows_written) and bumps the set's version, which names the base's content.
+struct Provenance {
+  const gcre_pathset* base = nullptr;
+  unsigned long long base_uid = 0, base_ver = 0;  // the base set's identity and version when the entries were made
+  int32_t* sel = nullptr;      // gcre_pathset_select: row k is base row sel[k]
+  uint32_t* tail = nullptr;    // KEEP join result: per row, its partner's base row (the path's last gene)
+  uint32_t* head = nullptr;    // ... and its upstream row's entry when every upstream row was exactly one base row (else null)
+  unsigned long long lo = 0, hi = 0;  // rows [lo, hi) carry entries (a sharded join writes only its rows)
+  bool single = false;         // every row IS its tail: the upstream rows were all zero (level 1a)
+};
+
 struct gcre_pathset {
   const gcre_exec* ex = nullptr;
   uint32_t size = 0;
   uint64_t* d_rows = nullptr;
+  unsigned long long uid = 0;  // process-wide unique: a provenance entry cannot mistake a new set at a reused address for its base
+  unsigned long long ver = 0;  // bumped by every write of the rows
+  bool known_zero = false;     // every row is zero (created and never written)
+  Provenance prov;
   long long max_half_pop = 0;  // max carriers in any half-row; -1 = unknown (recomputed on demand)
   bool zero_pending = false;   // rows are logically zero but the memset has not been issued yet (skipped altogether when
                                // the set's first use is as the fully overwritten result of a join)
@@ -389,6 +407,25 @@ static int materialize_zero(gcre_pathset* ps) {
   if (bytes) CK(cudaMemsetAsync(ps->d_rows, 0, bytes, ps->ex->stream));
   return GCRE_OK;
 }
+
+static void drop_prov(gcre_pathset* ps) {
+  dev_free(ps->ex, ps->prov.sel);
+  dev_free(ps->ex, ps->prov.tail);
+  dev_free(ps->ex, ps->prov.head);
+  ps->prov = Provenance();
+}
+
+// the rows of `ps` are (about to be) rewritten: whatever is known of their origin no longer holds
+static void rows_written(gcre_pathset* ps) {
+  ps->ver++;
+  ps->known_zero = false;
+  drop_prov(ps);
+}
+
+static std::atomic<unsigned long long> g_pathset_uid{0};
+
+// Only the 1,024-permutation kernel has the tail form: at <= 512 permutations (split-carrier kernels) nothing is recorded
+static bool provenance_useful(const gcre_exec* ex) { return !sparse_sc_enabled(ex->Ip, ex->Iw / 32); }
 
 static void drop_view(gcre_pathset* ps) {
   dev_free(ps->ex, ps->view.off);
@@ -539,6 +576,7 @@ extern "C" int gcre_exec_destroy(gcre_exec* ex) {
       dev_free(ex, ps->d_rows);
       ps->d_rows = nullptr;
       drop_view(ps);
+      drop_prov(ps);
       ps->ex = nullptr;
     }
     for (gcre_uidset* us : ex->uidsets) {
@@ -907,6 +945,8 @@ extern "C" int gcre_pathset_create(const gcre_exec* ex, uint32_t size, gcre_path
   if (!ps) return fail(GCRE_ERR_NOMEM, "host allocation failed");
   ps->ex = ex;
   ps->size = size;
+  ps->uid = ++g_pathset_uid;
+  ps->known_zero = true;
   const size_t bytes = (size_t)size * row_words(ex) * 8;
   if (bytes) {
     cudaError_t e = dev_alloc(ex, (void**)&ps->d_rows, bytes);
@@ -934,6 +974,7 @@ extern "C" int gcre_pathset_destroy(gcre_pathset* ps) {
     }
     dev_free(ps->ex, ps->d_rows);  // back to the block cache, no driver call
     drop_view(ps);
+    drop_prov(ps);
   }
   delete ps;
   return GCRE_OK;
@@ -993,6 +1034,7 @@ extern "C" int gcre_pathset_load_i32(gcre_pathset* ps, const int32_t* data, uint
   // width and count such bits as controls of the true score only - there is no patient they could belong to).
   if (rows > 0 && (cols < 0 || cols > ex->n)) return fail(GCRE_ERR_RANGE, "assertion");
   if (rows == 0) return GCRE_OK;
+  rows_written(ps);
   ps->zero_pending = false;
   CK(cudaMemsetAsync(ps->d_rows, 0, (size_t)ps->size * row_words(ex) * 8, ex->stream));
   // Where to pack.  The int matrix is 32x its bits: above a few tens of MB, and with enough host threads to stream it faster
@@ -1052,6 +1094,7 @@ extern "C" int gcre_pathset_load_bits_device(gcre_pathset* ps, const uint64_t* d
   if (rows != ps->size) return fail(GCRE_ERR_ASSERT, "assertion");
   if (rows > 0 && (words_per_row < 0 || words_per_row > ex->W64)) return fail(GCRE_ERR_RANGE, "assertion");
   if (rows == 0) return GCRE_OK;
+  rows_written(ps);
   ps->zero_pending = false;
   CK(cudaMemsetAsync(ps->d_rows, 0, (size_t)ps->size * row_words(ex) * 8, ex->stream));
   if (words_per_row > 0) {
@@ -1076,7 +1119,7 @@ extern "C" int gcre_exec_set_value_table_device(gcre_exec* ex, const double* d_t
   ex->vt_cols = cols;
   const size_t bytes = std::max<size_t>((size_t)rows * cols, 1) * 8;
   CK(dev_alloc(ex, (void**)&ex->d_vt, bytes));
-  if ((size_t)rows * cols) CK(cudaMemcpyAsync(ex->d_vt, d_table, (size_t)rows * cols * 8, cudaMemcpyDeviceToDevice, ex->stream));
+  if ((size_t)rows * cols != 0) CK(cudaMemcpyAsync(ex->d_vt, d_table, (size_t)rows * cols * 8, cudaMemcpyDeviceToDevice, ex->stream));
   ex->diag_cap = -1;
   return GCRE_OK;
 }
@@ -1097,6 +1140,7 @@ extern "C" int gcre_pathset_load_bits(gcre_pathset* ps, const uint64_t* bits, ui
   if (rows != ps->size) return fail(GCRE_ERR_ASSERT, "assertion");
   if (rows > 0 && (words_per_row < 0 || words_per_row > ex->W64)) return fail(GCRE_ERR_RANGE, "assertion");
   if (rows == 0) return GCRE_OK;
+  rows_written(ps);
   ps->zero_pending = false;
   CK(cudaMemsetAsync(ps->d_rows, 0, (size_t)ps->size * row_words(ex) * 8, ex->stream));
   const size_t bytes = (size_t)rows * words_per_row * 8;
@@ -1129,6 +1173,7 @@ extern "C" int gcre_pathset_select(const gcre_pathset* ps, const int32_t* indice
   CKS(gcre_pathset_create(ex, n, &res));
   if (n) {
     res->zero_pending = false;  // every row is written by the gather below
+    res->known_zero = false;
     int rc = [&]() -> int {
       CKS(ex->scratch.ensure((size_t)n * 4));
       CK(cudaMemcpyAsync(ex->scratch.p, indices, (size_t)n * 4, cudaMemcpyHostToDevice, ex->stream));
@@ -1137,6 +1182,14 @@ extern "C" int gcre_pathset_select(const gcre_pathset* ps, const int32_t* indice
                                                                                        row_vec, (ulonglong2*)res->d_rows);
       CK(cudaGetLastError());
       LAUNCHED();
+      // the selection remembers its rows' origin (a KEEP join with it as partner records which base row each result row adds)
+      if (ps->size <= 0x7fffffffu && provenance_useful(ex)) {
+        CK(dev_alloc(ex, (void**)&res->prov.sel, (size_t)n * 4));
+        CK(cudaMemcpyAsync(res->prov.sel, ex->scratch.p, (size_t)n * 4, cudaMemcpyDeviceToDevice, ex->stream));
+        res->prov.base = ps;
+        res->prov.base_uid = ps->uid;
+        res->prov.base_ver = ps->ver;
+      }
       // no host wait: the copy above has read `indices` when it returns unless they are page-locked - then wait for it
       cudaPointerAttributes attr;
       if (cudaPointerGetAttributes(&attr, indices) != cudaSuccess || attr.type != cudaMemoryTypeUnregistered) {
@@ -1168,6 +1221,7 @@ extern "C" int gcre_pathset_set_row(gcre_pathset* ps, uint32_t idx, const uint64
   CKS(use_device(ex));
   if (idx >= ps->size) return fail(GCRE_ERR_RANGE, "assertion");  // src/gcre_paths.h:50
   CKS(materialize_zero(ps));
+  rows_written(ps);
   for (int h = 0; h < ex->M; h++)
     CK(cudaMemcpyAsync(ps->d_rows + (size_t)idx * row_words(ex) + (size_t)h * ex->Wp, words + (size_t)h * ex->W64, (size_t)ex->W64 * 8,
                        cudaMemcpyHostToDevice, ex->stream));
@@ -1402,6 +1456,75 @@ static int ensure_precount(gcre_exec* ex, gcre_pathset* ps) {
 }
 
 // ------------------------------------------------------------------------------------------------------------------
+// provenance (tail form of the pre-counted sparse kernel, join_sparse.cuh)
+// ------------------------------------------------------------------------------------------------------------------
+// the base set `p` names is alive and unchanged since the entries were made
+static bool base_current(const gcre_exec* ex, const Provenance& p) {
+  if (!p.base) return false;
+  std::lock_guard<std::mutex> lock(ex->child_mu);
+  return ex->pathsets.count(const_cast<gcre_pathset*>(p.base)) && p.base->uid == p.base_uid && p.base->ver == p.base_ver;
+}
+
+static bool same_base(const Provenance& a, const Provenance& b) {
+  return a.base == b.base && a.base_uid == b.base_uid && a.base_ver == b.base_ver;
+}
+
+// A KEEP join has written result rows [pair_lo, pair_hi): record their tails (and heads) when the partner set is a selection
+// of a live base set.  Called after rows_written(paths_res).
+static int record_provenance(gcre_exec* ex, const gcre_uidset* us, const gcre_pathset* paths0, const gcre_pathset* paths1, gcre_pathset* paths_res,
+                             uint32_t ub, uint32_t ue, unsigned long long pair_lo, unsigned long long pair_hi) {
+  const Provenance& sel = paths1->prov;
+  if (!provenance_useful(ex) || !us->res_is_prefix || pair_hi <= pair_lo || paths_res == paths0 || paths_res == paths1 || !sel.sel || !base_current(ex, sel)) return GCRE_OK;
+  const Provenance& up = paths0->prov;
+  const bool single = paths0->known_zero;
+  const bool heads = !single && up.tail && up.single && same_base(up, sel) && ub >= up.lo && ue <= up.hi;
+  Provenance& p = paths_res->prov;
+  CK(dev_alloc(ex, (void**)&p.tail, (size_t)paths_res->size * 4));
+  if (heads) CK(dev_alloc(ex, (void**)&p.head, (size_t)paths_res->size * 4));
+  const unsigned grid = grid_for((long long)(ue - ub), 256);
+  if (ex->M == 1)
+    record_rows_kernel<1><<<grid, 256, 0, ex->stream>>>(ub, ue, (const int32_t*)us->count.p, (const uint32_t*)us->loc.p, (const unsigned long long*)us->res.p,
+                                                        (const int32_t*)us->signs.p, us->path_length, sel.sel, up.tail, p.tail, p.head);
+  else
+    record_rows_kernel<2><<<grid, 256, 0, ex->stream>>>(ub, ue, (const int32_t*)us->count.p, (const uint32_t*)us->loc.p, (const unsigned long long*)us->res.p,
+                                                        (const int32_t*)us->signs.p, us->path_length, sel.sel, up.tail, p.tail, p.head);
+  CK(cudaGetLastError());
+  LAUNCHED();
+  p.base = sel.base;
+  p.base_uid = sel.base_uid;
+  p.base_ver = sel.base_ver;
+  p.lo = pair_lo;
+  p.hi = pair_hi;
+  p.single = single;
+  return GCRE_OK;
+}
+
+// The base set whose gene rows a score-only join over upstream rows [ub, ue) may be scored against (tail form), or null:
+// both operands carry entries over the same live base set, and every pair's partner head, oriented by the pair, is its
+// upstream row's tail (one pass over the pairs, one flag read back).
+static int tail_form_base(gcre_exec* ex, const gcre_uidset* us, const gcre_pathset* paths0, const gcre_pathset* paths1, uint32_t ub, uint32_t ue,
+                          const gcre_pathset** out) {
+  *out = nullptr;
+  const Provenance &up = paths0->prov, &pt = paths1->prov;
+  if (!up.tail || !pt.tail || !pt.head || !same_base(up, pt) || !base_current(ex, up) || ub < up.lo || ue > up.hi || ue <= ub) return GCRE_OK;
+  unsigned* d_bad = ex->d_scalars + 12;
+  CK(cudaMemsetAsync(d_bad, 0, sizeof(unsigned), ex->stream));
+  const unsigned grid = grid_for((long long)(ue - ub), 256);
+  if (ex->M == 1)
+    tail_eligible_kernel<1><<<grid, 256, 0, ex->stream>>>(ub, ue, (const int32_t*)us->count.p, (const uint32_t*)us->loc.p, (const int32_t*)us->signs.p,
+                                                          us->path_length, up.tail, pt.head, pt.lo, pt.hi, d_bad);
+  else
+    tail_eligible_kernel<2><<<grid, 256, 0, ex->stream>>>(ub, ue, (const int32_t*)us->count.p, (const uint32_t*)us->loc.p, (const int32_t*)us->signs.p,
+                                                          us->path_length, up.tail, pt.head, pt.lo, pt.hi, d_bad);
+  CK(cudaGetLastError());
+  LAUNCHED();
+  CK(cudaMemcpyAsync(ex->h_scalars + 12, d_bad, sizeof(unsigned), cudaMemcpyDeviceToHost, ex->stream));
+  CK(cudaStreamSynchronize(ex->stream));
+  if (ex->h_scalars[12] == 0) *out = up.base;
+  return GCRE_OK;
+}
+
+// ------------------------------------------------------------------------------------------------------------------
 // join
 // ------------------------------------------------------------------------------------------------------------------
 static int launch_join_dense(gcre_exec* ex, const JoinParams& jp, bool keep, int* launches) {
@@ -1616,6 +1739,7 @@ static int join_impl(gcre_exec* ex, const gcre_uidset* us, const gcre_pathset* p
   CKS(materialize_zero(const_cast<gcre_pathset*>(paths0)));
   CKS(materialize_zero(const_cast<gcre_pathset*>(paths1)));
   if (keep) {
+    rows_written(paths_res);  // (provenance of the new rows is recorded once they are written)
     // result rows that are the running sums of the counts: the join overwrites every word of rows [pair_lo, pair_hi); only the
     // rest of a fresh set needs its zeros (nothing for a full join)
     if (us->res_is_prefix) {
@@ -1688,7 +1812,17 @@ static int join_impl(gcre_exec* ex, const gcre_uidset* us, const gcre_pathset* p
     if (const char* mb = std::getenv("GCRE_PRECOUNT_MAX_MB")) budget = (size_t)std::strtoull(mb, nullptr, 10) << 20;
     const int n_perm_blocks = ex->Iw / 32;
     const bool few_perms = sparse_sc_enabled(ex->Ip, n_perm_blocks);
-    int pc_mode = precount_mode(pair_hi - pair_lo, paths1->size, ex->M, n_perm_blocks, budget);
+    // Tail form (join_sparse.cuh): large score-only joins on the 1,024-permutation kernel whose every pair adds one gene of a
+    // base set to its upstream row, when the base set's count table fits the budget.  GCRE_TEST_TAIL=1 / 0 (test hook) takes
+    // it on joins of any size / never.
+    const gcre_pathset* tail_base = nullptr;
+    if (!keep && !few_perms && pair_hi > pair_lo) {
+      const char* tf = std::getenv("GCRE_TEST_TAIL");
+      const bool want = tf && (*tf == '0' || *tf == '1') ? *tf == '1' : pair_hi - pair_lo >= (1ull << 20);
+      if (want) CKS(tail_form_base(ex, us, paths0, paths1, ub, ue, &tail_base));
+      if (tail_base && (size_t)tail_base->size * ex->M * n_perm_blocks * 2048 > budget) tail_base = nullptr;
+    }
+    int pc_mode = tail_base ? PRECOUNT_NO : precount_mode(pair_hi - pair_lo, paths1->size, ex->M, n_perm_blocks, budget);
     if (few_perms && pc_mode == PRECOUNT_SAMPLE) pc_mode = PRECOUNT_NO;  // the split-carrier kernel is the better form there
     const bool split = few_perms && pc_mode != PRECOUNT_YES;
     const int layout = split ? sparse_sc_words(ex->Ip) : 0;
@@ -1698,10 +1832,12 @@ static int join_impl(gcre_exec* ex, const gcre_uidset* us, const gcre_pathset* p
     const bool base_emitted = paths0->view.pcnt && paths0->view.pcnt_gen == ex->mask_gen && paths0->view.pcnt_layout == layout &&
                               paths0->view.stats_valid && paths0 != paths_res && ub >= paths0->view.emit_lo && ue <= paths0->view.emit_hi;
     if (!base_emitted) CKS(ensure_view(ex, const_cast<gcre_pathset*>(paths0)));
-    CKS(ensure_view(ex, const_cast<gcre_pathset*>(paths1)));
+    // (tail form: the partner rows are scored through the base set's gene rows - their own lists are not needed)
+    const gcre_pathset* partner_lists = tail_base ? tail_base : paths1;
+    CKS(ensure_view(ex, const_cast<gcre_pathset*>(partner_lists)));
     sp.off0 = paths0->view.off; sp.len0 = paths0->view.len; sp.car0 = paths0->view.car; sp.ncase0 = paths0->view.ncase;
     sp.pcnt0 = base_emitted ? paths0->view.pcnt : nullptr;
-    sp.off1 = paths1->view.off; sp.len1 = paths1->view.len; sp.car1 = paths1->view.car; sp.ncase1 = paths1->view.ncase;
+    sp.off1 = partner_lists->view.off; sp.len1 = partner_lists->view.len; sp.car1 = partner_lists->view.car; sp.ncase1 = partner_lists->view.ncase;
     sp.n = ex->n;
     sp.unit_prefix = (const unsigned long long*)us->units.p;
     sp.unit_idx = (const uint32_t*)us->unit_idx.p;
@@ -1742,6 +1878,11 @@ static int join_impl(gcre_exec* ex, const gcre_uidset* us, const gcre_pathset* p
     if (pc_mode == PRECOUNT_YES) {
       CKS(ensure_precount(ex, const_cast<gcre_pathset*>(paths1)));
       sp.pcnt1 = paths1->view.pcnt;
+    }
+    if (tail_base) {
+      CKS(ensure_precount(ex, const_cast<gcre_pathset*>(tail_base)));
+      sp.pcnt1 = tail_base->view.pcnt;
+      sp.tail1 = paths1->prov.tail;
     }
     if (keep && paths_res != paths0 && paths_res != paths1) drop_view(paths_res);  // its rows are about to be rewritten
     if (emit) {
@@ -1933,6 +2074,7 @@ static int join_impl(gcre_exec* ex, const gcre_uidset* us, const gcre_pathset* p
     } else {
       drop_view(paths_res);
     }
+    CKS(record_provenance(ex, us, paths0, paths1, paths_res, ub, ue, pair_lo, pair_hi));
   }
 
   CKS(emit_topk(held, top_k, out_scores, n_scores));
@@ -1951,7 +2093,8 @@ static int join_impl(gcre_exec* ex, const gcre_uidset* us, const gcre_pathset* p
     opts->kernel_ms = kernel_ms;
     opts->kernel_used = kernel;
     opts->launches = launches;
-    opts->precounted = sp.pcnt1 != nullptr;
+    opts->precounted = sp.pcnt1 != nullptr && !sp.tail1;
+    opts->tail_form = sp.tail1 != nullptr;
     opts->split_carrier = kernel == GCRE_KERNEL_SPARSE && sparse_sc_applies(jp, sp);
     opts->shared_masks = shared_masks;
     opts->thresholded = thresholded ? 1 : 0;

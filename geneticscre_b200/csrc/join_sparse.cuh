@@ -29,6 +29,16 @@
 // where up & partner - the partner's carriers that ARE already in the upstream row - is a handful of patients for
 // rare-variant rows (|up|*|partner|/n) instead of the ~|partner| carriers the delta formulation walks.  A pair then costs
 // one 2 KB read of P (coalesced, 4 x LDG.128 per lane), the filter pass over the partner's list and the look-ups.
+//
+// Tail form (template flag TAIL, with PC).  In the level schedule of the reference a level-4 partner row is a path g3 -> t whose
+// first gene g3 is the last gene of the upstream path (a paths2 row against a paths3 row).  When the engine knows where the
+// rows came from (gcre_capi.cu: provenance) and every pair of the join has that shape - the partner's first gene, oriented by
+// the pair, is exactly the upstream row's last gene - then  up | partner == up | gene row of t  and the pre-counted form is
+// applied to the base-set GENE row of t instead of the partner row:
+//        count(up | partner) = count(up) + P[t] - count(up & t)
+// up & t is a fraction of a carrier for rare-variant rows, P over the few thousand gene rows fits in L2, and the gene's list
+// is half as long as the partner's.  s.tail1[loc] names that gene row and its orientation (base row << 1 | halves swapped);
+// off1 / len1 / car1 / ncase1 / pcnt1 then describe the base set.
 #pragma once
 #include <cstdlib>
 
@@ -99,6 +109,7 @@ struct SparseParams {
   uint32_t* len_res;
   uint32_t* ncase_res;
   unsigned long long* exact_pairs;        // diagnostic (thresholded look-ups): pairs whose exact permutation scores had to be looked up
+  const uint32_t* tail1;                  // TAIL kernels: per partner row, the base-set row of its last gene << 1 | halves swapped
 };
 
 // ---- view construction ----------------------------------------------------------------------------------------------
@@ -285,8 +296,10 @@ __device__ __forceinline__ void prefetch_l1(const void* p) { asm volatile("prefe
 
 // CT = carrier index type of the list views: uint16_t (n <= 65,535) or uint32_t
 // THR: thresholded look-ups (below) instead of 32 running maxima per lane in registers
-template <int M, bool KEEP, typename CT, bool PC, bool THR>
+// TAIL (with PC, score-only): partners are scored through the base-set gene row s.tail1 names (see the header)
+template <int M, bool KEEP, typename CT, bool PC, bool THR, bool TAIL = false>
 __global__ void __launch_bounds__(sparse::THREADS, sparse::min_blocks(M, THR)) join_sparse_kernel(const JoinParams a, const SparseParams s) {
+  static_assert(!TAIL || (PC && !KEEP), "the tail form is a score-only pre-counted form");
   using namespace sparse;
   const CT* car0 = static_cast<const CT*>(s.car0);
   const CT* car1 = static_cast<const CT*>(s.car1);
@@ -375,8 +388,9 @@ __global__ void __launch_bounds__(sparse::THREADS, sparse::min_blocks(M, THR)) j
     // PC: pull the pre-counted rows of a partner (2 KB per half and permutation block = 16 lines, one per lane) towards
     // the SM ahead of their use - the table is far larger than L2 and each row is read once per pair
     auto prefetch_partner = [&](uint32_t loc) {
+      const uint32_t row = TAIL ? (__ldg(s.tail1 + loc) >> 1) : loc;
       if (lane < 16 * M)
-        prefetch_l2(reinterpret_cast<const char*>(s.pcnt1) + (((size_t)loc * M + (lane >> 4)) * s.n_perm_blocks + pb) * 2048 + (lane & 15) * 128);
+        prefetch_l2(reinterpret_cast<const char*>(s.pcnt1) + (((size_t)row * M + (lane >> 4)) * s.n_perm_blocks + pb) * 2048 + (lane & 15) * 128);
     };
     if (PC && j0 < j1) prefetch_partner(loc0 + j0);
 
@@ -467,6 +481,7 @@ __global__ void __launch_bounds__(sparse::THREADS, sparse::min_blocks(M, THR)) j
       if (PC && j + 1 < j1) prefetch_partner(loc + 1);
       bool flip = true;
       if (M == 2) flip = need_flip(a.path_length, a.signs, idx, loc);
+      const uint32_t tail = TAIL ? __ldg(s.tail1 + loc) : 0u;
       uint32_t c16[16];          // counts of the half being accumulated (PC: of up & partner only)
       uint32_t nd[M], ncn[M];    // carriers / case carriers the partner adds to the upstream half
       size_t pitem[M];           // PC: the partner item joined into half h
@@ -478,7 +493,8 @@ __global__ void __launch_bounds__(sparse::THREADS, sparse::min_blocks(M, THR)) j
         for (int i = 0; i < 16; i++) c16[i] = PC ? 0u : s_base[h][i][tid];
         // joined half h = upstream half h | partner half hh   (src/methods.h:137-145)
         const int hh = (M == 1) ? 0 : (flip ? h : 1 - h);
-        const size_t item = (size_t)loc * M + hh;
+        // TAIL: half hh of the partner row holds half hh ^ swapped of its gene row
+        const size_t item = TAIL ? (size_t)(tail >> 1) * M + (M == 1 ? 0 : (hh ^ (int)(tail & 1u))) : (size_t)loc * M + hh;
         const CT* lst1 = car1 + s.off1[item];
         const uint32_t len = s.len1[item];
         const uint64_t* p0h = p0row + h * Wp;
@@ -821,14 +837,20 @@ static inline bool sparse_thr(int M, unsigned long long n_pairs) {
   return M == 2 && n_pairs >= (1ull << 20);
 }
 
-template <int M, bool KEEP, bool PC, bool THR>
+template <int M, bool KEEP, bool PC, bool THR, bool TAIL = false>
 static inline void launch_sparse_ct(unsigned grid, cudaStream_t stream, const JoinParams& jp, const SparseParams& sp, bool wide) {
-  if (wide) join_sparse_kernel<M, KEEP, uint32_t, PC, THR><<<grid, sparse::THREADS, 0, stream>>>(jp, sp);
-  else join_sparse_kernel<M, KEEP, uint16_t, PC, THR><<<grid, sparse::THREADS, 0, stream>>>(jp, sp);
+  if (wide) join_sparse_kernel<M, KEEP, uint32_t, PC, THR, TAIL><<<grid, sparse::THREADS, 0, stream>>>(jp, sp);
+  else join_sparse_kernel<M, KEEP, uint16_t, PC, THR, TAIL><<<grid, sparse::THREADS, 0, stream>>>(jp, sp);
 }
 
 template <int M, bool KEEP, bool THR>
 static inline void launch_sparse_pc(unsigned grid, cudaStream_t stream, const JoinParams& jp, const SparseParams& sp, bool wide) {
+  if constexpr (!KEEP) {
+    if (sp.tail1) {
+      launch_sparse_ct<M, false, true, THR, true>(grid, stream, jp, sp, wide);
+      return;
+    }
+  }
   if (sp.pcnt1) launch_sparse_ct<M, KEEP, true, THR>(grid, stream, jp, sp, wide);
   else launch_sparse_ct<M, KEEP, false, THR>(grid, stream, jp, sp, wide);
 }
@@ -839,7 +861,7 @@ static inline void launch_sparse_keep(unsigned grid, cudaStream_t stream, const 
   else launch_sparse_pc<M, false, THR>(grid, stream, jp, sp, wide);
 }
 
-// sp.pcnt1 != null selects the pre-counted-partner kernels; `thr` the thresholded look-ups
+// sp.pcnt1 != null selects the pre-counted-partner kernels (sp.tail1 != null as well: their tail form); `thr` the thresholded look-ups
 static inline cudaError_t launch_join_sparse(cudaStream_t stream, const JoinParams& jp, const SparseParams& sp, int M, bool keep, int sm_count, bool thr) {
   const unsigned long long n_work = sp.n_units * (unsigned long long)sp.n_perm_blocks;
   if (n_work == 0) return cudaSuccess;

@@ -231,4 +231,54 @@ __global__ void finish_uids_kernel(uint32_t n, const int32_t* __restrict__ count
   for (unsigned long long q = units[u]; q < units[u + 1]; q++) unit_idx[q] = u;
 }
 
+// ---- provenance of kept rows (the tail form of the pre-counted sparse kernel, join_sparse.cuh) -------------------------
+// Entries name a row of a base path set and its orientation: base row << 1 | 1 when the row's halves are swapped (method 2:
+// joined half h holds base half 1 - h).  A KEEP join whose partner set is a selection of the base set records, per result
+// row it writes, the partner's base row (`tail`) and - when every upstream row is exactly one oriented base row - the
+// upstream row's entry (`head`).  One thread per upstream row of [ub, ue).
+template <int M>
+__global__ void record_rows_kernel(uint32_t ub, uint32_t ue, const int32_t* __restrict__ count, const uint32_t* __restrict__ location,
+                                   const unsigned long long* __restrict__ res_idx, const int32_t* __restrict__ signs, int path_length,
+                                   const int32_t* __restrict__ sel_idx, const uint32_t* __restrict__ tail0, uint32_t* __restrict__ tail_res,
+                                   uint32_t* __restrict__ head_res) {
+  const uint32_t idx = ub + blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= ue) return;
+  const int c = count[idx];
+  const uint32_t head = head_res ? tail0[idx] : 0u;
+  for (int j = 0; j < c; j++) {
+    const uint32_t loc = location[idx] + (uint32_t)j;
+    const unsigned long long r = res_idx[idx] + (unsigned long long)j;
+    const bool swap = (M == 2) && !need_flip(path_length, signs, idx, loc);  // src/methods.h:137-145: partner half 1 - h joins half h
+    tail_res[r] = ((uint32_t)sel_idx[loc] << 1) | (swap ? 1u : 0u);
+    if (head_res) head_res[r] = head;
+  }
+}
+
+// Does every pair of upstream rows [ub, ue) meet the tail form's condition: the partner's head, oriented as the pair joins it,
+// is the upstream row's tail (same base row, same orientation)?  Partner rows outside [head_lo, head_hi) have no record.
+// Any pair that does not sets *bad.
+template <int M>
+__global__ void tail_eligible_kernel(uint32_t ub, uint32_t ue, const int32_t* __restrict__ count, const uint32_t* __restrict__ location,
+                                     const int32_t* __restrict__ signs, int path_length, const uint32_t* __restrict__ tail0,
+                                     const uint32_t* __restrict__ head1, unsigned long long head_lo, unsigned long long head_hi,
+                                     unsigned* __restrict__ bad) {
+  const uint32_t idx = ub + blockIdx.x * blockDim.x + threadIdx.x;
+  bool ok = true;
+  if (idx < ue) {
+    const int c = count[idx];
+    const uint32_t t = c > 0 ? tail0[idx] : 0u;
+    for (int j = 0; j < c && ok; j++) {
+      const uint32_t loc = location[idx] + (uint32_t)j;
+      if (loc < head_lo || loc >= head_hi) {
+        ok = false;
+        break;
+      }
+      uint32_t h = head1[loc];
+      if (M == 2 && !need_flip(path_length, signs, idx, loc)) h ^= 1u;  // the pair swaps the partner's halves
+      ok = (M == 2) ? h == t : (h >> 1) == (t >> 1);
+    }
+  }
+  if (__any_sync(0xffffffffu, !ok) && (threadIdx.x & 31) == 0) atomicOr(bad, 1u);
+}
+
 }  // namespace gcre

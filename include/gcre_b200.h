@@ -89,7 +89,9 @@ typedef struct {
   int32_t shared_masks;     /* out: 1 when that form ran with the permutation masks staged in shared memory (<= 128 permutations, small cohorts) */
   uint64_t exact_pairs;     /* out: with thresholded look-ups, the pairs (per 1,024-permutation block) whose exact permutation scores
                                had to be looked up; every other pair was ruled out by one compare per look-up */
-  uint64_t reserved2;
+  int32_t tail_form;        /* out: 1 when the pre-counted form ran against the gene rows of the base set the partner rows were
+                               selected from (join_sparse.cuh, tail form: every partner adds one gene to its upstream path) */
+  int32_t reserved2;
 } gcre_join_opts;
 
 /* One split of a reported path for the decorated p-value (R/DecoratedPvalue.R:198-304). */
