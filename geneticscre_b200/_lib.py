@@ -57,6 +57,9 @@ SYMBOLS = {
     "gcre_exec_set_permuted_cases_i32": (_I, [_VP, C.POINTER(C.c_int32), _I, _I]),
     "gcre_exec_set_permuted_masks_u64": (_I, [_VP, C.POINTER(C.c_uint64), _I]),
     "gcre_exec_set_permuted_masks_device": (_I, [_VP, _VP, _I]),
+    "gcre_exec_set_permutation_strata": (_I, [_VP, C.POINTER(C.c_int32), _I]),
+    "gcre_exec_generate_permuted_masks": (_I, [_VP, C.c_uint64, C.c_uint64]),
+    "gcre_exec_get_permuted_masks": (_I, [_VP, C.POINTER(C.c_uint64), _I]),
     "gcre_pathset_create": (_I, [_VP, _U32, C.POINTER(_VP)]),
     "gcre_pathset_destroy": (_I, [_VP]),
     "gcre_pathset_size": (_I, [_VP, C.POINTER(_U32)]),

@@ -9,7 +9,8 @@ reference's own harness (test/harness.cpp:50-181):
     UidRelSet(path_length, uids, signs)                   src/gcre.h:49-90
     Score, joined_res, uid_ref                            src/gcre_types.h:32-56
 
-Extensions (not in the reference): packed inputs (``load_bits``, ``setPermutedMasks``), ``PathSet.to_numpy`` and the
+Extensions (not in the reference): packed inputs (``load_bits``, ``setPermutedMasks``), seeded permutation masks made on the
+device (``setPermutationStrata``, ``generatePermutedMasks``, ``getPermutedMasks``), ``PathSet.to_numpy`` and the
 sharding / kernel-selection options of ``join``.
 """
 from __future__ import annotations
@@ -219,6 +220,27 @@ class JoinExec:
     def setPermutedMasksDevice(self, device_ptr, n_perms):
         """Packed masks uint64[n_perms][ceil(n/64)] already in this GPU's memory; ordered on the exec's stream (extension)."""
         check(self._lib.gcre_exec_set_permuted_masks_device(self._h, C.c_void_p(int(device_ptr)), int(n_perms)))
+
+    def setPermutationStrata(self, labels):
+        """One int32 label per patient for generatePermutedMasks (cases keep their count within every stratum); None or an
+        empty sequence goes back to one stratum (extension)."""
+        if labels is None or len(labels) == 0:
+            check(self._lib.gcre_exec_set_permutation_strata(self._h, None, 0))
+            return
+        lab = _as(labels, np.int32)
+        check(self._lib.gcre_exec_set_permutation_strata(self._h, _ptr(lab, C.c_int32), int(lab.shape[0])))
+
+    def generatePermutedMasks(self, seed, first_perm=0):
+        """Permutations first_perm .. first_perm + iters_requested - 1 of ``seed``, made on the device (include/gcre_b200.h,
+        synth.make_perm_masks_philox); ordered on the exec's stream (extension)."""
+        check(self._lib.gcre_exec_generate_permuted_masks(self._h, int(seed) & (2**64 - 1), int(first_perm) & (2**64 - 1)))
+
+    def getPermutedMasks(self, n_perms=None):
+        """The current masks as uint64[n_perms][ceil(n/64)] (default: all iters_requested rows), whichever setter made them."""
+        n_perms = self.iters_requested if n_perms is None else int(n_perms)
+        out = np.zeros((max(n_perms, 0), self.w64), dtype=np.uint64)
+        check(self._lib.gcre_exec_get_permuted_masks(self._h, _ptr(out, C.c_uint64), n_perms))
+        return out
 
     def createPathSet(self, size):
         out = C.c_void_p()

@@ -27,6 +27,7 @@
 #include "join_sparse_sc.cuh"
 #include "value_table.cuh"
 #include "decorated.cuh"
+#include "perm_gen.cuh"
 
 using namespace gcre;
 
@@ -336,6 +337,12 @@ struct gcre_exec {
   uint32_t* d_pt_sc = nullptr;
   bool pt_sc_valid = false;
   unsigned long long mask_gen = 1;  // bumped whenever the permutation masks change: per-path-set pre-count tables depend on them
+  // strata of the seeded mask generator (gcre_exec_set_permutation_strata); n_strata == 0: one stratum, no arrays
+  int n_strata = 0;
+  int32_t* d_strata_idx = nullptr;     // [64 * W64] dense stratum of each patient (0 past n)
+  uint32_t* d_strata_m = nullptr;      // [64 * W64] m_i | last-of-its-stratum-in-its-word << 31 (0 past n)
+  uint64_t* d_strata_peer = nullptr;   // [64 * W64] earlier same-stratum patients of the word, ballot order (perm_gen.cuh)
+  int32_t* d_strata_k = nullptr;       // [n_strata] true case count per stratum
   // value table
   double* d_vt = nullptr;
   int vt_rows = 0, vt_cols = 0;
@@ -587,7 +594,8 @@ extern "C" int gcre_exec_destroy(gcre_exec* ex) {
     ex->uidsets.clear();
   }
   for (void* p : {(void*)ex->d_masks, (void*)ex->d_pm, (void*)ex->d_pt, (void*)ex->d_pt_sc, (void*)ex->d_vt, (void*)ex->d_diagD, (void*)ex->d_diagF,
-                  (void*)ex->d_diagDM, (void*)ex->d_diagFM, (void*)ex->d_perm_max, (void*)ex->d_scalars, (void*)ex->d_topk})
+                  (void*)ex->d_diagDM, (void*)ex->d_diagFM, (void*)ex->d_perm_max, (void*)ex->d_scalars, (void*)ex->d_topk, (void*)ex->d_strata_idx,
+                  (void*)ex->d_strata_m, (void*)ex->d_strata_peer, (void*)ex->d_strata_k})
     dev_free(ex, p);
   ex->cand.release();
   ex->scan_tmp.release();
@@ -926,6 +934,97 @@ extern "C" int gcre_exec_set_permuted_masks_device(gcre_exec* ex, const uint64_t
     LAUNCHED();
   }
   CKS(rebuild_mask_layouts(ex));
+  return GCRE_OK;
+}
+
+static void free_strata(gcre_exec* ex) {
+  for (void* p : {(void*)ex->d_strata_idx, (void*)ex->d_strata_m, (void*)ex->d_strata_peer, (void*)ex->d_strata_k}) dev_free(ex, p);
+  ex->d_strata_idx = ex->d_strata_k = nullptr;
+  ex->d_strata_m = nullptr;
+  ex->d_strata_peer = nullptr;
+  ex->n_strata = 0;
+}
+
+// Strata of the seeded generator: per-patient arrays of perm_gen.cuh, built on the host once per setting (O(n)).
+extern "C" int gcre_exec_set_permutation_strata(gcre_exec* ex, const int32_t* labels, int n) {
+  if (!ex) return fail(GCRE_ERR_ARG, "null argument");
+  if (!labels && n == 0) {
+    CKS(use_device(ex));
+    free_strata(ex);
+    return GCRE_OK;
+  }
+  if (n != ex->n) return fail(GCRE_ERR_ASSERT, "assertion");
+  if (!labels) return fail(GCRE_ERR_ARG, "null argument");
+  // dense stratum index in order of first appearance: only the partition matters
+  std::unordered_map<int32_t, int> dense;
+  std::vector<int> g((size_t)n);
+  for (int i = 0; i < n; i++) {
+    g[i] = dense.emplace(labels[i], (int)dense.size()).first->second;
+    if ((int)dense.size() > PG_MAX_STRATA) return fail(GCRE_ERR_RANGE, "more than %d strata", PG_MAX_STRATA);
+  }
+  CKS(use_device(ex));
+  free_strata(ex);
+  const int S = (int)dense.size();
+  if (S <= 1) return GCRE_OK;  // one stratum: the arrays would say what the unstratified kernel assumes
+  const size_t np = (size_t)ex->W64 * 64;
+  std::vector<int32_t> idx(np, 0), k_init((size_t)S, 0);
+  std::vector<uint32_t> m(np, 0), after((size_t)S, 0);
+  std::vector<uint64_t> peer(np, 0), seen((size_t)S, 0);
+  std::vector<int> stamp((size_t)S, -1);
+  for (int i = n - 1; i >= 0; i--) m[i] = ++after[g[i]];
+  for (int i = 0; i < ex->n_cases; i++) k_init[g[i]]++;
+  for (int w = 0; w < ex->W64; w++) {
+    const int a = w * 64, b = std::min(n, a + 64);
+    for (int i = a; i < b; i++) {
+      const int p = i - a;
+      idx[i] = g[i];
+      peer[i] = seen[g[i]];
+      seen[g[i]] |= 1ull << ((p & 1) * 32 + (p >> 1));  // ballot order: lane p/2, half p%2
+    }
+    for (int i = b - 1; i >= a; i--) {
+      if (stamp[g[i]] != w) m[i] |= 1u << 31;  // last of its stratum in this word
+      stamp[g[i]] = w;
+      seen[g[i]] = 0;
+    }
+  }
+  CK(dev_alloc(ex, (void**)&ex->d_strata_idx, np * 4));
+  CK(dev_alloc(ex, (void**)&ex->d_strata_m, np * 4));
+  CK(dev_alloc(ex, (void**)&ex->d_strata_peer, np * 8));
+  CK(dev_alloc(ex, (void**)&ex->d_strata_k, (size_t)S * 4));
+  CK(cudaMemcpyAsync(ex->d_strata_idx, idx.data(), np * 4, cudaMemcpyHostToDevice, ex->stream));
+  CK(cudaMemcpyAsync(ex->d_strata_m, m.data(), np * 4, cudaMemcpyHostToDevice, ex->stream));
+  CK(cudaMemcpyAsync(ex->d_strata_peer, peer.data(), np * 8, cudaMemcpyHostToDevice, ex->stream));
+  CK(cudaMemcpyAsync(ex->d_strata_k, k_init.data(), (size_t)S * 4, cudaMemcpyHostToDevice, ex->stream));
+  CK(cudaStreamSynchronize(ex->stream));  // the host vectors go out of scope
+  ex->n_strata = S;  // only now: a failure above leaves one stratum
+  return GCRE_OK;
+}
+
+extern "C" int gcre_exec_generate_permuted_masks(gcre_exec* ex, uint64_t seed, uint64_t first_perm) {
+  if (!ex) return fail(GCRE_ERR_ARG, "null argument");
+  if (ex->iters == 0) return GCRE_OK;
+  CKS(use_device(ex));
+  const unsigned grid = grid_for(ex->iters, PG_WARPS);
+  if (ex->n_strata > 1)
+    perm_gen_kernel<true><<<grid, PG_WARPS * 32, (size_t)PG_WARPS * ex->n_strata * 4, ex->stream>>>(
+        ex->d_masks, ex->iters, ex->W64, ex->n, ex->n_cases, seed, first_perm, (const int2*)ex->d_strata_idx, (const uint2*)ex->d_strata_m,
+        (const ulonglong2*)ex->d_strata_peer, ex->d_strata_k, ex->n_strata);
+  else
+    perm_gen_kernel<false><<<grid, PG_WARPS * 32, 0, ex->stream>>>(ex->d_masks, ex->iters, ex->W64, ex->n, ex->n_cases, seed, first_perm, nullptr,
+                                                                   nullptr, nullptr, nullptr, 0);
+  CK(cudaGetLastError());
+  LAUNCHED();
+  CKS(rebuild_mask_layouts(ex));  // bumps mask_gen: count tables built against the previous masks are not reused
+  return GCRE_OK;
+}
+
+extern "C" int gcre_exec_get_permuted_masks(const gcre_exec* ex, uint64_t* out, int n_perms) {
+  if (!ex || (!out && n_perms > 0)) return fail(GCRE_ERR_ARG, "null argument");
+  if (n_perms < 0 || n_perms > ex->iters) return fail(GCRE_ERR_RANGE, "assertion");
+  if (n_perms == 0) return GCRE_OK;
+  CKS(use_device(ex));
+  CK(cudaMemcpyAsync(out, ex->d_masks, (size_t)n_perms * ex->W64 * 8, cudaMemcpyDeviceToHost, ex->stream));
+  CK(cudaStreamSynchronize(ex->stream));
   return GCRE_OK;
 }
 

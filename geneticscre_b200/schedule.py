@@ -65,3 +65,30 @@ def replay_levels(ex, uidrelset_cls, workload, path_length: int, use_int_matrice
     if path_length >= 5 and (only is None or "5" in only):  # src/wrapper.cpp:271-276
         run("5", paths3, paths3, zero_set)
     return results, kept
+
+
+def replay_permutation_batches(ex, uidrelset_cls, workload, path_length: int, n_perms: int, seed: int, first_perm: int = 0):
+    """Score the levels against permutations ``first_perm .. first_perm + n_perms - 1`` of ``seed`` in batches of
+    ``ex.iters_requested``, the masks made on the device (``generatePermutedMasks``): no host mask at any permutation count.
+
+    Batch b holds permutations ``first_perm + b * I ...`` (I = ``ex.iters_requested``).  Returns ``{level: joined_res}`` with the
+    batches' maxima concatenated and cut to ``n_perms``, and the top-K, which does not depend on the permutations (checked:
+    every batch must give the same).  ``ex`` must already hold the value table (and any strata).
+    """
+    per = int(ex.iters_requested)
+    if per <= 0:
+        raise ValueError("the exec scores no permutations")
+    out, perms = {}, {}
+    for b in range(-(-int(n_perms) // per)):
+        ex.generatePermutedMasks(seed, first_perm + b * per)
+        results, _ = replay_levels(ex, uidrelset_cls, workload, path_length)
+        for name, r in results.items():
+            top = [(s.score, s.src, s.trg, s.cases, s.ctrls) for s in r.scores]
+            if name in out:
+                if top != out[name]:
+                    raise RuntimeError(f"level {name}: the top-K of permutation batch {b} differs from batch 0's")
+            else:
+                out[name] = top
+                perms[name] = (r, [])
+            perms[name][1].append(np.asarray(r.permuted_scores, dtype=np.float64))
+    return {name: type(r)(r.scores, np.concatenate(ps)[: int(n_perms)]) for name, (r, ps) in perms.items()}

@@ -92,6 +92,88 @@ def make_perm_masks(n_cases: int, n_ctrls: int, n_perms: int, seed: int) -> np.n
     return out
 
 
+PHILOX_M0, PHILOX_M1 = 0xD2511F53, 0xCD9E8D57  # Philox4x32-10 (Salmon et al. 2011): round multipliers
+PHILOX_W0, PHILOX_W1 = 0x9E3779B9, 0xBB67AE85  # ... and key increments
+
+
+def philox4x32_10(c0, c1, c2, c3, k0: int, k1: int):
+    """Philox4x32-10 on numpy arrays (any broadcastable shapes) of 32-bit counter words; returns the four output words as uint64
+    arrays holding 32-bit values."""
+    u32 = np.uint64(0xFFFFFFFF)
+    c = [np.asarray(x, dtype=np.uint64) & u32 for x in (c0, c1, c2, c3)]
+    k0, k1 = int(k0) & 0xFFFFFFFF, int(k1) & 0xFFFFFFFF
+    m0, m1, s = np.uint64(PHILOX_M0), np.uint64(PHILOX_M1), np.uint64(32)
+    for _ in range(10):
+        p0, p1 = m0 * c[0], m1 * c[2]  # exact: 32 x 32 -> 64 bits
+        c = [(p1 >> s) ^ c[1] ^ np.uint64(k0), p1 & u32, (p0 >> s) ^ c[3] ^ np.uint64(k1), p0 & u32]
+        k0, k1 = (k0 + PHILOX_W0) & 0xFFFFFFFF, (k1 + PHILOX_W1) & 0xFFFFFFFF
+    return c
+
+
+def _perm_strata_plan(n_cases: int, n_ctrls: int, strata=None):
+    """(stratum index int64[n], m int64[n], k0 int64[S]) of the seeded generator: patient i's dense stratum, the number of its
+    stratum's patients with index >= i, and each stratum's true case count.  Only the partition ``strata`` induces matters."""
+    n = n_cases + n_ctrls
+    if strata is None:
+        g = np.zeros(n, dtype=np.int64)
+    else:
+        lab = np.asarray(strata)
+        if lab.shape != (n,):
+            raise ValueError("strata must hold one label per patient")
+        g = np.unique(lab, return_inverse=True)[1].reshape(n).astype(np.int64)
+    s = int(g.max()) + 1 if n else 0
+    seen_after = np.zeros(s, dtype=np.int64)
+    m = np.empty(n, dtype=np.int64)
+    for i in range(n - 1, -1, -1):  # O(n) once per strata setting
+        seen_after[g[i]] += 1
+        m[i] = seen_after[g[i]]
+    return g, m, np.bincount(g[:n_cases], minlength=s).astype(np.int64)
+
+
+def make_perm_masks_philox(n_cases: int, n_ctrls: int, n_perms: int, seed: int, first_perm: int = 0, strata=None) -> np.ndarray:
+    """Packed case masks ``uint64[n_perms][W64]`` of permutations ``first_perm .. first_perm + n_perms - 1`` of ``seed``: the
+    numpy restatement of the device generator (``gcre_exec_generate_permuted_masks``, csrc/perm_gen.cuh), bit for bit.
+
+    Patient i of permutation r draws ``u_i`` from Philox4x32-10 with key (lo32(seed), hi32(seed)) and counter
+    (i >> 1, lo32(r), hi32(r), 0): ``x0 | x1 << 32`` for even i, ``x2 | x3 << 32`` for odd i.  Patients are visited in index
+    order (sequential selection sampling per stratum); i is a case iff ``mulhi64(u_i, m_i) < k_g``, where m_i counts the
+    not-yet-visited patients of i's stratum g (i included) and k_g the cases still to place in g (initially g's patients with
+    index < n_cases).  Every row keeps each stratum's true case count; with one stratum every case set is equally likely up to
+    < 2^-64 per decision.  Pure numpy, no CUDA library: a CPU-only caller can feed the reference the same masks.
+    """
+    n = n_cases + n_ctrls
+    w = words_for(n)
+    out = np.zeros((n_perms, w), dtype=np.uint64)
+    if n_perms <= 0 or n == 0:
+        return out
+    g, m, k0 = _perm_strata_plan(n_cases, n_ctrls, strata)
+    seed, first_perm = int(seed) & (2**64 - 1), int(first_perm) & (2**64 - 1)
+    pairs = (n + 1) // 2
+    j = np.arange(pairs, dtype=np.uint64)[None, :]
+    u32, s32 = np.uint64(0xFFFFFFFF), np.uint64(32)
+    m_lo = m.astype(np.uint64)[None, :]
+    block = max(1, min(n_perms, (1 << 23) // max(pairs, 1)))  # bounds the temporaries to ~ 8 M pairs at a time
+    for b0 in range(0, n_perms, block):
+        nb = min(block, n_perms - b0)
+        r = ((np.arange(nb, dtype=object) + first_perm + b0) % (2**64)).astype(np.uint64)[:, None]
+        x0, x1, x2, x3 = philox4x32_10(j, r & u32, r >> s32, np.uint64(0), seed, seed >> 32)
+        u = np.empty((nb, 2 * pairs), dtype=np.uint64)
+        u[:, 0::2] = x0 | (x1 << s32)
+        u[:, 1::2] = x2 | (x3 << s32)
+        u = u[:, :n]
+        # mulhi64(u, m) for m < 2^32, exactly: (hi32(u) * m + ((lo32(u) * m) >> 32)) >> 32
+        v = (((u >> s32) * m_lo + (((u & u32) * m_lo) >> s32)) >> s32).astype(np.int64).T.copy()  # [n][nb]
+        k = np.repeat(k0[:, None], nb, axis=1)  # [S][nb]
+        case = np.empty((n, nb), dtype=bool)
+        for i in range(n):
+            kg = k[g[i]]
+            sel = v[i] < kg
+            case[i] = sel
+            kg -= sel
+        out[b0 : b0 + nb] = pack_bits(case.T)
+    return out
+
+
 def log_factorials(n: int) -> np.ndarray:
     """log(k!) for k = 0..n from libm's lgamma (math.lgamma) - the same routine the engine's host code calls
     (gcre_log_factorial_table: std::lgamma), so the device generator and this restatement start from identical doubles.

@@ -145,6 +145,20 @@ class JoinExec {
                          [&](size_t d) { return gcre_exec_set_permuted_cases_i32(handles_[d], flat.data(), (int)rows, (int)cols); });
   }
 
+  // Extensions (include/gcre_b200.h): strata of the seeded generator (one label per patient; empty = one stratum) and
+  // permutations first_perm .. first_perm + iters_requested - 1 of seed made on every GPU - identical seeds give identical
+  // masks everywhere, so the sharded joins see the same permutations on each device.
+  void setPermutationStrata(const vector<int>& labels) {
+    if (!labels.empty()) check_equal(labels.size(), (size_t)num_cases + num_ctrls);
+    std::vector<int32_t> lab(labels.begin(), labels.end());
+    gcre_for_each_device(handles_.size(), [&](size_t d) {
+      return gcre_exec_set_permutation_strata(handles_[d], lab.empty() ? nullptr : lab.data(), (int)lab.size());
+    });
+  }
+  void generatePermutedMasks(uint64_t seed, uint64_t first_perm = 0) {
+    gcre_for_each_device(handles_.size(), [&](size_t d) { return gcre_exec_generate_permuted_masks(handles_[d], seed, first_perm); });
+  }
+
   // src/join_base.cpp:156-161
   TPathSet createPathSet(st_pathset_size size) const {
     std::vector<gcre_pathset*> ps(handles_.size(), nullptr);

@@ -147,6 +147,32 @@ int gcre_exec_set_permuted_masks_u64(gcre_exec* ex, const uint64_t* masks, int n
  * exec's stream, returns without waiting. */
 int gcre_exec_set_permuted_masks_device(gcre_exec* ex, const uint64_t* d_masks, int n_perms);
 
+/* Seeded permutation masks made on the device (extension; no host matrix).  Permutation r (a global 64-bit index) of seed s:
+ *   draws    patient i takes u_i = x0 | x1 << 32 (i even) or x2 | x3 << 32 (i odd) of Philox4x32-10 (Salmon et al. 2011; M0 =
+ *            0xD2511F53, M1 = 0xCD9E8D57, W0 = 0x9E3779B9, W1 = 0xBB67AE85) with key (lo32(s), hi32(s)) and counter
+ *            (i >> 1, lo32(r), hi32(r), 0);
+ *   choice   patients are visited in index order i = 0 .. n-1; with g the stratum of i, m_g the patients of g not yet visited
+ *            (i included) and k_g the cases still to place in g (initially g's patients with index < num_cases), i is a case
+ *            iff mulhi64(u_i, m_g) < k_g (the high 64 bits of the 128-bit product); then m_g -= 1 and, if i was picked, k_g -= 1.
+ * So every row keeps each stratum's true case count, each decision's probability is within 2^-64 of k_g / m_g and, with one
+ * stratum, every case set of num_cases patients is equally likely: the null of R's permutation matrix, not R's sample() stream.
+ * Permutation r is the same whatever batch or GPU makes it.  geneticscre_b200/synth.py (make_perm_masks_philox) restates this
+ * in numpy bit for bit.
+ *
+ * gcre_exec_set_permutation_strata: labels = one arbitrary int32 per patient (n must be num_cases + num_ctrls, GCRE_ERR_ASSERT
+ * otherwise); only the partition matters, so relabelling gives identical masks.  At most 1,024 distinct labels
+ * (GCRE_ERR_RANGE beyond, the setting is left as it was).  labels = NULL with n = 0 goes back to one stratum.  The host buffer
+ * has been read on return; the per-patient tables stay on the device.  The current masks are not changed. */
+int gcre_exec_set_permutation_strata(gcre_exec* ex, const int32_t* labels, int n);
+/* Rows 0 .. iters_requested-1 := permutations first_perm, first_perm + 1, ... of seed (bit i % 64 of word i / 64 set iff
+ * patient i is a case; bits at i >= n zero: what gcre_exec_set_permuted_masks_* accepts).  Ordered on the exec's stream,
+ * returns without waiting; nothing to do with 0 iterations.  A batched or sharded job gives batch b of rank r
+ * first_perm = (r * n_batches + b) * iters_requested. */
+int gcre_exec_generate_permuted_masks(gcre_exec* ex, uint64_t seed, uint64_t first_perm);
+/* Copy the first n_perms (<= iters_requested, GCRE_ERR_RANGE otherwise) of the current masks to the host as
+ * uint64[n_perms][ceil(n/64)], whichever setter made them (setPermutedCases' int matrix included); waits for the exec's stream. */
+int gcre_exec_get_permuted_masks(const gcre_exec* ex, uint64_t* out, int n_perms);
+
 /* JoinExec::createPathSet(size)  (src/join_base.cpp:156-161): size rows of width_ul*method words, zero-filled. */
 int gcre_pathset_create(const gcre_exec* ex, uint32_t size, gcre_pathset** out);
 int gcre_pathset_destroy(gcre_pathset* ps);

@@ -1,4 +1,4 @@
-"""DESIGN.md = tools/design/DESIGN.template.md with its two tables (NUMBERS_TABLE, CONFIGS_TABLE) filled from the JSON lines under profiles/.
+"""DESIGN.md = tools/design/DESIGN.template.md with its tables (NUMBERS_TABLE, CONFIGS_TABLE, PERM_GEN_TABLE) filled from the JSON files under profiles/.
 
     python tools/design/assemble_design.py
 """
@@ -39,8 +39,21 @@ configs=f"""| Config | How it is covered | Result |
 | 3 at path length 5 (108 M level-5 pairs) | `bench.py --path-length 5` | {len5['value']:.3g} ({len5['ms_per_step']:.0f} ms per step; level 5 {ms(len5,'method1','5'):.0f} / {ms(len5,'method2','5'):.0f} ms; round 1: 6.0e11, 406 ms) |
 | 4 100k patients, len 5, 10,000 perms over 2/4/8 GPUs | `bench.py --n-cases 50000 --n-ctrls 50000 --path-length 5 --n-perms 10000/N` under torchrun; 32-bit carrier indices, value table generated on the device, 2 permutation batches at N = 2 (the reference cannot run this shape: App. D) | 2 / 4 / 8 GPUs: {c4[2]['value']:.3g} / {c4[4]['value']:.3g} / {c4[8]['value']:.3g} pair·perm/s = {c4[2]['ms_per_step']/1e3:.2f} / {c4[4]['ms_per_step']/1e3:.2f} / {c4[8]['ms_per_step']/1e3:.2f} s per 2.4e12-pair·perm step (level 5 of method 2: {ms(c4[2],'method2','5')/1e3:.1f} / {ms(c4[4],'method2','5')/1e3:.1f} / {ms(c4[8],'method2','5')/1e3:.1f} s); merged maxima checked against a single-rank recomputation (`multi_gpu_parity`: 0 mismatches). Not linear in N because a 1,024-permutation block is the unit of work: 5,000 / 2,500 / 1,250 permutations per GPU are 5 / 3 / 2 blocks. Limiter at 8 GPUs: the level-5 kernels themselves (90 % of the step), neither the replicated levels nor the collective (one 40 KB allreduce per method) |
 | 5 perm sweep at 50k patients, len 4 | `--n-cases 25000 --n-ctrls 25000 --n-perms P`; more than 4,096 permutations run as sequential batches with the masks resident (`--perm-batch`) | 1 GPU, 100 / 1,000 / 10,000 / 100,000 permutations: {c5[100]['value']:.3g} / {c5[1000]['value']:.3g} / {c5[10000]['value']:.3g} / {c5[100000]['value']:.3g} ({c5[100]['ms_per_step']:.0f} ms / {c5[1000]['ms_per_step']:.0f} ms / {c5[10000]['ms_per_step']/1e3:.2f} s / {c5[100000]['ms_per_step']/1e3:.2f} s per step); issue-slot roofline {c5[100]['roofline']['frac']:.2f} (100, split-carrier kernels) and {c5[1000]['roofline']['frac']:.2f} (1,000); 8 GPUs, 8,000 / 100,000 permutations in total (the second one measured with the build before the last two kernel changes): {c58a['value']:.3g} / {c58b['value']:.3g} ({c58a['ms_per_step']:.0f} ms / {c58b['ms_per_step']/1e3:.2f} s per step). CPU beside it (`r2_config5_n1_p1000.json`): the reference on the largest sub-shape it can run with the same W64 = 782 and value table (50,000 patients, 7,500 edges, 849 k level-4 pairs, method 1, 16 threads): {cpu5['value']:.3g} pair·perm/s - method 2 needs a private 20 GB table per thread and join and never frees it (one thread is all a 196 GB host can hold) |"""
+pg=L("r4_perm_gen.json")
+perm_gen="| patients | permutations | strata | generator call (incl. layout rebuild) | generator kernel | layout rebuild | host `make_perm_masks` | host / device |\n|---|---|---|---|---|---|---|---|\n"
+for r in pg["shapes"]:
+    host=f"{r['host_ms']:,.0f} ms"+(f" (scaled from {r['host_perms_timed']:,} masks)" if r["host_scaled"] else "")
+    perm_gen+=f"| {r['patients']:,} | {r['perms']:,} | {r['strata']} | {r['ms_per_call_with_layout']:.3f} ms | {r['kernel_ms']:.3f} ms | {r['layout_rebuild_kernel_ms']:.3f} ms | {host} | {r['host_over_device']:,.0f}× |\n"
+bw=pg["bench_workload"]["methods"]
+perm_gen+=(f"\n{pg['gpu']}; CUDA events over {pg['reps']} calls, kernel times from torch.profiler (`profiles/r4_perm_gen.json`, "
+           f"`tools/perm_gen_timing.py`). Bench workload (config 3): a level-schedule replay after `generatePermutedMasks` gives outputs "
+           f"byte-identical to one after `setPermutedMasks(make_perm_masks_philox(...))`: method 1 {'yes' if bw['method1']['byte_identical'] else 'NO'}, method 2 "
+           f"{'yes' if bw['method2']['byte_identical'] else 'NO'}. Replay steps (methods 1 / 2, two timed each): {' / '.join(', '.join(f'{x:.0f}' for x in bw[m]['step_ms_generated']) for m in ('method1', 'method2'))} ms "
+           f"after `generatePermutedMasks`, {' / '.join(', '.join(f'{x:.0f}' for x in bw[m]['step_ms_host_masks']) for m in ('method1', 'method2'))} ms with the host masks uploaded; "
+           f"a replay uploads its inputs inside the step, so these are host-bound and vary by tens of ms with the load of the shared host. "
+           f"The gap between the two method-1 columns cannot come from the generator, which takes 0.06 ms at this shape (table above).")
 s=open(os.path.join(ROOT,"tools","design","DESIGN.template.md")).read()
-s=s.replace("NUMBERS_TABLE",numbers).replace("CONFIGS_TABLE",configs)
+s=s.replace("NUMBERS_TABLE",numbers).replace("CONFIGS_TABLE",configs).replace("PERM_GEN_TABLE",perm_gen)
 s=s.replace("SC_P100_MS","%.1f"%p100['ms_per_step']).replace("SC_P100_L4","%.1f / %.1f"%(ms(p100,'method1','4'),ms(p100,'method2','4')))
 open(os.path.join(ROOT,"DESIGN.md"),"w").write(s)
 print("DESIGN.md written", len(s))
