@@ -315,6 +315,9 @@ constexpr unsigned kSpecCand = 8192;  // candidates copied to the host speculati
 
 struct gcre_exec {
   int M = 1, n_cases = 0, n_ctrls = 0, n = 0, W64 = 0, Wp = 0, iters = 0, Ip = 0, Iw = 0, device = 0, sm_count = 0;
+  // fixed by the shape (and a test hook each) at creation: carrier lists built at one width are read at the same width
+  bool wide = false;      // u32 carrier indices in the sparse views and kernels
+  bool split_ok = false;  // the split-carrier kernels (join_sparse_sc.cuh) are the sparse form of this exec
   cudaStream_t own_stream = nullptr, stream = nullptr;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
   cudaEvent_t ev_piece = nullptr;                                  // upload throttling (copy_pieces)
@@ -432,7 +435,7 @@ static void rows_written(gcre_pathset* ps) {
 static std::atomic<unsigned long long> g_pathset_uid{0};
 
 // Only the 1,024-permutation kernel has the tail form: at <= 512 permutations (split-carrier kernels) nothing is recorded
-static bool provenance_useful(const gcre_exec* ex) { return !sparse_sc_enabled(ex->Ip, ex->Iw / 32); }
+static bool provenance_useful(const gcre_exec* ex) { return !ex->split_ok; }
 
 static void drop_view(gcre_pathset* ps) {
   dev_free(ps->ex, ps->view.off);
@@ -536,6 +539,11 @@ extern "C" int gcre_exec_create(int method, int num_cases, int num_ctrls, int it
   ex->iters = iters;
   ex->Ip = ((std::max(iters, 1) + dense::TI - 1) / dense::TI) * dense::TI;
   ex->Iw = ((ex->Ip / 32 + 31) / 32) * 32;  // words per patient row of the patient-major masks: whole 1,024-perm blocks
+  // u32 carrier indices when n (which is also the sentinel index) does not fit u16; GCRE_TEST_WIDE_CARRIERS=1 (test hook)
+  // forces the u32 path on small cohorts
+  ex->wide = ex->n > 65535 || std::getenv("GCRE_TEST_WIDE_CARRIERS") != nullptr;
+  // few permutations; GCRE_TEST_NO_SPLIT=1 (test hook) keeps the one-word-per-lane kernel
+  ex->split_ok = ex->Ip <= sparse_sc::MAX_PERMS && ex->Iw == 32 && std::getenv("GCRE_TEST_NO_SPLIT") == nullptr;
   ex->device = device;
   int rc = [&]() -> int {
     CK(cudaSetDevice(device));
@@ -849,29 +857,20 @@ static int rebuild_mask_layouts(gcre_exec* ex) {
   return GCRE_OK;
 }
 
-static int ensure_patient_major(gcre_exec* ex) {
-  if (ex->pt_valid) return GCRE_OK;
+// the patient-major masks of the split-carrier kernels (d_pt_sc) or of the others (d_pt)
+static int ensure_patient_major(gcre_exec* ex, bool split) {
+  bool& valid = split ? ex->pt_sc_valid : ex->pt_valid;
+  if (valid) return GCRE_OK;
+  uint32_t*& pt = split ? ex->d_pt_sc : ex->d_pt;
+  const int iw = split ? sparse_sc_words(ex->Ip) : ex->Iw;
   // n + 1 rows: row n is all zero and is what the sentinel entries that pad the carrier lists point at
-  if (!ex->d_pt) CK(dev_alloc(ex, (void**)&ex->d_pt, (size_t)(ex->n + 1) * ex->Iw * 4));
-  CK(cudaMemsetAsync(ex->d_pt + (size_t)ex->n * ex->Iw, 0, (size_t)ex->Iw * 4, ex->stream));
-  const long long warps = (long long)ex->Iw * ((ex->n + 31) / 32);
-  masks_to_patient_major_kernel<<<grid_for(warps * 32, 256), 256, 0, ex->stream>>>(ex->d_masks, ex->iters, ex->W64, ex->n, ex->d_pt, ex->Iw);
-  CK(cudaGetLastError());
-      LAUNCHED();
-  ex->pt_valid = true;
-  return GCRE_OK;
-}
-
-static int ensure_patient_major_sc(gcre_exec* ex) {
-  if (ex->pt_sc_valid) return GCRE_OK;
-  const int iw = sparse_sc_words(ex->Ip);
-  if (!ex->d_pt_sc) CK(dev_alloc(ex, (void**)&ex->d_pt_sc, (size_t)(ex->n + 1) * iw * 4));
-  CK(cudaMemsetAsync(ex->d_pt_sc + (size_t)ex->n * iw, 0, (size_t)iw * 4, ex->stream));
+  if (!pt) CK(dev_alloc(ex, (void**)&pt, (size_t)(ex->n + 1) * iw * 4));
+  CK(cudaMemsetAsync(pt + (size_t)ex->n * iw, 0, (size_t)iw * 4, ex->stream));
   const long long warps = (long long)iw * ((ex->n + 31) / 32);
-  masks_to_patient_major_kernel<<<grid_for(warps * 32, 256), 256, 0, ex->stream>>>(ex->d_masks, ex->iters, ex->W64, ex->n, ex->d_pt_sc, iw);
+  masks_to_patient_major_kernel<<<grid_for(warps * 32, 256), 256, 0, ex->stream>>>(ex->d_masks, ex->iters, ex->W64, ex->n, pt, iw);
   CK(cudaGetLastError());
   LAUNCHED();
-  ex->pt_sc_valid = true;
+  valid = true;
   return GCRE_OK;
 }
 
@@ -1105,10 +1104,8 @@ static int pathset_max_half_pop(gcre_pathset* ps, long long* out) {
     CK(cudaMemsetAsync(ex->d_scalars + 1, 0, sizeof(unsigned), ex->stream));
     if (ps->size) {
       const long long warps = (long long)ps->size * ex->M;
-      if (ex->M == 1)
-        row_maxpop_kernel<1><<<grid_for(warps * 32, 256), 256, 0, ex->stream>>>(ps->d_rows, ps->size, ex->Wp, ex->d_scalars + 1);
-      else
-        row_maxpop_kernel<2><<<grid_for(warps * 32, 256), 256, 0, ex->stream>>>(ps->d_rows, ps->size, ex->Wp, ex->d_scalars + 1);
+      (ex->M == 1 ? row_maxpop_kernel<1> : row_maxpop_kernel<2>)<<<grid_for(warps * 32, 256), 256, 0, ex->stream>>>(ps->d_rows, ps->size, ex->Wp,
+                                                                                                                  ex->d_scalars + 1);
       CK(cudaGetLastError());
       LAUNCHED();
     }
@@ -1461,7 +1458,7 @@ extern "C" int gcre_merge_topk(const gcre_score* lists, const int* list_sizes, i
 // carrier-list views for the sparse kernels
 // ------------------------------------------------------------------------------------------------------------------
 constexpr unsigned long long kViewBoundEntries = 16ull << 20;  // carrier lists up to this many entries (32 / 64 MB) are allocated by their bound
-static int ensure_view(gcre_exec* ex, gcre_pathset* ps) {
+static int ensure_view(gcre_exec* ex, gcre_pathset* ps, bool view_exact) {
   if (ps->view.valid) return GCRE_OK;
   CKS(materialize_zero(ps));
   {  // (re)build lists and stats; counts emitted with the rows stay - the rows have not changed
@@ -1500,7 +1497,7 @@ static int ensure_view(gcre_exec* ex, gcre_pathset* ps) {
     // that bound is small the lists are allocated by the bound and the host does not wait for the scan's total
     // (one device round trip per view, ~10 views per level schedule).
     const unsigned long long bound = ps->max_half_pop >= 0 ? (unsigned long long)items * (((unsigned long long)ps->max_half_pop + 7ull) & ~7ull) : ~0ull;
-    if (bound <= kViewBoundEntries && !std::getenv("GCRE_TEST_VIEW_EXACT")) {
+    if (bound <= kViewBoundEntries && !view_exact) {
       total = bound;
     } else {
       CK(cudaMemcpyAsync(&total, ps->view.off + items, 8, cudaMemcpyDeviceToHost, ex->stream));
@@ -1508,9 +1505,8 @@ static int ensure_view(gcre_exec* ex, gcre_pathset* ps) {
     }
   }
   ps->view.total = (size_t)total;
-  const bool wide = sparse_wide(ex->n);
   {
-    const size_t car_bytes = std::max<size_t>((size_t)total, 8) * (wide ? 4 : 2);
+    const size_t car_bytes = std::max<size_t>((size_t)total, 8) * (ex->wide ? 4 : 2);
     cudaError_t e = dev_alloc(ex, (void**)&ps->view.car, car_bytes);
     if (e != cudaSuccess) {
       cudaGetLastError();
@@ -1519,7 +1515,7 @@ static int ensure_view(gcre_exec* ex, gcre_pathset* ps) {
     }
   }
   if (items > 0) {
-    if (wide)
+    if (ex->wide)
       build_lists_kernel<uint32_t><<<grid_for(items * 32, 256), 256, 0, ex->stream>>>(ps->d_rows, items, ex->Wp, ex->n_cases, ex->n, ps->view.off,
                                                                                      (uint32_t*)ps->view.car, ps->view.ncase);
     else
@@ -1543,7 +1539,7 @@ static int ensure_precount(gcre_exec* ex, gcre_pathset* ps) {
   CK(dev_alloc(ex, (void**)&ps->view.pcnt, std::max<size_t>((size_t)items * nb, 1) * 2048));
   if (items > 0) {
     const unsigned grid = grid_for(items * nb * 32, 128);
-    if (sparse_wide(ex->n))
+    if (ex->wide)
       build_precount_kernel<uint32_t><<<grid, 128, 0, ex->stream>>>(ps->view.off, (const uint32_t*)ps->view.car, items, nb, ex->d_pt, ex->Iw, ps->view.pcnt);
     else
       build_precount_kernel<uint16_t><<<grid, 128, 0, ex->stream>>>(ps->view.off, (const uint16_t*)ps->view.car, items, nb, ex->d_pt, ex->Iw, ps->view.pcnt);
@@ -1580,13 +1576,9 @@ static int record_provenance(gcre_exec* ex, const gcre_uidset* us, const gcre_pa
   Provenance& p = paths_res->prov;
   CK(dev_alloc(ex, (void**)&p.tail, (size_t)paths_res->size * 4));
   if (heads) CK(dev_alloc(ex, (void**)&p.head, (size_t)paths_res->size * 4));
-  const unsigned grid = grid_for((long long)(ue - ub), 256);
-  if (ex->M == 1)
-    record_rows_kernel<1><<<grid, 256, 0, ex->stream>>>(ub, ue, (const int32_t*)us->count.p, (const uint32_t*)us->loc.p, (const unsigned long long*)us->res.p,
-                                                        (const int32_t*)us->signs.p, us->path_length, sel.sel, up.tail, p.tail, p.head);
-  else
-    record_rows_kernel<2><<<grid, 256, 0, ex->stream>>>(ub, ue, (const int32_t*)us->count.p, (const uint32_t*)us->loc.p, (const unsigned long long*)us->res.p,
-                                                        (const int32_t*)us->signs.p, us->path_length, sel.sel, up.tail, p.tail, p.head);
+  (ex->M == 1 ? record_rows_kernel<1> : record_rows_kernel<2>)<<<grid_for((long long)(ue - ub), 256), 256, 0, ex->stream>>>(
+      ub, ue, (const int32_t*)us->count.p, (const uint32_t*)us->loc.p, (const unsigned long long*)us->res.p, (const int32_t*)us->signs.p, us->path_length,
+      sel.sel, up.tail, p.tail, p.head);
   CK(cudaGetLastError());
   LAUNCHED();
   p.base = sel.base;
@@ -1608,13 +1600,8 @@ static int tail_form_base(gcre_exec* ex, const gcre_uidset* us, const gcre_paths
   if (!up.tail || !pt.tail || !pt.head || !same_base(up, pt) || !base_current(ex, up) || ub < up.lo || ue > up.hi || ue <= ub) return GCRE_OK;
   unsigned* d_bad = ex->d_scalars + 12;
   CK(cudaMemsetAsync(d_bad, 0, sizeof(unsigned), ex->stream));
-  const unsigned grid = grid_for((long long)(ue - ub), 256);
-  if (ex->M == 1)
-    tail_eligible_kernel<1><<<grid, 256, 0, ex->stream>>>(ub, ue, (const int32_t*)us->count.p, (const uint32_t*)us->loc.p, (const int32_t*)us->signs.p,
-                                                          us->path_length, up.tail, pt.head, pt.lo, pt.hi, d_bad);
-  else
-    tail_eligible_kernel<2><<<grid, 256, 0, ex->stream>>>(ub, ue, (const int32_t*)us->count.p, (const uint32_t*)us->loc.p, (const int32_t*)us->signs.p,
-                                                          us->path_length, up.tail, pt.head, pt.lo, pt.hi, d_bad);
+  (ex->M == 1 ? tail_eligible_kernel<1> : tail_eligible_kernel<2>)<<<grid_for((long long)(ue - ub), 256), 256, 0, ex->stream>>>(
+      ub, ue, (const int32_t*)us->count.p, (const uint32_t*)us->loc.p, (const int32_t*)us->signs.p, us->path_length, up.tail, pt.head, pt.lo, pt.hi, d_bad);
   CK(cudaGetLastError());
   LAUNCHED();
   CK(cudaMemcpyAsync(ex->h_scalars + 12, d_bad, sizeof(unsigned), cudaMemcpyDeviceToHost, ex->stream));
@@ -1772,36 +1759,348 @@ extern "C" int gcre_uidset_destroy(gcre_uidset* us) {
   return GCRE_OK;
 }
 
-static int join_impl(gcre_exec* ex, const gcre_uidset* us, const gcre_pathset* paths0, const gcre_pathset* paths1, gcre_pathset* paths_res,
-                     int top_k, gcre_score* out_scores, int* n_scores, double* out_perm, gcre_join_opts* opts, PhaseTrace& tr);
-
-extern "C" int gcre_join(gcre_exec* ex, int path_length, const gcre_uid_ref* uids, uint32_t n_uids, const int32_t* signs, uint32_t n_signs,
-                         const gcre_pathset* paths0, const gcre_pathset* paths1, gcre_pathset* paths_res, int top_k, gcre_score* out_scores,
-                         int* n_scores, double* out_perm, gcre_join_opts* opts) {
-  if (!ex || !paths0 || !paths1 || !out_scores || !n_scores || (!uids && n_uids) || (!signs && n_signs))
-    return fail(GCRE_ERR_ARG, "null argument");
-  if (paths0->ex != ex || paths1->ex != ex || (paths_res && paths_res->ex != ex)) return fail(GCRE_ERR_ARG, "path set belongs to another exec");
-  CKS(use_device(ex));
-  PhaseTrace tr;
-  // src/join_base.cpp:196: check_equal(uids.size(), paths0.size) - before any work on the index
-  if (n_uids != paths0->size) return fail(GCRE_ERR_ASSERT, "assertion");
-  gcre_uidset us;
-  int rc = build_uidset(ex, path_length, uids, n_uids, signs, n_signs, &us);
-  tr.mark("index");
-  if (rc == GCRE_OK) rc = join_impl(ex, &us, paths0, paths1, paths_res, top_k, out_scores, n_scores, out_perm, opts, tr);
-  if (rc == GCRE_OK) cudaStreamSynchronize(ex->stream);
-  free_uidset_buffers(&us);
-  return rc;
+static int env_01(const char* name) {  // '0' / '1' -> 0 / 1, anything else -1
+  const char* e = std::getenv(name);
+  return e && (*e == '0' || *e == '1') ? *e - '0' : -1;
 }
 
-extern "C" int gcre_join_uidset(gcre_exec* ex, const gcre_uidset* uidset, const gcre_pathset* paths0, const gcre_pathset* paths1,
-                                gcre_pathset* paths_res, int top_k, gcre_score* out_scores, int* n_scores, double* out_perm,
-                                gcre_join_opts* opts) {
-  if (!ex || !uidset || !paths0 || !paths1 || !out_scores || !n_scores) return fail(GCRE_ERR_ARG, "null argument");
-  if (uidset->ex != ex) return fail(GCRE_ERR_ARG, "join index belongs to another exec");
-  CKS(use_device(ex));
-  PhaseTrace tr;
-  return join_impl(ex, uidset, paths0, paths1, paths_res, top_k, out_scores, n_scores, out_perm, opts, tr);
+static size_t env_mb(const char* name, size_t otherwise) {  // megabytes, in bytes
+  const char* e = std::getenv(name);
+  return e ? (size_t)std::strtoull(e, nullptr, 10) << 20 : otherwise;
+}
+
+static int env_precount() {  // GCRE_PRECOUNT (GCRE_TEST_PRECOUNT in the tests) = 0 / 1 / s
+  const char* f = std::getenv("GCRE_TEST_PRECOUNT");
+  if (!f) f = std::getenv("GCRE_PRECOUNT");
+  if (f && (*f == '0' || *f == '1')) return *f == '1' ? PRECOUNT_YES : PRECOUNT_NO;
+  return f && *f == 's' ? PRECOUNT_SAMPLE : -1;
+}
+
+// Tuning knobs and test hooks of one join, read from the environment when the join starts (not once per process: tests change
+// them between joins).  -1: not set.
+struct JoinKnobs {
+  int thr = env_01("GCRE_THR");            // 0 / 1: thresholded look-ups off / on for every join
+  int precount = env_precount();           // PRECOUNT_NO / _YES / _SAMPLE for every join the budget allows (precount_mode)
+  int tail = env_01("GCRE_TEST_TAIL");     // 0 / 1: the tail form never / on joins of any size
+  int sc_pts = env_01("GCRE_SC_PTS");      // 0 / 1: the shared-memory form of the split-carrier kernels off / on where it fits
+  bool no_emit = env_01("GCRE_TEST_EMIT") == 0;  // kept rows do not take their counts along
+  // every launch-plan size shrunk, so the prefix / budget-overflow / redo paths of run_launch_plan run on tiny joins
+  bool small_plan = std::getenv("GCRE_TEST_SMALL_PLAN") != nullptr;
+  bool view_exact = std::getenv("GCRE_TEST_VIEW_EXACT") != nullptr;  // carrier lists allocated by their exact total (ensure_view)
+  size_t precount_budget = env_mb("GCRE_PRECOUNT_MAX_MB", (size_t)24 << 30);  // device bytes a table of per-permutation counts may take
+};
+
+// One join: its operands and the upstream rows [ub, ue) it covers, with their pairs and sparse work units
+struct JoinCall {
+  gcre_exec* ex;
+  const gcre_uidset* us;
+  const gcre_pathset *paths0, *paths1;
+  gcre_pathset* paths_res;
+  bool keep;
+  int top_k;
+  uint32_t ub, ue;
+  unsigned long long pair_lo, pair_hi, unit_lo, unit_hi;
+  JoinKnobs knobs;
+};
+
+// How a join runs.  choose_join_form decides it; what follows reads it and decides nothing again.
+struct JoinForm {
+  int kernel = GCRE_KERNEL_DENSE;
+  bool split = false;                        // the split-carrier kernels (join_sparse_sc.cuh)
+  bool precount = false;                     // pre-counted partners (PC kernels of join_sparse.cuh)
+  const gcre_pathset* tail_base = nullptr;   // tail form: partners scored through this set's gene rows (PC + TAIL kernels)
+  bool emit = false;                         // kept rows take their counts along
+  bool base_emitted = false;                 // the upstream rows carry counts and totals from the join that made them
+  bool thr = false;                          // thresholded look-ups
+  int layout = 0;                            // count-table layout: 0, or the split-carrier kernels' words per lane group
+  size_t entry_bytes = 0;                    // bytes of one (row, half) entry of a count table in that layout
+};
+
+// the kernel parameters that name a join's operands and its index: the pairs, whatever the form
+static JoinParams pair_params(const gcre_exec* ex, const gcre_uidset* us, const gcre_pathset* paths0, const gcre_pathset* paths1) {
+  JoinParams q;
+  memset(&q, 0, sizeof q);
+  q.p0 = paths0->d_rows;
+  q.p1 = paths1->d_rows;
+  q.Wp = ex->Wp;
+  q.count = (const int32_t*)us->count.p;
+  q.location = (const uint32_t*)us->loc.p;
+  q.prefix = (const unsigned long long*)us->prefix.p;
+  q.res_idx = (const unsigned long long*)us->res.p;
+  q.n_uids = us->n_uids;
+  q.signs = (const int32_t*)us->signs.p;
+  q.path_length = us->path_length;
+  return q;
+}
+
+// Carriers the partner rows share with (sums[0]) and add to (sums[1]) their upstream rows, over n_samples pairs spread evenly
+// over [pair_lo, pair_hi): one launch and one read-back (~40 us)
+static int sample_overlap(gcre_exec* ex, const gcre_uidset* us, const gcre_pathset* paths0, const gcre_pathset* paths1, unsigned long long pair_lo,
+                          unsigned long long pair_hi, int n_samples, unsigned long long sums[2]) {
+  const JoinParams q = pair_params(ex, us, paths0, paths1);
+  unsigned long long* d_sums = reinterpret_cast<unsigned long long*>(ex->d_scalars + 8);
+  CK(cudaMemsetAsync(d_sums, 0, 2 * sizeof(unsigned long long), ex->stream));
+  (ex->M == 1 ? sample_overlap_kernel<1> : sample_overlap_kernel<2>)<<<grid_for((long long)n_samples * 32, 256), 256, 0, ex->stream>>>(q, pair_lo, pair_hi,
+                                                                                                                                      n_samples, d_sums);
+  CK(cudaGetLastError());
+  LAUNCHED();
+  CK(cudaMemcpyAsync(ex->h_scalars + 8, d_sums, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ex->stream));
+  CK(cudaStreamSynchronize(ex->stream));
+  memcpy(sums, ex->h_scalars + 8, 2 * sizeof(unsigned long long));
+  return GCRE_OK;
+}
+
+// The kernel form of a join, in this order: the requested family or AUTO's (cost model, and an overlap sample when the bound
+// does not decide); the fallback to dense where the sparse kernel cannot run; for the sparse kernel the tail form (one device
+// pass), pre-counted partners, split carriers, emitted counts, and the overlap sample that settles pre-counting.  The only
+// device work of the decision is here.  t_needed: carriers a joined half-row may have; mp1: the partner's densest half-row.
+static int choose_join_form(const JoinCall& c, int requested, long long t_needed, long long mp1, JoinForm* f) {
+  gcre_exec* ex = c.ex;
+  const unsigned long long pairs = c.pair_hi - c.pair_lo;
+  const int npb = ex->Iw / 32;
+  f->kernel = requested == GCRE_KERNEL_SPARSE ? GCRE_KERNEL_SPARSE : GCRE_KERNEL_DENSE;
+  if (requested != GCRE_KERNEL_DENSE && requested != GCRE_KERNEL_SPARSE && sparse_supported(ex->n, t_needed, ex->Iw)) {  // AUTO
+    const double dense_ns = dense_pair_ns(ex->W64, ex->Ip, ex->M);
+    if (sparse_pair_ns(npb, ex->M, (double)mp1 * ex->M) <= dense_ns) {
+      f->kernel = GCRE_KERNEL_SPARSE;  // wins even if every partner added its densest half-row in full
+    } else if (sparse_pair_ns(npb, ex->M, 0.0) < dense_ns && pairs > 0) {
+      // it depends on the rows: carriers a partner adds to its upstream row, averaged over 2,048 pairs spread over the join
+      const int n_samples = (int)std::min<unsigned long long>(2048, pairs);
+      unsigned long long sums[2];
+      CKS(sample_overlap(ex, c.us, c.paths0, c.paths1, c.pair_lo, c.pair_hi, n_samples, sums));
+      if (sparse_pair_ns(npb, ex->M, (double)sums[1] / n_samples) <= dense_ns) f->kernel = GCRE_KERNEL_SPARSE;
+    }
+  }
+  // an explicit request for the sparse kernel is honoured whenever its index widths allow
+  if (f->kernel == GCRE_KERNEL_SPARSE && !sparse_supported(ex->n, t_needed, ex->Iw)) f->kernel = GCRE_KERNEL_DENSE;
+  if (f->kernel != GCRE_KERNEL_SPARSE) return GCRE_OK;
+  const size_t budget = c.knobs.precount_budget;
+  // Tail form (join_sparse.cuh): large score-only joins on the 1,024-permutation kernel whose every pair adds one gene of a
+  // base set to its upstream row, when the base set's count table fits the budget.  GCRE_TEST_TAIL=1 / 0 (test hook) takes
+  // it on joins of any size / never.
+  if (!c.keep && !ex->split_ok && pairs > 0) {
+    const bool want = c.knobs.tail >= 0 ? c.knobs.tail == 1 : pairs >= (1ull << 20);
+    if (want) CKS(tail_form_base(ex, c.us, c.paths0, c.paths1, c.ub, c.ue, &f->tail_base));
+    if (f->tail_base && (size_t)f->tail_base->size * ex->M * npb * 2048 > budget) f->tail_base = nullptr;
+  }
+  int pc_mode = f->tail_base ? PRECOUNT_NO : precount_mode(pairs, c.paths1->size, ex->M, npb, budget, c.knobs.precount);
+  if (ex->split_ok && pc_mode == PRECOUNT_SAMPLE) pc_mode = PRECOUNT_NO;  // the split-carrier kernel is the better form there
+  // <= 512 permutations: the split-carrier kernels (join_sparse_sc.cuh) run - unless pre-counted partners are forced
+  // (GCRE_PRECOUNT=1) - and emit / consume count tables in their own, smaller layout
+  f->split = ex->split_ok && pc_mode != PRECOUNT_YES;
+  f->layout = f->split ? sparse_sc_words(ex->Ip) : 0;
+  f->entry_bytes = f->split ? sparse_sc_table_bytes(ex->Ip) : (size_t)npb * 2048;
+  f->thr = !f->split && sparse_thr(ex->M, pairs, c.knobs.thr);
+  // upstream operand: rows that came out of a KEEP join carry their counts and totals - no carrier lists needed
+  const SparseView& v0 = c.paths0->view;
+  f->base_emitted = v0.pcnt && v0.pcnt_gen == ex->mask_gen && v0.pcnt_layout == f->layout && v0.stats_valid && c.paths0 != c.paths_res &&
+                    c.ub >= v0.emit_lo && c.ue <= v0.emit_hi;
+  // kept rows take their counts along (join_sparse.cuh, join_sparse_sc.cuh) when result rows are the running sums of the
+  // counts (res_is_prefix: rows [pair_lo, pair_hi) are exactly the ones this call writes)
+  f->emit = (f->split || !ex->split_ok) && c.keep && pairs > 0 && c.us->res_is_prefix && c.paths_res != c.paths0 && c.paths_res != c.paths1 &&
+            !c.knobs.no_emit && (size_t)c.paths_res->size * ex->M * f->entry_bytes <= budget;
+  if (f->emit && !f->split) pc_mode = PRECOUNT_NO;  // the emitting form of the 1,024-permutation kernel has no pre-counted variant
+  if (pc_mode == PRECOUNT_SAMPLE) {
+    // how much of a partner row is already in its upstream row
+    unsigned long long sums[2];
+    CKS(sample_overlap(ex, c.us, c.paths0, c.paths1, c.pair_lo, c.pair_hi, 2048, sums));
+    pc_mode = (sums[0] * 10 < sums[1] * 6) ? PRECOUNT_YES : PRECOUNT_NO;
+  }
+  f->precount = pc_mode == PRECOUNT_YES;
+  return GCRE_OK;
+}
+
+// What the form reads: patient-major masks, carrier lists of the upstream rows and of the partner (the tail base in tail form),
+// count tables, the result's emitted tables; then the kernel parameters
+static int prepare_join_operands(const JoinCall& c, const JoinForm& f, JoinParams* jp, SparseParams* sp) {
+  gcre_exec* ex = c.ex;
+  memset(sp, 0, sizeof *sp);
+  if (f.kernel == GCRE_KERNEL_SPARSE) {
+    CKS(ensure_patient_major(ex, f.split));
+    gcre_pathset* p0 = const_cast<gcre_pathset*>(c.paths0);
+    gcre_pathset* p1 = const_cast<gcre_pathset*>(f.tail_base ? f.tail_base : c.paths1);
+    if (!f.base_emitted) CKS(ensure_view(ex, p0, c.knobs.view_exact));
+    CKS(ensure_view(ex, p1, c.knobs.view_exact));
+    if (f.precount || f.tail_base) CKS(ensure_precount(ex, p1));
+    sp->off0 = p0->view.off; sp->len0 = p0->view.len; sp->car0 = p0->view.car; sp->ncase0 = p0->view.ncase;
+    sp->pcnt0 = f.base_emitted ? p0->view.pcnt : nullptr;
+    sp->off1 = p1->view.off; sp->len1 = p1->view.len; sp->car1 = p1->view.car; sp->ncase1 = p1->view.ncase;
+    sp->pcnt1 = (f.precount || f.tail_base) ? p1->view.pcnt : nullptr;
+    sp->tail1 = f.tail_base ? c.paths1->prov.tail : nullptr;
+    sp->n = ex->n;
+    sp->unit_prefix = (const unsigned long long*)c.us->units.p;
+    sp->unit_idx = (const uint32_t*)c.us->unit_idx.p;
+    sp->work_counter = (unsigned long long*)(ex->d_scalars + 2);
+    sp->n_perm_blocks = ex->Iw / 32;
+    sp->exact_pairs = reinterpret_cast<unsigned long long*>(ex->d_scalars + 4);
+    gcre_pathset* res = c.paths_res;
+    if (c.keep && res != c.paths0 && res != c.paths1) drop_view(res);  // its rows are about to be rewritten
+    if (f.emit) {
+      const size_t items = (size_t)res->size * ex->M;
+      CK(dev_alloc(ex, (void**)&res->view.pcnt, items * f.entry_bytes));
+      res->view.pcnt_layout = f.layout;
+      CK(dev_alloc(ex, (void**)&res->view.len, items * 4));
+      CK(dev_alloc(ex, (void**)&res->view.ncase, items * 4));
+      sp->pcnt_res = res->view.pcnt;
+      sp->len_res = res->view.len;
+      sp->ncase_res = res->view.ncase;
+    }
+  }
+  CK(cudaMemsetAsync(ex->d_perm_max, 0, (size_t)ex->Ip * 4, ex->stream));
+  CK(cudaMemsetAsync(ex->d_scalars, 0, 2 * sizeof(unsigned), ex->stream));
+  *jp = pair_params(ex, c.us, c.paths0, c.paths1);
+  jp->pres = c.keep ? c.paths_res->d_rows : nullptr;
+  jp->n_cases = ex->n_cases;
+  jp->pm = ex->d_pm;
+  jp->pt = f.split ? ex->d_pt_sc : ex->d_pt;
+  jp->Ip = ex->Ip;
+  jp->Iw = f.split ? sparse_sc_words(ex->Ip) : ex->Iw;
+  jp->n_perm_tiles = ex->Ip / dense::TI;
+  jp->diagD = ex->d_diagD;
+  jp->diagF = ex->d_diagF;
+  jp->diagDM = ex->d_diagDM;
+  jp->diagFM = ex->d_diagFM;
+  jp->perm_max = ex->d_perm_max;
+  jp->cand_count = ex->d_scalars;
+  jp->max_total = ex->d_scalars + 1;
+  if (f.kernel == GCRE_KERNEL_SPARSE && c.top_k <= 64) {
+    CK(cudaMemsetAsync(ex->d_topk, 0, 65 * sizeof(unsigned long long), ex->stream));
+    jp->dyn_thr = ex->d_topk;
+    jp->slots = ex->d_topk + 1;
+    jp->n_slots = c.top_k;
+  }
+  return GCRE_OK;
+}
+
+struct LaunchStats {  // of one join's launch plan (gcre_join_opts)
+  double kernel_ms = 0.0;
+  int launches = 0;
+  unsigned long long exact_pairs = 0;
+  bool shared_masks = false;
+};
+
+// The join's launches; their candidates are merged on the host into the top-K `held`.
+static int run_launch_plan(const JoinCall& c, const JoinForm& f, JoinParams jp, SparseParams sp, PhaseTrace& tr, std::vector<gcre_score>* held,
+                           LaunchStats* st) {
+  gcre_exec* ex = c.ex;
+  // dense kernel: chunks are ranges of flattened pairs; sparse kernel: ranges of units (<= PB pairs each)
+  const bool sparse_k = f.kernel == GCRE_KERNEL_SPARSE;
+  const unsigned long long per_item = sparse_k ? sparse::PB : 1;
+  const unsigned long long item_lo = sparse_k ? c.unit_lo : c.pair_lo, item_hi = sparse_k ? c.unit_hi : c.pair_hi;
+  // Launch plan.  Top-K candidates are appended by the kernels only when their score beats the K-th best known so far,
+  // and a launch must be able to hold every candidate it may produce:
+  //   * small joins (<= 64K pairs): one launch with room for every pair;
+  //   * large joins, sparse kernel, top_k <= 64: ONE launch with the fixed candidate budget - the kernel raises its own
+  //     threshold as candidates arrive (JoinParams::slots; measured: ~300 candidates out of 12 M pairs);
+  //   * other large joins: a short prefix (threshold unknown: every pair is a candidate) establishes the K-th score, then
+  //     ONE launch covers the rest with a fixed candidate budget.  Pairs are visited in ascending (src, trg) order
+  //     across launches, so later pairs only displace on a strictly greater score.  If the budget overflows (scores that
+  //     keep rising), that launch's candidates are dropped and the range is redone in safe chunks (cap = chunk size);
+  //     permutation maxima are max-merged, so re-scoring a pair is harmless.
+  struct Seg { unsigned long long b, e; bool safe; };
+  std::vector<Seg> plan;
+  const bool tiny_plan = c.knobs.small_plan;
+  const unsigned long long small_items = std::max<unsigned long long>(1, (tiny_plan ? 128ull : (64ull << 10)) / per_item);
+  const unsigned long long prefix_items = std::max<unsigned long long>(1, (tiny_plan ? 64ull : (16ull << 10)) / per_item);
+  const unsigned budget = tiny_plan ? 16u : (1u << 20);
+  const unsigned long long redo_first = std::max<unsigned long long>(1, (tiny_plan ? 128ull : (256ull << 10)) / per_item);
+  const unsigned long long redo_max = std::max<unsigned long long>(1, (tiny_plan ? 512ull : (4ull << 20)) / per_item);
+  if (item_hi - item_lo <= small_items) {
+    if (item_hi > item_lo) plan.push_back({item_lo, item_hi, true});
+  } else if (jp.n_slots > 0) {
+    // the kernel tightens its own threshold (JoinParams::slots): no prefix launch needed, a few hundred candidates in all
+    plan.push_back({item_lo, item_hi, false});
+  } else {
+    plan.push_back({item_lo, item_lo + prefix_items, true});
+    plan.push_back({item_lo + prefix_items, item_hi, false});
+  }
+  ex->h_perm_fresh = false;
+  std::vector<Cand> h_cand;
+  unsigned long long thr_key = score_key(-std::numeric_limits<double>::infinity());
+  for (size_t si = 0; si < plan.size(); si++) {
+    const Seg seg = plan[si];
+    const unsigned long long p = seg.b, pe = seg.e;
+    const unsigned cap = seg.safe ? (unsigned)((pe - p) * per_item) : budget;
+    CKS(ex->cand.ensure((size_t)cap * sizeof(Cand)));
+    jp.cand = (Cand*)ex->cand.p;
+    jp.cand_cap = cap;
+    jp.thr_key = thr_key;
+    CK(cudaMemsetAsync(ex->d_scalars, 0, sizeof(unsigned), ex->stream));
+    CK(cudaEventRecord(ex->ev0, ex->stream));
+    if (sparse_k) {
+      sp.unit_begin = p;
+      sp.n_units = pe - p;
+      CK(cudaMemsetAsync(ex->d_scalars + 2, 0, 6 * sizeof(unsigned), ex->stream));
+      if (f.split) CK(launch_join_sparse_sc(ex->stream, jp, sp, ex->M, c.keep, ex->sm_count, ex->wide, c.knobs.sc_pts, &st->shared_masks));
+      else CK(launch_join_sparse(ex->stream, jp, sp, ex->M, c.keep, ex->sm_count, f.precount, f.tail_base != nullptr, f.thr, ex->wide));
+      LAUNCHED();
+      st->launches++;
+    } else {
+      jp.pair_begin = p;
+      jp.pair_end = pe;
+      CKS(launch_join_dense(ex, jp, c.keep, &st->launches));
+    }
+    CK(cudaEventRecord(ex->ev1, ex->stream));
+    CK(cudaMemcpyAsync(ex->h_scalars, ex->d_scalars, 6 * sizeof(unsigned), cudaMemcpyDeviceToHost, ex->stream));
+    if (!ex->h_res.p) CK(pinned_big_acquire((size_t)kSpecCand * sizeof(Cand) + (size_t)ex->Ip * 4, &ex->h_res));
+    Cand* h_spec = static_cast<Cand*>(ex->h_res.p);
+    const unsigned n_spec = std::min(cap, kSpecCand);
+    CK(cudaMemcpyAsync(h_spec, ex->cand.p, (size_t)n_spec * sizeof(Cand), cudaMemcpyDeviceToHost, ex->stream));
+    CK(cudaMemcpyAsync(h_spec + kSpecCand, ex->d_perm_max, (size_t)ex->Ip * 4, cudaMemcpyDeviceToHost, ex->stream));
+    CK(cudaStreamSynchronize(ex->stream));
+    ex->h_perm_fresh = true;
+    float ms = 0.f;
+    CK(cudaEventElapsedTime(&ms, ex->ev0, ex->ev1));
+    st->kernel_ms += ms;
+    st->exact_pairs += (unsigned long long)ex->h_scalars[4] | ((unsigned long long)ex->h_scalars[5] << 32);
+    if (ex->h_scalars[0] > cap) {
+      // budget overflow: redo this range in safe chunks (growing x8 up to 4M pairs)
+      unsigned long long chunk = redo_first;
+      std::vector<Seg> redo;
+      for (unsigned long long q = p; q < pe;) {
+        const unsigned long long qe = std::min(pe, q + chunk);
+        redo.push_back({q, qe, true});
+        q = qe;
+        chunk = std::min(chunk * 8, redo_max);
+      }
+      plan.insert(plan.begin() + si + 1, redo.begin(), redo.end());
+      continue;
+    }
+    const unsigned n_cand = ex->h_scalars[0];
+    if (tr.on) {
+      char buf[96];
+      snprintf(buf, sizeof buf, " [launch %llu..%llu cand=%u %.3fms]", p, pe, n_cand, ms);
+      tr.line += buf;
+      tr.mark("run");
+    }
+    if (n_cand) {
+      h_cand.resize(n_cand);
+      if (n_cand <= n_spec) {
+        memcpy(h_cand.data(), h_spec, (size_t)n_cand * sizeof(Cand));  // already here
+      } else {
+        CK(cudaMemcpyAsync(h_cand.data(), ex->cand.p, (size_t)n_cand * sizeof(Cand), cudaMemcpyDeviceToHost, ex->stream));
+        CK(cudaStreamSynchronize(ex->stream));
+      }
+      for (unsigned k = 0; k < n_cand; k++) {
+        gcre_score sc;
+        sc.score = key_score(h_cand[k].key);
+        sc.src = (int32_t)h_cand[k].idx;
+        sc.trg = (int32_t)h_cand[k].loc;
+        sc.cases = h_cand[k].cases;
+        sc.ctrls = h_cand[k].ctrls;
+        held->push_back(sc);
+      }
+      trim_topk(*held, c.top_k);
+      if ((int)held->size() == c.top_k) {
+        double kth = (*held)[0].score;
+        for (const auto& sc : *held) kth = std::min(kth, sc.score);
+        // later launches hold larger (src, trg) only, so a tie with the K-th score can no longer win a place
+        thr_key = score_key(kth);
+      }
+    }
+    tr.mark("cands");
+  }
+  return GCRE_OK;
 }
 
 static int join_impl(gcre_exec* ex, const gcre_uidset* us, const gcre_pathset* paths0, const gcre_pathset* paths1, gcre_pathset* paths_res,
@@ -1863,309 +2162,21 @@ static int join_impl(gcre_exec* ex, const gcre_uidset* us, const gcre_pathset* p
   CKS(ensure_diag(ex, t_needed));
   tr.mark("diag");
 
-  // ---- kernel choice ----
-  int kernel = opts ? opts->kernel : GCRE_KERNEL_AUTO;
-  if (kernel != GCRE_KERNEL_DENSE && kernel != GCRE_KERNEL_SPARSE) {
-    kernel = GCRE_KERNEL_DENSE;
-    if (sparse_supported(ex->n, t_needed, ex->Iw)) {
-      const int npb = ex->Iw / 32;
-      const double dense_ns = dense_pair_ns(ex->W64, ex->Ip, ex->M);
-      if (sparse_pair_ns(npb, ex->M, (double)mp1 * ex->M) <= dense_ns) {
-        kernel = GCRE_KERNEL_SPARSE;  // wins even if every partner added its densest half-row in full
-      } else if (sparse_pair_ns(npb, ex->M, 0.0) < dense_ns && pair_hi > pair_lo) {
-        // it depends on the rows: carriers a partner adds to its upstream row, averaged over 2,048 pairs spread over the join
-        JoinParams q;
-        memset(&q, 0, sizeof q);
-        q.p0 = paths0->d_rows;
-        q.p1 = paths1->d_rows;
-        q.Wp = ex->Wp;
-        q.prefix = (const unsigned long long*)us->prefix.p;
-        q.location = (const uint32_t*)us->loc.p;
-        q.n_uids = n_uids;
-        q.signs = (const int32_t*)us->signs.p;
-        q.path_length = path_length;
-        const int n_samples = (int)std::min<unsigned long long>(2048, pair_hi - pair_lo);
-        unsigned long long* d_sums = reinterpret_cast<unsigned long long*>(ex->d_scalars + 8);
-        CK(cudaMemsetAsync(d_sums, 0, 2 * sizeof(unsigned long long), ex->stream));
-        if (ex->M == 1) sample_overlap_kernel<1><<<grid_for((long long)n_samples * 32, 256), 256, 0, ex->stream>>>(q, pair_lo, pair_hi, n_samples, d_sums);
-        else sample_overlap_kernel<2><<<grid_for((long long)n_samples * 32, 256), 256, 0, ex->stream>>>(q, pair_lo, pair_hi, n_samples, d_sums);
-        CK(cudaGetLastError());
-        LAUNCHED();
-        CK(cudaMemcpyAsync(ex->h_scalars + 8, d_sums, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ex->stream));
-        CK(cudaStreamSynchronize(ex->stream));
-        unsigned long long sums[2];
-        memcpy(sums, ex->h_scalars + 8, sizeof sums);
-        const double new_per_pair = (double)sums[1] / n_samples;
-        if (sparse_pair_ns(npb, ex->M, new_per_pair) <= dense_ns) kernel = GCRE_KERNEL_SPARSE;
-      }
-    }
-  }
-  // an explicit request for the sparse kernel is honoured whenever its index widths allow
-  if (kernel == GCRE_KERNEL_SPARSE && !sparse_supported(ex->n, t_needed, ex->Iw)) kernel = GCRE_KERNEL_DENSE;
-  SparseParams sp;
-  memset(&sp, 0, sizeof sp);
-  if (kernel == GCRE_KERNEL_SPARSE) {
-    // <= 512 permutations: the split-carrier kernels (join_sparse_sc.cuh) run instead - unless pre-counted partners are forced
-    // (GCRE_PRECOUNT=1) - and emit / consume count tables in their own, smaller layout
-    size_t budget = (size_t)24 << 30;  // device bytes a table of per-permutation counts may take (GCRE_PRECOUNT_MAX_MB overrides)
-    if (const char* mb = std::getenv("GCRE_PRECOUNT_MAX_MB")) budget = (size_t)std::strtoull(mb, nullptr, 10) << 20;
-    const int n_perm_blocks = ex->Iw / 32;
-    const bool few_perms = sparse_sc_enabled(ex->Ip, n_perm_blocks);
-    // Tail form (join_sparse.cuh): large score-only joins on the 1,024-permutation kernel whose every pair adds one gene of a
-    // base set to its upstream row, when the base set's count table fits the budget.  GCRE_TEST_TAIL=1 / 0 (test hook) takes
-    // it on joins of any size / never.
-    const gcre_pathset* tail_base = nullptr;
-    if (!keep && !few_perms && pair_hi > pair_lo) {
-      const char* tf = std::getenv("GCRE_TEST_TAIL");
-      const bool want = tf && (*tf == '0' || *tf == '1') ? *tf == '1' : pair_hi - pair_lo >= (1ull << 20);
-      if (want) CKS(tail_form_base(ex, us, paths0, paths1, ub, ue, &tail_base));
-      if (tail_base && (size_t)tail_base->size * ex->M * n_perm_blocks * 2048 > budget) tail_base = nullptr;
-    }
-    int pc_mode = tail_base ? PRECOUNT_NO : precount_mode(pair_hi - pair_lo, paths1->size, ex->M, n_perm_blocks, budget);
-    if (few_perms && pc_mode == PRECOUNT_SAMPLE) pc_mode = PRECOUNT_NO;  // the split-carrier kernel is the better form there
-    const bool split = few_perms && pc_mode != PRECOUNT_YES;
-    const int layout = split ? sparse_sc_words(ex->Ip) : 0;
-    CKS(split ? ensure_patient_major_sc(ex) : ensure_patient_major(ex));
-    const size_t entry_bytes = split ? sparse_sc_table_bytes(ex->Ip) : (size_t)n_perm_blocks * 2048;  // per (row, half)
-    // upstream operand: rows that came out of a KEEP join carry their counts and totals - no carrier lists needed
-    const bool base_emitted = paths0->view.pcnt && paths0->view.pcnt_gen == ex->mask_gen && paths0->view.pcnt_layout == layout &&
-                              paths0->view.stats_valid && paths0 != paths_res && ub >= paths0->view.emit_lo && ue <= paths0->view.emit_hi;
-    if (!base_emitted) CKS(ensure_view(ex, const_cast<gcre_pathset*>(paths0)));
-    // (tail form: the partner rows are scored through the base set's gene rows - their own lists are not needed)
-    const gcre_pathset* partner_lists = tail_base ? tail_base : paths1;
-    CKS(ensure_view(ex, const_cast<gcre_pathset*>(partner_lists)));
-    sp.off0 = paths0->view.off; sp.len0 = paths0->view.len; sp.car0 = paths0->view.car; sp.ncase0 = paths0->view.ncase;
-    sp.pcnt0 = base_emitted ? paths0->view.pcnt : nullptr;
-    sp.off1 = partner_lists->view.off; sp.len1 = partner_lists->view.len; sp.car1 = partner_lists->view.car; sp.ncase1 = partner_lists->view.ncase;
-    sp.n = ex->n;
-    sp.unit_prefix = (const unsigned long long*)us->units.p;
-    sp.unit_idx = (const uint32_t*)us->unit_idx.p;
-    sp.work_counter = (unsigned long long*)(ex->d_scalars + 2);
-    sp.n_perm_blocks = n_perm_blocks;
-    sp.exact_pairs = reinterpret_cast<unsigned long long*>(ex->d_scalars + 4);
-    // kept rows take their counts along (join_sparse.cuh, join_sparse_sc.cuh) when result rows are the running sums of the
-    // counts (res_is_prefix: rows [pair_lo, pair_hi) are exactly the ones this call writes); GCRE_TEST_EMIT=0 (test hook) turns it off
-    const char* emit_env = std::getenv("GCRE_TEST_EMIT");
-    const bool emit = (split || !few_perms) && keep && pair_hi > pair_lo && us->res_is_prefix && paths_res != paths0 && paths_res != paths1 &&
-                      !(emit_env && *emit_env == '0') && (size_t)paths_res->size * ex->M * entry_bytes <= budget;
-    if (emit && !split) pc_mode = PRECOUNT_NO;  // the emitting form of the 1,024-permutation kernel has no pre-counted variant
-    if (pc_mode == PRECOUNT_SAMPLE) {
-      // how much of a partner row is already in its upstream row: 2,048 pairs spread over the join (~40 us incl. the read-back)
-      JoinParams q;
-      memset(&q, 0, sizeof q);
-      q.p0 = paths0->d_rows;
-      q.p1 = paths1->d_rows;
-      q.Wp = ex->Wp;
-      q.prefix = (const unsigned long long*)us->prefix.p;
-      q.location = (const uint32_t*)us->loc.p;
-      q.n_uids = n_uids;
-      q.signs = (const int32_t*)us->signs.p;
-      q.path_length = path_length;
-      const int n_samples = 2048;
-      unsigned long long* d_sums = reinterpret_cast<unsigned long long*>(ex->d_scalars + 8);
-      CK(cudaMemsetAsync(d_sums, 0, 2 * sizeof(unsigned long long), ex->stream));
-      if (ex->M == 1) sample_overlap_kernel<1><<<grid_for((long long)n_samples * 32, 256), 256, 0, ex->stream>>>(q, pair_lo, pair_hi, n_samples, d_sums);
-      else sample_overlap_kernel<2><<<grid_for((long long)n_samples * 32, 256), 256, 0, ex->stream>>>(q, pair_lo, pair_hi, n_samples, d_sums);
-      CK(cudaGetLastError());
-      LAUNCHED();
-      CK(cudaMemcpyAsync(ex->h_scalars + 8, d_sums, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ex->stream));
-      CK(cudaStreamSynchronize(ex->stream));
-      unsigned long long sums[2];
-      memcpy(sums, ex->h_scalars + 8, sizeof sums);
-      pc_mode = (sums[0] * 10 < sums[1] * 6) ? PRECOUNT_YES : PRECOUNT_NO;
-    }
-    if (pc_mode == PRECOUNT_YES) {
-      CKS(ensure_precount(ex, const_cast<gcre_pathset*>(paths1)));
-      sp.pcnt1 = paths1->view.pcnt;
-    }
-    if (tail_base) {
-      CKS(ensure_precount(ex, const_cast<gcre_pathset*>(tail_base)));
-      sp.pcnt1 = tail_base->view.pcnt;
-      sp.tail1 = paths1->prov.tail;
-    }
-    if (keep && paths_res != paths0 && paths_res != paths1) drop_view(paths_res);  // its rows are about to be rewritten
-    if (emit) {
-      const size_t items = (size_t)paths_res->size * ex->M;
-      CK(dev_alloc(ex, (void**)&paths_res->view.pcnt, items * entry_bytes));
-      paths_res->view.pcnt_layout = layout;
-      CK(dev_alloc(ex, (void**)&paths_res->view.len, items * 4));
-      CK(dev_alloc(ex, (void**)&paths_res->view.ncase, items * 4));
-      sp.pcnt_res = paths_res->view.pcnt;
-      sp.len_res = paths_res->view.len;
-      sp.ncase_res = paths_res->view.ncase;
-    }
-  }
-
-  tr.mark("views");
-  CK(cudaMemsetAsync(ex->d_perm_max, 0, (size_t)ex->Ip * 4, ex->stream));
-  CK(cudaMemsetAsync(ex->d_scalars, 0, 2 * sizeof(unsigned), ex->stream));
-
+  const JoinCall c{ex, us, paths0, paths1, paths_res, keep, top_k, ub, ue, pair_lo, pair_hi, unit_lo, unit_hi, JoinKnobs()};
+  JoinForm form;
+  CKS(choose_join_form(c, opts ? opts->kernel : GCRE_KERNEL_AUTO, t_needed, mp1, &form));
   JoinParams jp;
-  memset(&jp, 0, sizeof jp);
-  jp.p0 = paths0->d_rows;
-  jp.p1 = paths1->d_rows;
-  jp.pres = keep ? paths_res->d_rows : nullptr;
-  jp.Wp = ex->Wp;
-  jp.n_cases = ex->n_cases;
-  jp.count = (const int32_t*)us->count.p;
-  jp.location = (const uint32_t*)us->loc.p;
-  jp.prefix = (const unsigned long long*)us->prefix.p;
-  jp.res_idx = (const unsigned long long*)us->res.p;
-  jp.n_uids = n_uids;
-  jp.signs = (const int32_t*)us->signs.p;
-  jp.path_length = path_length;
-  jp.pm = ex->d_pm;
-  const bool split_form = kernel == GCRE_KERNEL_SPARSE && sparse_sc_enabled(ex->Ip, sp.n_perm_blocks) && !sp.pcnt1;  // == sparse_sc_applies
-  jp.pt = split_form ? ex->d_pt_sc : ex->d_pt;
-  jp.Ip = ex->Ip;
-  jp.Iw = split_form ? sparse_sc_words(ex->Ip) : ex->Iw;
-  jp.n_perm_tiles = ex->Ip / dense::TI;
-  jp.diagD = ex->d_diagD;
-  jp.diagF = ex->d_diagF;
-  jp.diagDM = ex->d_diagDM;
-  jp.diagFM = ex->d_diagFM;
-  jp.perm_max = ex->d_perm_max;
-  jp.cand_count = ex->d_scalars;
-  jp.max_total = ex->d_scalars + 1;
-  if (kernel == GCRE_KERNEL_SPARSE && top_k <= 64) {
-    CK(cudaMemsetAsync(ex->d_topk, 0, 65 * sizeof(unsigned long long), ex->stream));
-    jp.dyn_thr = ex->d_topk;
-    jp.slots = ex->d_topk + 1;
-    jp.n_slots = top_k;
-  }
-
-  // ---- chunked launches; candidates merged on the host between chunks ----
-  // dense kernel: chunks are ranges of flattened pairs; sparse kernel: ranges of units (<= PB pairs each)
-  const bool sparse_k = kernel == GCRE_KERNEL_SPARSE;
-  const unsigned long long per_item = sparse_k ? sparse::PB : 1;
-  const unsigned long long item_lo = sparse_k ? unit_lo : pair_lo, item_hi = sparse_k ? unit_hi : pair_hi;
-  // Launch plan.  Top-K candidates are appended by the kernels only when their score beats the K-th best known so far,
-  // and a launch must be able to hold every candidate it may produce:
-  //   * small joins (<= 64K pairs): one launch with room for every pair;
-  //   * large joins, sparse kernel, top_k <= 64: ONE launch with the fixed candidate budget - the kernel raises its own
-  //     threshold as candidates arrive (JoinParams::slots; measured: ~300 candidates out of 12 M pairs);
-  //   * other large joins: a short prefix (threshold unknown: every pair is a candidate) establishes the K-th score, then
-  //     ONE launch covers the rest with a fixed candidate budget.  Pairs are visited in ascending (src, trg) order
-  //     across launches, so later pairs only displace on a strictly greater score.  If the budget overflows (scores that
-  //     keep rising), that launch's candidates are dropped and the range is redone in safe chunks (cap = chunk size);
-  //     permutation maxima are max-merged, so re-scoring a pair is harmless.
-  struct Seg { unsigned long long b, e; bool safe; };
-  std::vector<Seg> plan;
-  // GCRE_TEST_SMALL_PLAN=1 (test hook) shrinks every size so the prefix / budget-overflow / redo paths run on tiny joins
-  const bool tiny_plan = std::getenv("GCRE_TEST_SMALL_PLAN") != nullptr;
-  const unsigned long long small_items = std::max<unsigned long long>(1, (tiny_plan ? 128ull : (64ull << 10)) / per_item);
-  const unsigned long long prefix_items = std::max<unsigned long long>(1, (tiny_plan ? 64ull : (16ull << 10)) / per_item);
-  const unsigned budget = tiny_plan ? 16u : (1u << 20);
-  const unsigned long long redo_first = std::max<unsigned long long>(1, (tiny_plan ? 128ull : (256ull << 10)) / per_item);
-  const unsigned long long redo_max = std::max<unsigned long long>(1, (tiny_plan ? 512ull : (4ull << 20)) / per_item);
-  if (item_hi - item_lo <= small_items) {
-    if (item_hi > item_lo) plan.push_back({item_lo, item_hi, true});
-  } else if (jp.n_slots > 0) {
-    // the kernel tightens its own threshold (JoinParams::slots): no prefix launch needed, a few hundred candidates in all
-    plan.push_back({item_lo, item_hi, false});
-  } else {
-    plan.push_back({item_lo, item_lo + prefix_items, true});
-    plan.push_back({item_lo + prefix_items, item_hi, false});
-  }
-  ex->h_perm_fresh = false;
+  SparseParams sp;
+  CKS(prepare_join_operands(c, form, &jp, &sp));
+  tr.mark("views");
   std::vector<gcre_score> held;
-  std::vector<Cand> h_cand;
-  unsigned long long thr_key = score_key(-std::numeric_limits<double>::infinity());
-  double kernel_ms = 0.0;
-  int launches = 0;
-  bool thresholded = false;
-  unsigned long long exact_pairs = 0;
-  bool shared_masks = false;
-  for (size_t si = 0; si < plan.size(); si++) {
-    const Seg seg = plan[si];
-    const unsigned long long p = seg.b, pe = seg.e;
-    const unsigned cap = seg.safe ? (unsigned)((pe - p) * per_item) : budget;
-    CKS(ex->cand.ensure((size_t)cap * sizeof(Cand)));
-    jp.cand = (Cand*)ex->cand.p;
-    jp.cand_cap = cap;
-    jp.thr_key = thr_key;
-    CK(cudaMemsetAsync(ex->d_scalars, 0, sizeof(unsigned), ex->stream));
-    CK(cudaEventRecord(ex->ev0, ex->stream));
-    if (sparse_k) {
-      sp.unit_begin = p;
-      sp.n_units = pe - p;
-      CK(cudaMemsetAsync(ex->d_scalars + 2, 0, 6 * sizeof(unsigned), ex->stream));
-      const bool thr = sparse_thr(ex->M, pair_hi - pair_lo);
-      if (sparse_sc_applies(jp, sp)) CK(launch_join_sparse_sc(ex->stream, jp, sp, ex->M, keep, ex->sm_count, &shared_masks));
-      else CK(launch_join_sparse(ex->stream, jp, sp, ex->M, keep, ex->sm_count, thr));
-      thresholded = thresholded || (thr && !sparse_sc_applies(jp, sp));
-      LAUNCHED();
-      launches++;
-    } else {
-      jp.pair_begin = p;
-      jp.pair_end = pe;
-      CKS(launch_join_dense(ex, jp, keep, &launches));
-    }
-    CK(cudaEventRecord(ex->ev1, ex->stream));
-    CK(cudaMemcpyAsync(ex->h_scalars, ex->d_scalars, 6 * sizeof(unsigned), cudaMemcpyDeviceToHost, ex->stream));
-    if (!ex->h_res.p) CK(pinned_big_acquire((size_t)kSpecCand * sizeof(Cand) + (size_t)ex->Ip * 4, &ex->h_res));
-    Cand* h_spec = static_cast<Cand*>(ex->h_res.p);
-    const unsigned n_spec = std::min(cap, kSpecCand);
-    CK(cudaMemcpyAsync(h_spec, ex->cand.p, (size_t)n_spec * sizeof(Cand), cudaMemcpyDeviceToHost, ex->stream));
-    CK(cudaMemcpyAsync(h_spec + kSpecCand, ex->d_perm_max, (size_t)ex->Ip * 4, cudaMemcpyDeviceToHost, ex->stream));
-    CK(cudaStreamSynchronize(ex->stream));
-    ex->h_perm_fresh = true;
-    float ms = 0.f;
-    CK(cudaEventElapsedTime(&ms, ex->ev0, ex->ev1));
-    kernel_ms += ms;
-    exact_pairs += (unsigned long long)ex->h_scalars[4] | ((unsigned long long)ex->h_scalars[5] << 32);
-    if (ex->h_scalars[0] > cap) {
-      // budget overflow: redo this range in safe chunks (growing x8 up to 4M pairs)
-      unsigned long long chunk = redo_first;
-      std::vector<Seg> redo;
-      for (unsigned long long q = p; q < pe;) {
-        const unsigned long long qe = std::min(pe, q + chunk);
-        redo.push_back({q, qe, true});
-        q = qe;
-        chunk = std::min(chunk * 8, redo_max);
-      }
-      plan.insert(plan.begin() + si + 1, redo.begin(), redo.end());
-      continue;
-    }
-    const unsigned n_cand = ex->h_scalars[0];
-    if (tr.on) {
-      char buf[96];
-      snprintf(buf, sizeof buf, " [launch %llu..%llu cand=%u %.3fms]", p, pe, n_cand, ms);
-      tr.line += buf;
-      tr.mark("run");
-    }
-    if (n_cand) {
-      h_cand.resize(n_cand);
-      if (n_cand <= n_spec) {
-        memcpy(h_cand.data(), h_spec, (size_t)n_cand * sizeof(Cand));  // already here
-      } else {
-        CK(cudaMemcpyAsync(h_cand.data(), ex->cand.p, (size_t)n_cand * sizeof(Cand), cudaMemcpyDeviceToHost, ex->stream));
-        CK(cudaStreamSynchronize(ex->stream));
-      }
-      for (unsigned k = 0; k < n_cand; k++) {
-        gcre_score sc;
-        sc.score = key_score(h_cand[k].key);
-        sc.src = (int32_t)h_cand[k].idx;
-        sc.trg = (int32_t)h_cand[k].loc;
-        sc.cases = h_cand[k].cases;
-        sc.ctrls = h_cand[k].ctrls;
-        held.push_back(sc);
-      }
-      trim_topk(held, top_k);
-      if ((int)held.size() == top_k) {
-        double kth = held[0].score;
-        for (const auto& sc : held) kth = std::min(kth, sc.score);
-        // later launches hold larger (src, trg) only, so a tie with the K-th score can no longer win a place
-        thr_key = score_key(kth);
-      }
-    }
-    tr.mark("cands");
-  }
+  LaunchStats st;
+  CKS(run_launch_plan(c, form, jp, sp, tr, &held, &st));
   tr.mark("launches");
   if (keep) {
     // (rows outside a shard of a fresh result set are zero: the kernel's maximum over the written rows is the set's)
     paths_res->max_half_pop = ((pair_lo == 0 && pair_hi == total) || us->res_is_prefix) ? std::max<long long>(paths_res->max_half_pop, (long long)ex->h_scalars[1]) : -1;
-    if (sp.pcnt_res) {  // emitted with the rows
+    if (form.emit) {  // emitted with the rows
       paths_res->view.pcnt_gen = ex->mask_gen;
       paths_res->view.stats_valid = true;
       paths_res->view.emit_lo = pair_lo;
@@ -2178,7 +2189,7 @@ static int join_impl(gcre_exec* ex, const gcre_uidset* us, const gcre_pathset* p
 
   CKS(emit_topk(held, top_k, out_scores, n_scores));
   if (out_perm && !(opts && opts->skip_host_perm)) {
-    if (ex->h_perm_fresh && launches > 0) {  // the maxima came back with the last launch's scalars
+    if (ex->h_perm_fresh && st.launches > 0) {  // the maxima came back with the last launch's scalars
       const float* hp = reinterpret_cast<const float*>(static_cast<Cand*>(ex->h_res.p) + kSpecCand);
       for (int r = 0; r < ex->iters; r++) out_perm[r] = (double)hp[r];  // src/join_base.cpp:145-146
     } else {
@@ -2189,17 +2200,46 @@ static int join_impl(gcre_exec* ex, const gcre_uidset* us, const gcre_pathset* p
   tr.done(keep ? "join(keep)" : "join");
   if (opts) {
     opts->pairs_scored = pair_hi - pair_lo;
-    opts->kernel_ms = kernel_ms;
-    opts->kernel_used = kernel;
-    opts->launches = launches;
-    opts->precounted = sp.pcnt1 != nullptr && !sp.tail1;
-    opts->tail_form = sp.tail1 != nullptr;
-    opts->split_carrier = kernel == GCRE_KERNEL_SPARSE && sparse_sc_applies(jp, sp);
-    opts->shared_masks = shared_masks;
-    opts->thresholded = thresholded ? 1 : 0;
-    opts->exact_pairs = exact_pairs;
+    opts->kernel_ms = st.kernel_ms;
+    opts->kernel_used = form.kernel;
+    opts->launches = st.launches;
+    opts->precounted = form.precount;
+    opts->tail_form = form.tail_base != nullptr;
+    opts->split_carrier = form.split;
+    opts->shared_masks = st.shared_masks;
+    opts->thresholded = form.thr && st.launches > 0 ? 1 : 0;
+    opts->exact_pairs = st.exact_pairs;
   }
   return GCRE_OK;
+}
+
+extern "C" int gcre_join(gcre_exec* ex, int path_length, const gcre_uid_ref* uids, uint32_t n_uids, const int32_t* signs, uint32_t n_signs,
+                         const gcre_pathset* paths0, const gcre_pathset* paths1, gcre_pathset* paths_res, int top_k, gcre_score* out_scores,
+                         int* n_scores, double* out_perm, gcre_join_opts* opts) {
+  if (!ex || !paths0 || !paths1 || !out_scores || !n_scores || (!uids && n_uids) || (!signs && n_signs))
+    return fail(GCRE_ERR_ARG, "null argument");
+  if (paths0->ex != ex || paths1->ex != ex || (paths_res && paths_res->ex != ex)) return fail(GCRE_ERR_ARG, "path set belongs to another exec");
+  CKS(use_device(ex));
+  PhaseTrace tr;
+  // src/join_base.cpp:196: check_equal(uids.size(), paths0.size) - before any work on the index
+  if (n_uids != paths0->size) return fail(GCRE_ERR_ASSERT, "assertion");
+  gcre_uidset us;
+  int rc = build_uidset(ex, path_length, uids, n_uids, signs, n_signs, &us);
+  tr.mark("index");
+  if (rc == GCRE_OK) rc = join_impl(ex, &us, paths0, paths1, paths_res, top_k, out_scores, n_scores, out_perm, opts, tr);
+  if (rc == GCRE_OK) cudaStreamSynchronize(ex->stream);
+  free_uidset_buffers(&us);
+  return rc;
+}
+
+extern "C" int gcre_join_uidset(gcre_exec* ex, const gcre_uidset* uidset, const gcre_pathset* paths0, const gcre_pathset* paths1,
+                                gcre_pathset* paths_res, int top_k, gcre_score* out_scores, int* n_scores, double* out_perm,
+                                gcre_join_opts* opts) {
+  if (!ex || !uidset || !paths0 || !paths1 || !out_scores || !n_scores) return fail(GCRE_ERR_ARG, "null argument");
+  if (uidset->ex != ex) return fail(GCRE_ERR_ARG, "join index belongs to another exec");
+  CKS(use_device(ex));
+  PhaseTrace tr;
+  return join_impl(ex, uidset, paths0, paths1, paths_res, top_k, out_scores, n_scores, out_perm, opts, tr);
 }
 
 extern "C" int gcre_exec_device_perm_max(const gcre_exec* ex, void** device_ptr, int* n_floats) {

@@ -40,8 +40,6 @@
 // is half as long as the partner's.  s.tail1[loc] names that gene row and its orientation (base row << 1 | halves swapped);
 // off1 / len1 / car1 / ncase1 / pcnt1 then describe the base set.
 #pragma once
-#include <cstdlib>
-
 #include <cub/device/device_scan.cuh>
 
 #include "common.cuh"
@@ -804,10 +802,6 @@ __global__ void __launch_bounds__(sparse::THREADS, sparse::min_blocks(M, THR)) j
   if (!THR && pb_cur >= 0) flush_best(pb_cur);
 }
 
-// u32 carrier indices when n (which is also the sentinel index) does not fit u16; GCRE_TEST_WIDE_CARRIERS=1 (test hook)
-// forces the u32 path on small cohorts
-static inline bool sparse_wide(int n) { return n > 65535 || std::getenv("GCRE_TEST_WIDE_CARRIERS") != nullptr; }
-
 // can the sparse kernel run this shape at all: packed u16 counters, 32-bit row offsets into the patient-major masks
 static inline bool sparse_supported(int n, long long t_needed, int Iw) {
   return t_needed <= 65535 && ((unsigned long long)n + 1) * (unsigned long long)Iw < 0xffffffffull;
@@ -829,12 +823,10 @@ static inline double sparse_pair_ns(int n_perm_blocks, int M, double new_carrier
   return n_perm_blocks * ((M == 1 ? 1.5 : 2.0) + (M == 1 ? 0.075 : 0.1) * new_carriers_per_pair);
 }
 
-// Thresholded look-ups pay on large method-2 joins only (see the kernel); GCRE_THR=0 / 1 forces them off / on for every join
-static inline bool sparse_thr(int M, unsigned long long n_pairs) {
-  if (const char* e = std::getenv("GCRE_THR")) {
-    if (*e == '0' || *e == '1') return *e == '1';
-  }
-  return M == 2 && n_pairs >= (1ull << 20);
+// Thresholded look-ups pay on large method-2 joins only (see the kernel); forced = 0 / 1 (GCRE_THR) turns them off / on for
+// every join, -1 applies that rule
+static inline bool sparse_thr(int M, unsigned long long n_pairs, int forced) {
+  return forced >= 0 ? forced == 1 : M == 2 && n_pairs >= (1ull << 20);
 }
 
 template <int M, bool KEEP, bool PC, bool THR, bool TAIL = false>
@@ -843,37 +835,29 @@ static inline void launch_sparse_ct(unsigned grid, cudaStream_t stream, const Jo
   else join_sparse_kernel<M, KEEP, uint16_t, PC, THR, TAIL><<<grid, sparse::THREADS, 0, stream>>>(jp, sp);
 }
 
-template <int M, bool KEEP, bool THR>
-static inline void launch_sparse_pc(unsigned grid, cudaStream_t stream, const JoinParams& jp, const SparseParams& sp, bool wide) {
-  if constexpr (!KEEP) {
-    if (sp.tail1) {
-      launch_sparse_ct<M, false, true, THR, true>(grid, stream, jp, sp, wide);
-      return;
-    }
-  }
-  if (sp.pcnt1) launch_sparse_ct<M, KEEP, true, THR>(grid, stream, jp, sp, wide);
-  else launch_sparse_ct<M, KEEP, false, THR>(grid, stream, jp, sp, wide);
-}
-
 template <int M, bool THR>
-static inline void launch_sparse_keep(unsigned grid, cudaStream_t stream, const JoinParams& jp, const SparseParams& sp, bool wide, bool keep) {
-  if (keep) launch_sparse_pc<M, true, THR>(grid, stream, jp, sp, wide);
-  else launch_sparse_pc<M, false, THR>(grid, stream, jp, sp, wide);
+static inline void launch_sparse_form(unsigned grid, cudaStream_t stream, const JoinParams& jp, const SparseParams& sp, bool keep, bool pc, bool tail, bool wide) {
+  if (keep && pc) launch_sparse_ct<M, true, true, THR>(grid, stream, jp, sp, wide);
+  else if (keep) launch_sparse_ct<M, true, false, THR>(grid, stream, jp, sp, wide);
+  else if (tail) launch_sparse_ct<M, false, true, THR, true>(grid, stream, jp, sp, wide);  // (the tail form is score-only)
+  else if (pc) launch_sparse_ct<M, false, true, THR>(grid, stream, jp, sp, wide);
+  else launch_sparse_ct<M, false, false, THR>(grid, stream, jp, sp, wide);
 }
 
-// sp.pcnt1 != null selects the pre-counted-partner kernels (sp.tail1 != null as well: their tail form); `thr` the thresholded look-ups
-static inline cudaError_t launch_join_sparse(cudaStream_t stream, const JoinParams& jp, const SparseParams& sp, int M, bool keep, int sm_count, bool thr) {
+// `pc`: the pre-counted-partner kernels (sp.pcnt1 set); `tail`: their tail form (sp.tail1 set as well, never with `keep`);
+// `thr`: the thresholded look-ups; `wide`: u32 carrier indices
+static inline cudaError_t launch_join_sparse(cudaStream_t stream, const JoinParams& jp, const SparseParams& sp, int M, bool keep, int sm_count, bool pc,
+                                             bool tail, bool thr, bool wide) {
   const unsigned long long n_work = sp.n_units * (unsigned long long)sp.n_perm_blocks;
   if (n_work == 0) return cudaSuccess;
   const unsigned long long want = (n_work + sparse::WARPS - 1) / sparse::WARPS;
   const unsigned grid = (unsigned)std::min<unsigned long long>(want, (unsigned long long)sm_count * sparse::min_blocks(M, thr));
-  const bool wide = sparse_wide(sp.n);
   if (M == 1) {
-    if (thr) launch_sparse_keep<1, true>(grid, stream, jp, sp, wide, keep);
-    else launch_sparse_keep<1, false>(grid, stream, jp, sp, wide, keep);
+    if (thr) launch_sparse_form<1, true>(grid, stream, jp, sp, keep, pc, tail, wide);
+    else launch_sparse_form<1, false>(grid, stream, jp, sp, keep, pc, tail, wide);
   } else {
-    if (thr) launch_sparse_keep<2, true>(grid, stream, jp, sp, wide, keep);
-    else launch_sparse_keep<2, false>(grid, stream, jp, sp, wide, keep);
+    if (thr) launch_sparse_form<2, true>(grid, stream, jp, sp, keep, pc, tail, wide);
+    else launch_sparse_form<2, false>(grid, stream, jp, sp, keep, pc, tail, wide);
   }
   return cudaGetLastError();
 }
@@ -884,16 +868,13 @@ static inline cudaError_t launch_join_sparse(cudaStream_t stream, const JoinPara
 // delta / pre-counted: level 4 method 1 13.1 / 15.0, method 2 22.4 / 27.0), while at level 5 (two new genes per shared one)
 // and level 3 (single-gene partners, nothing shared) method 1 gains: 147 / 123 and 2.7 / 2.4; method 2, whose look-ups
 // dominate, does not (244 / 242, 5.8 / 5.8).  So: method 1, large score-only joins, and only when a sample of the pairs
-// (sample_overlap_kernel) shows the shared part below 0.6 of the new part.  GCRE_PRECOUNT=1 / 0 (GCRE_TEST_PRECOUNT in the
-// tests) forces it on / off.
+// (sample_overlap_kernel) shows the shared part below 0.6 of the new part.  `forced` (GCRE_PRECOUNT=1 / 0, GCRE_TEST_PRECOUNT
+// in the tests; -1: not set) forces it on / off, or with PRECOUNT_SAMPLE lets the sample decide whatever the method and the size.
 enum { PRECOUNT_NO = 0, PRECOUNT_YES = 1, PRECOUNT_SAMPLE = 2 };
-static inline int precount_mode(unsigned long long pairs, unsigned long long partner_rows, int M, int n_perm_blocks, size_t budget_bytes) {
+static inline int precount_mode(unsigned long long pairs, unsigned long long partner_rows, int M, int n_perm_blocks, size_t budget_bytes, int forced) {
   if (partner_rows == 0 || pairs == 0) return PRECOUNT_NO;
   if ((size_t)partner_rows * M * n_perm_blocks * 2048 > budget_bytes) return PRECOUNT_NO;
-  const char* f = std::getenv("GCRE_TEST_PRECOUNT");
-  if (!f) f = std::getenv("GCRE_PRECOUNT");
-  if (f && (*f == '0' || *f == '1')) return *f == '1' ? PRECOUNT_YES : PRECOUNT_NO;
-  if (f && *f == 's') return PRECOUNT_SAMPLE;  // test hook: let the sample decide whatever the method and the size
+  if (forced >= 0) return forced;
   return (M == 1 && pairs >= (1ull << 20)) ? PRECOUNT_SAMPLE : PRECOUNT_NO;
 }
 

@@ -579,34 +579,26 @@ __global__ void __launch_bounds__(PTS ? sparse_sc::PTS_THREADS : sparse_sc::THRE
   }
 }
 
-// few permutations, no pre-counted partners; GCRE_TEST_NO_SPLIT=1 (test hook) keeps the one-word-per-lane kernel
-static inline bool sparse_sc_enabled(int Ip, int n_perm_blocks) {
-  return Ip <= sparse_sc::MAX_PERMS && n_perm_blocks == 1 && std::getenv("GCRE_TEST_NO_SPLIT") == nullptr;
-}
-// words per lane group (4, 8, 16): also the tag of the count-table layout these kernels emit and consume
+// words per lane group (4, 8, 16): also the tag of the count-table layout these kernels emit and consume; pcnt0 / pcnt_res,
+// when set, must be in that layout (gcre_capi.cu tags every table with the layout it was emitted in)
 static inline int sparse_sc_words(int Ip) { return Ip <= 128 ? 4 : Ip <= 256 ? 8 : 16; }
 // bytes of one (row, half) entry of that table: 32 lanes x NW / 2 registers
 static inline size_t sparse_sc_table_bytes(int Ip) { return (size_t)32 * (sparse_sc_words(Ip) / 2) * 4; }
-// pcnt0 / pcnt_res, when set, must be in THIS layout (gcre_capi.cu tags every table with the layout it was emitted in)
-static inline bool sparse_sc_applies(const JoinParams& jp, const SparseParams& sp) {
-  return sparse_sc_enabled(jp.Ip, sp.n_perm_blocks) && !sp.pcnt1;
-}
 
 // PTS applies to <= 128 permutations when the matrix fits beside the CTA's static shared memory (queues, parked totals:
-// n <= ~12,400) and the launch has enough units to pay for staging it (160 KB per SM, ~10 us); GCRE_SC_PTS=0 / 1 (test hook)
-// forces it off / on where it fits
-static inline bool sparse_sc_pts_wanted(const JoinParams& jp, const SparseParams& sp, int sm_count) {
-  if (jp.Iw != 4 || sparse_wide(sp.n)) return false;
-  if (const char* e = std::getenv("GCRE_SC_PTS")) {
-    if (*e == '0' || *e == '1') return *e == '1';
-  }
+// n <= ~12,400) and the launch has enough units to pay for staging it (160 KB per SM, ~10 us); pts_forced = 0 / 1 (GCRE_SC_PTS,
+// a test hook; -1: not set) turns it off / on where it fits
+static inline bool sparse_sc_pts_wanted(const JoinParams& jp, const SparseParams& sp, int sm_count, bool wide, int pts_forced) {
+  if (jp.Iw != 4 || wide) return false;
+  if (pts_forced >= 0) return pts_forced == 1;
   return sp.n_units >= (unsigned long long)sm_count * (sparse_sc::PTS_THREADS / 32) * 4;
 }
 
 template <int M, bool KEEP, int NW>
-static inline cudaError_t launch_sparse_sc_ct(cudaStream_t stream, const JoinParams& jp, const SparseParams& sp, int sm_count, bool* pts) {
+static inline cudaError_t launch_sparse_sc_ct(cudaStream_t stream, const JoinParams& jp, const SparseParams& sp, int sm_count, bool wide, int pts_forced,
+                                              bool* pts) {
   if constexpr (NW == 4) {
-    if (sparse_sc_pts_wanted(jp, sp, sm_count)) {
+    if (sparse_sc_pts_wanted(jp, sp, sm_count, wide, pts_forced)) {
       constexpr int warps = sparse_sc::PTS_THREADS / 32;
       auto kern = join_sparse_sc_kernel<M, KEEP, uint16_t, 4, true>;
       static int static_smem[64];  // per instantiation and device: static shared memory of the kernel, 0 = not asked yet
@@ -634,24 +626,29 @@ static inline cudaError_t launch_sparse_sc_ct(cudaStream_t stream, const JoinPar
   }
   const unsigned long long want = (sp.n_units + sparse_sc::WARPS - 1) / sparse_sc::WARPS;
   const unsigned grid = (unsigned)std::min<unsigned long long>(want, (unsigned long long)sm_count * sparse_sc::min_blocks(NW));
-  if (sparse_wide(sp.n)) join_sparse_sc_kernel<M, KEEP, uint32_t, NW, false><<<grid, sparse_sc::THREADS, 0, stream>>>(jp, sp);
+  if (wide) join_sparse_sc_kernel<M, KEEP, uint32_t, NW, false><<<grid, sparse_sc::THREADS, 0, stream>>>(jp, sp);
   else join_sparse_sc_kernel<M, KEEP, uint16_t, NW, false><<<grid, sparse_sc::THREADS, 0, stream>>>(jp, sp);
   return cudaGetLastError();
 }
 
 template <int M, bool KEEP>
-static inline cudaError_t launch_sparse_sc_nw(cudaStream_t stream, const JoinParams& jp, const SparseParams& sp, int sm_count, bool* pts) {
+static inline cudaError_t launch_sparse_sc_nw(cudaStream_t stream, const JoinParams& jp, const SparseParams& sp, int sm_count, bool wide, int pts_forced,
+                                              bool* pts) {
   const int nw = sparse_sc_words(jp.Ip);
-  if (nw == 4) return launch_sparse_sc_ct<M, KEEP, 4>(stream, jp, sp, sm_count, pts);
-  if (nw == 8) return launch_sparse_sc_ct<M, KEEP, 8>(stream, jp, sp, sm_count, pts);
-  return launch_sparse_sc_ct<M, KEEP, 16>(stream, jp, sp, sm_count, pts);
+  if (nw == 4) return launch_sparse_sc_ct<M, KEEP, 4>(stream, jp, sp, sm_count, wide, pts_forced, pts);
+  if (nw == 8) return launch_sparse_sc_ct<M, KEEP, 8>(stream, jp, sp, sm_count, wide, pts_forced, pts);
+  return launch_sparse_sc_ct<M, KEEP, 16>(stream, jp, sp, sm_count, wide, pts_forced, pts);
 }
 
-// *pts is set when the shared-memory form was launched
-static inline cudaError_t launch_join_sparse_sc(cudaStream_t stream, const JoinParams& jp, const SparseParams& sp, int M, bool keep, int sm_count, bool* pts) {
+// `wide`: u32 carrier indices; *pts is set when the shared-memory form was launched
+static inline cudaError_t launch_join_sparse_sc(cudaStream_t stream, const JoinParams& jp, const SparseParams& sp, int M, bool keep, int sm_count, bool wide,
+                                                int pts_forced, bool* pts) {
   if (sp.n_units == 0) return cudaSuccess;
-  if (M == 1) return keep ? launch_sparse_sc_nw<1, true>(stream, jp, sp, sm_count, pts) : launch_sparse_sc_nw<1, false>(stream, jp, sp, sm_count, pts);
-  return keep ? launch_sparse_sc_nw<2, true>(stream, jp, sp, sm_count, pts) : launch_sparse_sc_nw<2, false>(stream, jp, sp, sm_count, pts);
+  if (M == 1)
+    return keep ? launch_sparse_sc_nw<1, true>(stream, jp, sp, sm_count, wide, pts_forced, pts)
+                : launch_sparse_sc_nw<1, false>(stream, jp, sp, sm_count, wide, pts_forced, pts);
+  return keep ? launch_sparse_sc_nw<2, true>(stream, jp, sp, sm_count, wide, pts_forced, pts)
+              : launch_sparse_sc_nw<2, false>(stream, jp, sp, sm_count, wide, pts_forced, pts);
 }
 
 }  // namespace gcre
