@@ -379,7 +379,7 @@ struct gcre_exec {
 struct Provenance {
   const gcre_pathset* base = nullptr;
   unsigned long long base_uid = 0, base_ver = 0;  // the base set's identity and version when the entries were made
-  int32_t* sel = nullptr;      // gcre_pathset_select: row k is base row sel[k]
+  uint32_t* sel = nullptr;     // gcre_pathset_select: row k is base row sel[k] >> 1 (entries, halves as they are)
   uint32_t* tail = nullptr;    // KEEP join result: per row, its partner's base row (the path's last gene)
   uint32_t* head = nullptr;    // ... and its upstream row's entry when every upstream row was exactly one base row (else null)
   unsigned long long lo = 0, hi = 0;  // rows [lo, hi) carry entries (a sharded join writes only its rows)
@@ -1278,10 +1278,13 @@ extern "C" int gcre_pathset_select(const gcre_pathset* ps, const int32_t* indice
                                                                                        row_vec, (ulonglong2*)res->d_rows);
       CK(cudaGetLastError());
       LAUNCHED();
-      // the selection remembers its rows' origin (a KEEP join with it as partner records which base row each result row adds)
+      // the selection remembers its rows' origin (a KEEP join with it as partner scores its rows through the base set's, and
+      // records which base row each result row adds)
       if (ps->size <= 0x7fffffffu && provenance_useful(ex)) {
         CK(dev_alloc(ex, (void**)&res->prov.sel, (size_t)n * 4));
-        CK(cudaMemcpyAsync(res->prov.sel, ex->scratch.p, (size_t)n * 4, cudaMemcpyDeviceToDevice, ex->stream));
+        selection_entries_kernel<<<grid_for((long long)n, 256), 256, 0, ex->stream>>>((const int32_t*)ex->scratch.p, n, res->prov.sel);
+        CK(cudaGetLastError());
+        LAUNCHED();
         res->prov.base = ps;
         res->prov.base_uid = ps->uid;
         res->prov.base_ver = ps->ver;
@@ -1808,7 +1811,8 @@ struct JoinForm {
   int kernel = GCRE_KERNEL_DENSE;
   bool split = false;                        // the split-carrier kernels (join_sparse_sc.cuh)
   bool precount = false;                     // pre-counted partners (PC kernels of join_sparse.cuh)
-  const gcre_pathset* tail_base = nullptr;   // tail form: partners scored through this set's gene rows (PC + TAIL kernels)
+  const gcre_pathset* tail_base = nullptr;   // partners scored through this set's rows (PC + TAIL kernels): the tail form, or ...
+  bool selected = false;                     // ... with `precount`, a KEEP join whose partners are a selection of this set
   bool emit = false;                         // kept rows take their counts along
   bool base_emitted = false;                 // the upstream rows carry counts and totals from the join that made them
   bool thr = false;                          // thresholded look-ups
@@ -1883,7 +1887,13 @@ static int choose_join_form(const JoinCall& c, int requested, long long t_needed
     if (want) CKS(tail_form_base(ex, c.us, c.paths0, c.paths1, c.ub, c.ue, &f->tail_base));
     if (f->tail_base && (size_t)f->tail_base->size * ex->M * npb * 2048 > budget) f->tail_base = nullptr;
   }
-  int pc_mode = f->tail_base ? PRECOUNT_NO : precount_mode(pairs, c.paths1->size, ex->M, npb, budget, c.knobs.precount);
+  // A KEEP join whose partner set is a live selection of a base set (level 3: data1's gene rows) may score its partners through
+  // the base set's rows and pre-counted table (join_sparse.cuh): a selected row is its base row, so no eligibility pass
+  const Provenance& sel = c.paths1->prov;
+  const gcre_pathset* sel_base = c.keep && !ex->split_ok && sel.sel && base_current(ex, sel) ? sel.base : nullptr;
+  int pc_mode = f->tail_base ? PRECOUNT_NO
+                : sel_base   ? precount_mode(pairs, sel_base->size, ex->M, npb, budget, c.knobs.precount, true)
+                             : precount_mode(pairs, c.paths1->size, ex->M, npb, budget, c.knobs.precount, false);
   if (ex->split_ok && pc_mode == PRECOUNT_SAMPLE) pc_mode = PRECOUNT_NO;  // the split-carrier kernel is the better form there
   // <= 512 permutations: the split-carrier kernels (join_sparse_sc.cuh) run - unless pre-counted partners are forced
   // (GCRE_PRECOUNT=1) - and emit / consume count tables in their own, smaller layout
@@ -1899,7 +1909,9 @@ static int choose_join_form(const JoinCall& c, int requested, long long t_needed
   // counts (res_is_prefix: rows [pair_lo, pair_hi) are exactly the ones this call writes)
   f->emit = (f->split || !ex->split_ok) && c.keep && pairs > 0 && c.us->res_is_prefix && c.paths_res != c.paths0 && c.paths_res != c.paths1 &&
             !c.knobs.no_emit && (size_t)c.paths_res->size * ex->M * f->entry_bytes <= budget;
-  if (f->emit && !f->split) pc_mode = PRECOUNT_NO;  // the emitting form of the 1,024-permutation kernel has no pre-counted variant
+  // unforced, an emitting join pre-counts only through a selection's base set (a table of the partner set itself would be built
+  // for this one join)
+  if (f->emit && !f->split && !sel_base && c.knobs.precount < 0) pc_mode = PRECOUNT_NO;
   if (pc_mode == PRECOUNT_SAMPLE) {
     // how much of a partner row is already in its upstream row
     unsigned long long sums[2];
@@ -1907,6 +1919,10 @@ static int choose_join_form(const JoinCall& c, int requested, long long t_needed
     pc_mode = (sums[0] * 10 < sums[1] * 6) ? PRECOUNT_YES : PRECOUNT_NO;
   }
   f->precount = pc_mode == PRECOUNT_YES;
+  if (f->precount && sel_base) {
+    f->tail_base = sel_base;
+    f->selected = true;
+  }
   return GCRE_OK;
 }
 
@@ -1926,7 +1942,7 @@ static int prepare_join_operands(const JoinCall& c, const JoinForm& f, JoinParam
     sp->pcnt0 = f.base_emitted ? p0->view.pcnt : nullptr;
     sp->off1 = p1->view.off; sp->len1 = p1->view.len; sp->car1 = p1->view.car; sp->ncase1 = p1->view.ncase;
     sp->pcnt1 = (f.precount || f.tail_base) ? p1->view.pcnt : nullptr;
-    sp->tail1 = f.tail_base ? c.paths1->prov.tail : nullptr;
+    sp->tail1 = f.selected ? c.paths1->prov.sel : f.tail_base ? c.paths1->prov.tail : nullptr;
     sp->n = ex->n;
     sp->unit_prefix = (const unsigned long long*)c.us->units.p;
     sp->unit_idx = (const uint32_t*)c.us->unit_idx.p;
@@ -2204,7 +2220,7 @@ static int join_impl(gcre_exec* ex, const gcre_uidset* us, const gcre_pathset* p
     opts->kernel_used = form.kernel;
     opts->launches = st.launches;
     opts->precounted = form.precount;
-    opts->tail_form = form.tail_base != nullptr;
+    opts->tail_form = form.tail_base != nullptr && !form.selected;
     opts->split_carrier = form.split;
     opts->shared_masks = st.shared_masks;
     opts->thresholded = form.thr && st.launches > 0 ? 1 : 0;

@@ -39,6 +39,12 @@
 // up & t is a fraction of a carrier for rare-variant rows, P over the few thousand gene rows fits in L2, and the gene's list
 // is half as long as the partner's.  s.tail1[loc] names that gene row and its orientation (base row << 1 | halves swapped);
 // off1 / len1 / car1 / ncase1 / pcnt1 then describe the base set.
+//
+// The same mapping scores a partner set that is a selection of a base set (gcre_pathset_select: level 3's partners are copies
+// of data1's gene rows): s.tail1 is then the selection's own entries (base row << 1, halves as they are), and the partner is
+// scored through its base row's carrier list and pre-counted row - no lists of the copy, and one table shared with level 4.
+// That form keeps its rows (KEEP): it emits the final base + P - overlap counts in the same register image the delta form
+// emits, so the next level cannot tell which form made them.
 #pragma once
 #include <cub/device/device_scan.cuh>
 
@@ -294,10 +300,10 @@ __device__ __forceinline__ void prefetch_l1(const void* p) { asm volatile("prefe
 
 // CT = carrier index type of the list views: uint16_t (n <= 65,535) or uint32_t
 // THR: thresholded look-ups (below) instead of 32 running maxima per lane in registers
-// TAIL (with PC, score-only): partners are scored through the base-set gene row s.tail1 names (see the header)
+// TAIL (with PC): partners are scored through the base-set row s.tail1 names (see the header)
 template <int M, bool KEEP, typename CT, bool PC, bool THR, bool TAIL = false>
 __global__ void __launch_bounds__(sparse::THREADS, sparse::min_blocks(M, THR)) join_sparse_kernel(const JoinParams a, const SparseParams s) {
-  static_assert(!TAIL || (PC && !KEEP), "the tail form is a score-only pre-counted form");
+  static_assert(!TAIL || PC, "the tail mapping is a pre-counted form");
   using namespace sparse;
   const CT* car0 = static_cast<const CT*>(s.car0);
   const CT* car1 = static_cast<const CT*>(s.car1);
@@ -552,7 +558,12 @@ __global__ void __launch_bounds__(sparse::THREADS, sparse::min_blocks(M, THR)) j
 
       bool empty = nd[0] == 0;
       if (M == 2) empty = empty && nd[M - 1] == 0;
-      if (!empty || !base_done) {
+      // KEEP + PC: the final counts formed below are the kept row's emitted counts (a partner skipped as empty has the base's);
+      // with running maxima they are stored where they are formed, at emit_at
+      const bool scored = !empty || !base_done;
+      uint4* emit_at = nullptr;
+      if (KEEP && PC && !THR && s.pcnt_res) emit_at = reinterpret_cast<uint4*>(s.pcnt_res) + ((((size_t)(a.res_idx[idx] + j) * M) * s.n_perm_blocks + pb) * 4) * 32 + lane;
+      if (scored) {
         if (empty) base_done = true;
         if constexpr (THR) {
           if (PC) {
@@ -636,13 +647,15 @@ __global__ void __launch_bounds__(sparse::THREADS, sparse::min_blocks(M, THR)) j
               for (int q = 0; q < 4; q++) {
                 const uint4 pv = __ldg(P0 + q * 32);
                 const uint32_t pr[4] = {pv.x, pv.y, pv.z, pv.w};
+                uint32_t v[4];
 #pragma unroll
                 for (int k = 0; k < 4; k++) {
                   const int i = 4 * q + k;
-                  const uint32_t v = s_base[0][i][tid] + pr[k] - c16[i];
-                  best[((i & 1) * 2) * 8 + (i >> 1)] = fmaxf(best[((i & 1) * 2) * 8 + (i >> 1)], lookup_f32(row, v & 0xffffu));
-                  best[((i & 1) * 2 + 1) * 8 + (i >> 1)] = fmaxf(best[((i & 1) * 2 + 1) * 8 + (i >> 1)], lookup_f32(row, v >> 16));
+                  v[k] = s_base[0][i][tid] + pr[k] - c16[i];
+                  best[((i & 1) * 2) * 8 + (i >> 1)] = fmaxf(best[((i & 1) * 2) * 8 + (i >> 1)], lookup_f32(row, v[k] & 0xffffu));
+                  best[((i & 1) * 2 + 1) * 8 + (i >> 1)] = fmaxf(best[((i & 1) * 2 + 1) * 8 + (i >> 1)], lookup_f32(row, v[k] >> 16));
                 }
+                if (KEEP && emit_at) __stcs(emit_at + q * 32, make_uint4(v[0], v[1], v[2], v[3]));
               }
             } else {
               const uint4* P1 = reinterpret_cast<const uint4*>(s.pcnt1) + ((pitem[M - 1] * s.n_perm_blocks + pb) * 4) * 32 + lane;
@@ -653,16 +666,21 @@ __global__ void __launch_bounds__(sparse::THREADS, sparse::min_blocks(M, THR)) j
               for (int q = 0; q < 4; q++) {
                 const uint4 pvp = __ldg(P0 + q * 32), pvn = __ldg(P1 + q * 32);
                 const uint32_t prp[4] = {pvp.x, pvp.y, pvp.z, pvp.w}, prn[4] = {pvn.x, pvn.y, pvn.z, pvn.w};
+                uint32_t vp[4], vn[4];
 #pragma unroll
                 for (int k = 0; k < 4; k++) {
                   const int i = 4 * q + k;
-                  const uint32_t vp = s_base[0][i][tid] + prp[k] - s_cnt[0][M == 2 ? i : 0][tid];
-                  const uint32_t vn = s_base[M - 1][i][tid] + prn[k] - s_cnt[M == 2 ? 1 : 0][M == 2 ? i : 0][tid];
+                  vp[k] = s_base[0][i][tid] + prp[k] - s_cnt[0][M == 2 ? i : 0][tid];
+                  vn[k] = s_base[M - 1][i][tid] + prn[k] - s_cnt[M == 2 ? 1 : 0][M == 2 ? i : 0][tid];
                   // src/methods.h:223-227: vtmax[pcp][total_pos - pcp] + vtmax[total_neg - pnp][pnp]
-                  const double vlo = lookup_f64(rowp, vp & 0xffffu) + lookup_f64(rown, tn - (vn & 0xffffu));
-                  const double vhi = lookup_f64(rowp, vp >> 16) + lookup_f64(rown, tn - (vn >> 16));
+                  const double vlo = lookup_f64(rowp, vp[k] & 0xffffu) + lookup_f64(rown, tn - (vn[k] & 0xffffu));
+                  const double vhi = lookup_f64(rowp, vp[k] >> 16) + lookup_f64(rown, tn - (vn[k] >> 16));
                   best[((i & 1) * 2) * 8 + (i >> 1)] = fmaxf(best[((i & 1) * 2) * 8 + (i >> 1)], __double2float_rn(vlo));
                   best[((i & 1) * 2 + 1) * 8 + (i >> 1)] = fmaxf(best[((i & 1) * 2 + 1) * 8 + (i >> 1)], __double2float_rn(vhi));
+                }
+                if (KEEP && emit_at) {  // halves 0 and 1 of the kept row, n_perm_blocks * 128 uint4 apart
+                  __stcs(emit_at + q * 32, make_uint4(vp[0], vp[1], vp[2], vp[3]));
+                  __stcs(emit_at + (size_t)s.n_perm_blocks * 128 + q * 32, make_uint4(vn[0], vn[1], vn[2], vn[3]));
                 }
               }
             }
@@ -692,17 +710,22 @@ __global__ void __launch_bounds__(sparse::THREADS, sparse::min_blocks(M, THR)) j
         }
       }
 
-      if (KEEP && !PC && s.pcnt_res) {
+      if (KEEP && s.pcnt_res) {
         // ---- the kept row's counts and carrier totals travel with it (base of the next level) ----
+        // (PC with running maxima stored its final counts beside the look-ups already)
         const size_t r = (size_t)(a.res_idx[idx] + j);
 #pragma unroll
         for (int h = 0; h < M; h++) {
-          uint4* out = reinterpret_cast<uint4*>(s.pcnt_res) + (((r * M + h) * s.n_perm_blocks + pb) * 4) * 32 + lane;
-          uint32_t v16[16];  // method 1 / THR: the last half is in registers; method 2: parked halves in shared memory
+          if (!(PC && !THR && scored)) {
+            uint4* out = reinterpret_cast<uint4*>(s.pcnt_res) + (((r * M + h) * s.n_perm_blocks + pb) * 4) * 32 + lane;
+            uint32_t v16[16];  // method 1 / THR: the last half is in registers; method 2: parked halves in shared memory
 #pragma unroll
-          for (int i = 0; i < 16; i++) v16[i] = (M == 1 || (THR && h == M - 1)) ? c16[i] : s_cnt[(M == 2 && !THR) ? h : 0][M == 2 ? i : 0][tid];
+            for (int i = 0; i < 16; i++)
+              v16[i] = (PC && !scored) ? s_base[h][i][tid]
+                                       : (M == 1 || (THR && h == M - 1)) ? c16[i] : s_cnt[(M == 2 && !THR) ? h : 0][M == 2 ? i : 0][tid];
 #pragma unroll
-          for (int q = 0; q < 4; q++) __stcs(out + q * 32, make_uint4(v16[4 * q], v16[4 * q + 1], v16[4 * q + 2], v16[4 * q + 3]));
+            for (int q = 0; q < 4; q++) __stcs(out + q * 32, make_uint4(v16[4 * q], v16[4 * q + 1], v16[4 * q + 2], v16[4 * q + 3]));
+          }
           if (first_pb && lane == 0) {
             s.len_res[r * M + h] = t0[h == 0 ? 0 : M - 1] + nd[h == 0 ? 0 : M - 1];
             s.ncase_res[r * M + h] = nc0[h == 0 ? 0 : M - 1] + ncn[h == 0 ? 0 : M - 1];
@@ -837,14 +860,16 @@ static inline void launch_sparse_ct(unsigned grid, cudaStream_t stream, const Jo
 
 template <int M, bool THR>
 static inline void launch_sparse_form(unsigned grid, cudaStream_t stream, const JoinParams& jp, const SparseParams& sp, bool keep, bool pc, bool tail, bool wide) {
-  if (keep && pc) launch_sparse_ct<M, true, true, THR>(grid, stream, jp, sp, wide);
+  if (keep && tail) launch_sparse_ct<M, true, true, THR, true>(grid, stream, jp, sp, wide);  // (a selection's partners)
+  else if (keep && pc) launch_sparse_ct<M, true, true, THR>(grid, stream, jp, sp, wide);
   else if (keep) launch_sparse_ct<M, true, false, THR>(grid, stream, jp, sp, wide);
-  else if (tail) launch_sparse_ct<M, false, true, THR, true>(grid, stream, jp, sp, wide);  // (the tail form is score-only)
+  else if (tail) launch_sparse_ct<M, false, true, THR, true>(grid, stream, jp, sp, wide);
   else if (pc) launch_sparse_ct<M, false, true, THR>(grid, stream, jp, sp, wide);
   else launch_sparse_ct<M, false, false, THR>(grid, stream, jp, sp, wide);
 }
 
-// `pc`: the pre-counted-partner kernels (sp.pcnt1 set); `tail`: their tail form (sp.tail1 set as well, never with `keep`);
+// `pc`: the pre-counted-partner kernels (sp.pcnt1 set); `tail`: partners read through sp.tail1 (the tail form, or with `keep` a
+// selection's partners);
 // `thr`: the thresholded look-ups; `wide`: u32 carrier indices
 static inline cudaError_t launch_join_sparse(cudaStream_t stream, const JoinParams& jp, const SparseParams& sp, int M, bool keep, int sm_count, bool pc,
                                              bool tail, bool thr, bool wide) {
@@ -868,13 +893,23 @@ static inline cudaError_t launch_join_sparse(cudaStream_t stream, const JoinPara
 // delta / pre-counted: level 4 method 1 13.1 / 15.0, method 2 22.4 / 27.0), while at level 5 (two new genes per shared one)
 // and level 3 (single-gene partners, nothing shared) method 1 gains: 147 / 123 and 2.7 / 2.4; method 2, whose look-ups
 // dominate, does not (244 / 242, 5.8 / 5.8).  So: method 1, large score-only joins, and only when a sample of the pairs
-// (sample_overlap_kernel) shows the shared part below 0.6 of the new part.  `forced` (GCRE_PRECOUNT=1 / 0, GCRE_TEST_PRECOUNT
-// in the tests; -1: not set) forces it on / off, or with PRECOUNT_SAMPLE lets the sample decide whatever the method and the size.
+// (sample_overlap_kernel) shows the shared part below 0.6 of the new part.
+// KEEP joins whose partners are a selection (levels 2 and 3: single gene rows) are scored through the base set's rows and table
+// and emit their counts (see the header).  Measured on B200 (BASELINE config 3, delta -> this form, ms per join, methods 1 / 2):
+// level 2 (150 k pairs) 0.72 -> 0.64 / 0.90 -> 0.85, level 3 (1.35 M pairs) 2.24 -> 2.11 / 3.91 -> 4.06 (thresholded look-ups);
+// the step also loses the carrier lists of the two partner copies (~0.3 / 0.5 ms of list builds per method): 31.0 -> 30.2 ms
+// per step (profiles/r5_selection_ab.txt).  So: such joins of >= 128 K pairs, either method, when the sample agrees.
+// `forced` (GCRE_PRECOUNT=1 / 0, GCRE_TEST_PRECOUNT in the tests; -1: not set) forces it on / off for every join (KEEP joins
+// included), or with PRECOUNT_SAMPLE lets the sample decide whatever the method and the size.
 enum { PRECOUNT_NO = 0, PRECOUNT_YES = 1, PRECOUNT_SAMPLE = 2 };
-static inline int precount_mode(unsigned long long pairs, unsigned long long partner_rows, int M, int n_perm_blocks, size_t budget_bytes, int forced) {
-  if (partner_rows == 0 || pairs == 0) return PRECOUNT_NO;
-  if ((size_t)partner_rows * M * n_perm_blocks * 2048 > budget_bytes) return PRECOUNT_NO;
+// `table_rows`: rows of the set the table is built over (the partner set, or the base set of a selection partner)
+// `kept_selection`: a KEEP join whose partners are a selection, scored through the base set (SELECTION_MIN_PAIRS below)
+static inline int precount_mode(unsigned long long pairs, unsigned long long table_rows, int M, int n_perm_blocks, size_t budget_bytes, int forced,
+                                bool kept_selection) {
+  if (table_rows == 0 || pairs == 0) return PRECOUNT_NO;
+  if ((size_t)table_rows * M * n_perm_blocks * 2048 > budget_bytes) return PRECOUNT_NO;
   if (forced >= 0) return forced;
+  if (kept_selection) return pairs >= (1ull << 17) ? PRECOUNT_SAMPLE : PRECOUNT_NO;
   return (M == 1 && pairs >= (1ull << 20)) ? PRECOUNT_SAMPLE : PRECOUNT_NO;
 }
 

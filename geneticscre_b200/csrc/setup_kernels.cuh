@@ -235,11 +235,11 @@ __global__ void finish_uids_kernel(uint32_t n, const int32_t* __restrict__ count
 // Entries name a row of a base path set and its orientation: base row << 1 | 1 when the row's halves are swapped (method 2:
 // joined half h holds base half 1 - h).  A KEEP join whose partner set is a selection of the base set records, per result
 // row it writes, the partner's base row (`tail`) and - when every upstream row is exactly one oriented base row - the
-// upstream row's entry (`head`).  One thread per upstream row of [ub, ue).
+// upstream row's entry (`head`).  One thread per upstream row of [ub, ue).  `sel`: the selection's own entries (below).
 template <int M>
 __global__ void record_rows_kernel(uint32_t ub, uint32_t ue, const int32_t* __restrict__ count, const uint32_t* __restrict__ location,
                                    const unsigned long long* __restrict__ res_idx, const int32_t* __restrict__ signs, int path_length,
-                                   const int32_t* __restrict__ sel_idx, const uint32_t* __restrict__ tail0, uint32_t* __restrict__ tail_res,
+                                   const uint32_t* __restrict__ sel, const uint32_t* __restrict__ tail0, uint32_t* __restrict__ tail_res,
                                    uint32_t* __restrict__ head_res) {
   const uint32_t idx = ub + blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= ue) return;
@@ -249,9 +249,15 @@ __global__ void record_rows_kernel(uint32_t ub, uint32_t ue, const int32_t* __re
     const uint32_t loc = location[idx] + (uint32_t)j;
     const unsigned long long r = res_idx[idx] + (unsigned long long)j;
     const bool swap = (M == 2) && !need_flip(path_length, signs, idx, loc);  // src/methods.h:137-145: partner half 1 - h joins half h
-    tail_res[r] = ((uint32_t)sel_idx[loc] << 1) | (swap ? 1u : 0u);
+    tail_res[r] = sel[loc] | (swap ? 1u : 0u);
     if (head_res) head_res[r] = head;
   }
+}
+
+// The entries of a selection (gcre_pathset_select): row k is base row idx[k], halves as they are
+__global__ void selection_entries_kernel(const int32_t* __restrict__ idx, uint32_t n, uint32_t* __restrict__ sel) {
+  const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
+  if (k < n) sel[k] = (uint32_t)idx[k] << 1;
 }
 
 // Does every pair of upstream rows [ub, ue) meet the tail form's condition: the partner's head, oriented as the pair joins it,

@@ -1,5 +1,6 @@
-# kernel times of one level schedule (bench workload) per method under torch.profiler: P build of data1, eligibility pass,
-# provenance recording, level-4 join
+# kernel times and launch counts of one level schedule (bench workload) per method under torch.profiler, every kernel: carrier-list
+# builds (half_popcount / build_lists), P build of data1, eligibility pass, provenance recording, level-3 and level-4 joins.
+# Run from the root of the tree whose build is measured.
 import json, os, sys
 sys.path.insert(0, os.getcwd())
 import torch
@@ -25,6 +26,7 @@ for method in ("method1", "method2"):
             a = agg.setdefault(k, [0, 0.0])
             a[0] += 1
             a[1] += e.device_time_total / 1000.0 if hasattr(e, "device_time_total") else e.cuda_time_total / 1000.0
-    out[method] = {"level4_info": res["4"].info, "kernels_ms": {k: v for k, v in sorted(agg.items(), key=lambda kv: -kv[1][1])[:20]}}
+    out[method] = {"level3_info": res["3"].info, "level4_info": res["4"].info,
+                   "kernels_ms": {k: v for k, v in sorted(agg.items(), key=lambda kv: -kv[1][1])}}
     ex.close()
 print(json.dumps(out, indent=1))
