@@ -82,6 +82,10 @@ SYMBOLS = {
     "gcre_exec_import_perm_max": (_I, [_VP, _VP, _I]),
     "gcre_exec_read_perm_max": (_I, [_VP, C.POINTER(C.c_double)]),
     "gcre_merge_topk": (_I, [C.POINTER(ScoreC), C.POINTER(_I), _I, _I, C.POINTER(ScoreC), C.POINTER(_I)]),
+    # test and diagnostics only
+    "gcre_pathset_debug_view_info": (_I, [_VP, C.POINTER(C.c_int64)]),
+    "gcre_pathset_debug_counts": (_I, [_VP, C.POINTER(C.c_uint16), C.POINTER(_U32), C.POINTER(_U32)]),
+    "gcre_pathset_debug_lists": (_I, [_VP, C.POINTER(C.c_uint64), C.POINTER(_U32), C.POINTER(_U32), C.POINTER(_U32)]),
 }
 
 _lib = None

@@ -147,6 +147,30 @@ class PathSet:
         check(self.ex._lib.gcre_pathset_download(self._h, _ptr(out, C.c_uint64)))
         return out
 
+    def debug_view(self):
+        """The sparse kernels' state of this set, read back for tests and diagnostics (include/gcre_b200.h, gcre_pathset_debug_*):
+        ``{"lists": {off, len, ncase, car} or None, "table": {counts [rows][method][iters_requested] uint16, len, ncase
+        [rows][method], lo, hi, layout, current} or None, "stats_valid": bool}``."""
+        lib, m = self.ex._lib, self.ex.m
+        info = np.zeros(8, dtype=np.int64)
+        check(lib.gcre_pathset_debug_view_info(self._h, _ptr(info, C.c_int64)))
+        lists = table = None
+        if info[0]:
+            items = self.size * m
+            off = np.zeros(items + 1, dtype=np.uint64)
+            ln, nc = np.zeros(max(items, 1), dtype=np.uint32), np.zeros(max(items, 1), dtype=np.uint32)
+            car = np.zeros(max(int(info[1]), 1), dtype=np.uint32)
+            check(lib.gcre_pathset_debug_lists(self._h, _ptr(off, C.c_uint64), _ptr(ln, C.c_uint32), _ptr(nc, C.c_uint32), _ptr(car, C.c_uint32)))
+            lists = {"off": off, "len": ln[:items].reshape(self.size, m), "ncase": nc[:items].reshape(self.size, m), "car": car[: int(info[1])]}
+        if info[3]:
+            lo, hi = int(info[6]), int(info[7])
+            counts = np.zeros((max(hi - lo, 1), m, max(self.ex.iters_requested, 1)), dtype=np.uint16)
+            ln, nc = np.zeros((max(hi - lo, 1), m), dtype=np.uint32), np.zeros((max(hi - lo, 1), m), dtype=np.uint32)
+            check(lib.gcre_pathset_debug_counts(self._h, _ptr(counts, C.c_uint16), _ptr(ln, C.c_uint32), _ptr(nc, C.c_uint32)))
+            table = {"counts": counts[: hi - lo, :, : self.ex.iters_requested], "len": ln[: hi - lo], "ncase": nc[: hi - lo], "lo": lo, "hi": hi,
+                     "layout": int(info[4]), "current": bool(info[5])}
+        return {"lists": lists, "table": table, "stats_valid": bool(info[2])}
+
 
 class JoinExec:
     """JoinExec (src/gcre.h:103-180).  ``nthreads`` is accepted and ignored (the join runs on the GPU)."""

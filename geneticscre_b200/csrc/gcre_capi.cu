@@ -1366,6 +1366,79 @@ extern "C" int gcre_pathset_download(const gcre_pathset* ps, uint64_t* out) {
 }
 
 // ------------------------------------------------------------------------------------------------------------------
+// read-backs of a path set's sparse view (tests and diagnostics only; nothing calls them on the join path)
+// ------------------------------------------------------------------------------------------------------------------
+extern "C" int gcre_pathset_debug_view_info(const gcre_pathset* ps, int64_t* out) {
+  if (!ps || !out) return fail(GCRE_ERR_ARG, "null argument");
+  LIVE(ps);
+  const gcre_exec* ex = ps->ex;
+  CKS(use_device(ex));
+  const SparseView& v = ps->view;
+  uint64_t entries = 0;
+  if (v.valid) {
+    CK(cudaMemcpyAsync(&entries, v.off + (size_t)ps->size * ex->M, 8, cudaMemcpyDeviceToHost, ex->stream));
+    CK(cudaStreamSynchronize(ex->stream));
+  }
+  const bool table = v.pcnt != nullptr;
+  const int64_t info[8] = {v.valid, (int64_t)entries, v.stats_valid, table, table ? v.pcnt_layout : 0, table && v.pcnt_gen == ex->mask_gen,
+                           table ? (int64_t)v.emit_lo : 0, table ? (int64_t)v.emit_hi : 0};
+  memcpy(out, info, sizeof info);
+  return GCRE_OK;
+}
+
+extern "C" int gcre_pathset_debug_counts(const gcre_pathset* ps, uint16_t* counts, uint32_t* len, uint32_t* ncase) {
+  if (!ps) return fail(GCRE_ERR_ARG, "null argument");
+  LIVE(ps);
+  const gcre_exec* ex = ps->ex;
+  CKS(use_device(ex));
+  const SparseView& v = ps->view;
+  if (!v.pcnt) return fail(GCRE_ERR_ASSERT, "the path set holds no count table");
+  const size_t lo = (size_t)v.emit_lo, items = ((size_t)v.emit_hi - lo) * ex->M;
+  if (items && !counts) return fail(GCRE_ERR_ARG, "null argument");
+  const size_t entry_words = (v.pcnt_layout == 0 ? (size_t)(ex->Iw / 32) * 2048 : sparse_sc_table_bytes(ex->Ip)) / 4;
+  std::vector<uint32_t> raw(items * entry_words);
+  if (items) CK(cudaMemcpyAsync(raw.data(), v.pcnt + lo * ex->M * entry_words, raw.size() * 4, cudaMemcpyDeviceToHost, ex->stream));
+  if (items && len && v.len) CK(cudaMemcpyAsync(len, v.len + lo * ex->M, items * 4, cudaMemcpyDeviceToHost, ex->stream));
+  if (items && ncase && v.ncase) CK(cudaMemcpyAsync(ncase, v.ncase + lo * ex->M, items * 4, cudaMemcpyDeviceToHost, ex->stream));
+  CK(cudaStreamSynchronize(ex->stream));
+  for (size_t i = 0; i < items; i++) {
+    const uint32_t* entry = raw.data() + i * entry_words;
+    uint16_t* dst = counts + i * ex->iters;
+    for (int r = 0; r < ex->iters; r++)
+      dst[r] = (uint16_t)(v.pcnt_layout == 0 ? c16_table_count(entry, r) : sc_table_count(entry, v.pcnt_layout, r));
+  }
+  return GCRE_OK;
+}
+
+extern "C" int gcre_pathset_debug_lists(const gcre_pathset* ps, uint64_t* off, uint32_t* len, uint32_t* ncase, uint32_t* car) {
+  if (!ps || !off || !len || !ncase) return fail(GCRE_ERR_ARG, "null argument");
+  LIVE(ps);
+  const gcre_exec* ex = ps->ex;
+  CKS(use_device(ex));
+  const SparseView& v = ps->view;
+  if (!v.valid) return fail(GCRE_ERR_ASSERT, "the path set's carrier lists are not built");
+  const size_t items = (size_t)ps->size * ex->M;
+  CK(cudaMemcpyAsync(off, v.off, (items + 1) * 8, cudaMemcpyDeviceToHost, ex->stream));
+  if (items) {
+    CK(cudaMemcpyAsync(len, v.len, items * 4, cudaMemcpyDeviceToHost, ex->stream));
+    CK(cudaMemcpyAsync(ncase, v.ncase, items * 4, cudaMemcpyDeviceToHost, ex->stream));
+  }
+  CK(cudaStreamSynchronize(ex->stream));
+  const size_t total = (size_t)off[items];
+  if (total && !car) return fail(GCRE_ERR_ARG, "null argument");
+  if (total && ex->wide) {
+    CK(cudaMemcpyAsync(car, v.car, total * 4, cudaMemcpyDeviceToHost, ex->stream));
+    CK(cudaStreamSynchronize(ex->stream));
+  } else if (total) {
+    std::vector<uint16_t> narrow(total);
+    CK(cudaMemcpyAsync(narrow.data(), v.car, total * 2, cudaMemcpyDeviceToHost, ex->stream));
+    CK(cudaStreamSynchronize(ex->stream));
+    for (size_t k = 0; k < total; k++) car[k] = narrow[k];
+  }
+  return GCRE_OK;
+}
+
+// ------------------------------------------------------------------------------------------------------------------
 // value-table re-layout
 // ------------------------------------------------------------------------------------------------------------------
 static int ensure_diag(gcre_exec* ex, long long t_needed) {
@@ -1532,8 +1605,10 @@ static int ensure_view(gcre_exec* ex, gcre_pathset* ps, bool view_exact) {
 }
 
 // per-permutation counts of every (row, half) of a path set under the exec's current masks (join_sparse.cuh, PC kernels)
+// (a table a KEEP join emitted serves when it is current and holds every row: a row-sharded join emits its rows only)
 static int ensure_precount(gcre_exec* ex, gcre_pathset* ps) {
-  if (ps->view.pcnt && ps->view.pcnt_gen == ex->mask_gen && ps->view.pcnt_layout == 0) return GCRE_OK;
+  if (ps->view.pcnt && ps->view.pcnt_gen == ex->mask_gen && ps->view.pcnt_layout == 0 && ps->view.emit_lo == 0 && ps->view.emit_hi >= ps->size)
+    return GCRE_OK;
   dev_free(ex, ps->view.pcnt);
   ps->view.pcnt = nullptr;
   ps->view.pcnt_layout = 0;
@@ -1550,6 +1625,8 @@ static int ensure_precount(gcre_exec* ex, gcre_pathset* ps) {
     LAUNCHED();
   }
   ps->view.pcnt_gen = ex->mask_gen;
+  ps->view.emit_lo = 0;
+  ps->view.emit_hi = ps->size;
   return GCRE_OK;
 }
 

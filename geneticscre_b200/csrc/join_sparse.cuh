@@ -227,6 +227,15 @@ __device__ __forceinline__ int bits_for(int count) { return 32 - __clz(count); }
 #define GCRE_C16_REG(b) (2 * ((b) & 7) + ((b) >> 4))
 #define GCRE_C16_HI(b) (((b) >> 3) & 1)
 
+// host: the count of permutation r in one (row, half) entry of a count table in this register image (SparseView::pcnt,
+// layout 0: [perm block][q][lane][4] u32, register 4q + k in component k).  Tests read tables back through it
+// (gcre_pathset_debug_counts) and so depend on neither image.
+static inline uint32_t c16_table_count(const uint32_t* entry, int r) {
+  const int b = r & 31, lane = (r >> 5) & 31, pb = r >> 10, reg = GCRE_C16_REG(b);
+  const uint32_t v = entry[(((size_t)pb * 4 + (reg >> 2)) * 32 + lane) * 4 + (reg & 3)];
+  return GCRE_C16_HI(b) ? v >> 16 : v & 0xffffu;
+}
+
 // eight consecutive carriers of a (16-byte aligned, padded) list -> eight patient indices
 __device__ __forceinline__ void load8(const uint16_t* p, uint32_t (&c)[8]) {
   const uint4 v = __ldg(reinterpret_cast<const uint4*>(p));

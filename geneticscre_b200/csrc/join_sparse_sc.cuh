@@ -584,6 +584,13 @@ __global__ void __launch_bounds__(PTS ? sparse_sc::PTS_THREADS : sparse_sc::THRE
 static inline int sparse_sc_words(int Ip) { return Ip <= 128 ? 4 : Ip <= 256 ? 8 : 16; }
 // bytes of one (row, half) entry of that table: 32 lanes x NW / 2 registers
 static inline size_t sparse_sc_table_bytes(int Ip) { return (size_t)32 * (sparse_sc_words(Ip) / 2) * 4; }
+// host: the count of permutation r in one (row, half) entry of a table in that layout (nw words per lane group): lane
+// sub * nw + w holds registers R * sub .. R * sub + R - 1 of word w, R = nw / 2 (sc_reduce_scatter)
+static inline uint32_t sc_table_count(const uint32_t* entry, int nw, int r) {
+  const int b = r & 31, reg = GCRE_C16_REG(b), R = nw / 2;
+  const uint32_t v = entry[((reg / R) * nw + (r >> 5)) * R + reg % R];
+  return GCRE_C16_HI(b) ? v >> 16 : v & 0xffffu;
+}
 
 // PTS applies to <= 128 permutations when the matrix fits beside the CTA's static shared memory (queues, parked totals:
 // n <= ~12,400) and the launch has enough units to pay for staging it (160 KB per SM, ~10 us); pts_forced = 0 / 1 (GCRE_SC_PTS,

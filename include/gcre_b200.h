@@ -245,6 +245,26 @@ int gcre_exec_read_perm_max(const gcre_exec* ex, double* out_perm);
 int gcre_merge_topk(const gcre_score* lists, const int* list_sizes, int n_lists, int top_k, gcre_score* out_scores,
                     int* n_scores);
 
+/*
+ * ---- Test and diagnostics only ----
+ * Read-backs of the state the sparse kernels keep per path set, so that tests can check it directly and not only through
+ * the join results it feeds.  Each copies on the exec's stream and waits for it.  Not part of the reference's surface.
+ *
+ * gcre_pathset_debug_view_info: out = int64[8]: [0] carrier lists built, [1] their padded entries, [2] len / ncase filled,
+ *   [3] a count table present, [4] its layout (0: the 1,024-permutation register image of join_sparse.cuh; 4 / 8 / 16: the
+ *   split-carrier layout of join_sparse_sc.cuh), [5] it was built for the exec's current permutation masks, [6] / [7] the rows
+ *   [lo, hi) it holds (a KEEP join's emitted rows, or every row of a pre-count table).
+ * gcre_pathset_debug_counts: the table decoded: counts = uint16[hi - lo][method][iters_requested], the count of permutation r
+ *   in half h of row lo + i; len / ncase = uint32[hi - lo][method] carriers and carriers < num_cases per half (NULL: not
+ *   copied).  GCRE_ERR_ASSERT when the set holds no table.
+ * gcre_pathset_debug_lists: the carrier lists: off = uint64[size * method + 1] (list starts, in entries), len / ncase =
+ *   uint32[size * method], car = uint32[off[size * method]] (patient indices, sentinel num_cases + num_ctrls as padding).
+ *   GCRE_ERR_ASSERT when the lists are not built.
+ */
+int gcre_pathset_debug_view_info(const gcre_pathset* ps, int64_t* out);
+int gcre_pathset_debug_counts(const gcre_pathset* ps, uint16_t* counts, uint32_t* len, uint32_t* ncase);
+int gcre_pathset_debug_lists(const gcre_pathset* ps, uint64_t* off, uint32_t* len, uint32_t* ncase, uint32_t* car);
+
 #ifdef __cplusplus
 }
 #endif
