@@ -1647,7 +1647,8 @@ static bool same_base(const Provenance& a, const Provenance& b) {
 // A KEEP join has written result rows [pair_lo, pair_hi): record their tails (and heads) when the partner set is a selection
 // of a live base set.  Called after rows_written(paths_res).
 static int record_provenance(gcre_exec* ex, const gcre_uidset* us, const gcre_pathset* paths0, const gcre_pathset* paths1, gcre_pathset* paths_res,
-                             uint32_t ub, uint32_t ue, unsigned long long pair_lo, unsigned long long pair_hi) {
+                             uint32_t ub, uint32_t ue, unsigned long long pair_lo, unsigned long long pair_hi, unsigned long long unit_lo,
+                             unsigned long long unit_hi) {
   const Provenance& sel = paths1->prov;
   if (!provenance_useful(ex) || !us->res_is_prefix || pair_hi <= pair_lo || paths_res == paths0 || paths_res == paths1 || !sel.sel || !base_current(ex, sel)) return GCRE_OK;
   const Provenance& up = paths0->prov;
@@ -1656,9 +1657,9 @@ static int record_provenance(gcre_exec* ex, const gcre_uidset* us, const gcre_pa
   Provenance& p = paths_res->prov;
   CK(dev_alloc(ex, (void**)&p.tail, (size_t)paths_res->size * 4));
   if (heads) CK(dev_alloc(ex, (void**)&p.head, (size_t)paths_res->size * 4));
-  (ex->M == 1 ? record_rows_kernel<1> : record_rows_kernel<2>)<<<grid_for((long long)(ue - ub), 256), 256, 0, ex->stream>>>(
-      ub, ue, (const int32_t*)us->count.p, (const uint32_t*)us->loc.p, (const unsigned long long*)us->res.p, (const int32_t*)us->signs.p, us->path_length,
-      sel.sel, up.tail, p.tail, p.head);
+  (ex->M == 1 ? record_rows_kernel<1> : record_rows_kernel<2>)<<<grid_for((long long)(unit_hi - unit_lo), 256), 256, 0, ex->stream>>>(
+      unit_lo, unit_hi, (const uint32_t*)us->unit_idx.p, (const unsigned long long*)us->units.p, sparse::PB, (const int32_t*)us->count.p,
+      (const uint32_t*)us->loc.p, (const unsigned long long*)us->res.p, (const int32_t*)us->signs.p, us->path_length, sel.sel, up.tail, p.tail, p.head);
   CK(cudaGetLastError());
   LAUNCHED();
   p.base = sel.base;
@@ -1672,16 +1673,17 @@ static int record_provenance(gcre_exec* ex, const gcre_uidset* us, const gcre_pa
 
 // The base set whose gene rows a score-only join over upstream rows [ub, ue) may be scored against (tail form), or null:
 // both operands carry entries over the same live base set, and every pair's partner head, oriented by the pair, is its
-// upstream row's tail (one pass over the pairs, one flag read back).
+// upstream row's tail (one pass over the work units [unit_lo, unit_hi) of those rows, one flag read back).
 static int tail_form_base(gcre_exec* ex, const gcre_uidset* us, const gcre_pathset* paths0, const gcre_pathset* paths1, uint32_t ub, uint32_t ue,
-                          const gcre_pathset** out) {
+                          unsigned long long unit_lo, unsigned long long unit_hi, const gcre_pathset** out) {
   *out = nullptr;
   const Provenance &up = paths0->prov, &pt = paths1->prov;
   if (!up.tail || !pt.tail || !pt.head || !same_base(up, pt) || !base_current(ex, up) || ub < up.lo || ue > up.hi || ue <= ub) return GCRE_OK;
   unsigned* d_bad = ex->d_scalars + 12;
   CK(cudaMemsetAsync(d_bad, 0, sizeof(unsigned), ex->stream));
-  (ex->M == 1 ? tail_eligible_kernel<1> : tail_eligible_kernel<2>)<<<grid_for((long long)(ue - ub), 256), 256, 0, ex->stream>>>(
-      ub, ue, (const int32_t*)us->count.p, (const uint32_t*)us->loc.p, (const int32_t*)us->signs.p, us->path_length, up.tail, pt.head, pt.lo, pt.hi, d_bad);
+  (ex->M == 1 ? tail_eligible_kernel<1> : tail_eligible_kernel<2>)<<<grid_for((long long)(unit_hi - unit_lo), 256), 256, 0, ex->stream>>>(
+      unit_lo, unit_hi, (const uint32_t*)us->unit_idx.p, (const unsigned long long*)us->units.p, sparse::PB, (const int32_t*)us->count.p,
+      (const uint32_t*)us->loc.p, (const int32_t*)us->signs.p, us->path_length, up.tail, pt.head, pt.lo, pt.hi, d_bad);
   CK(cudaGetLastError());
   LAUNCHED();
   CK(cudaMemcpyAsync(ex->h_scalars + 12, d_bad, sizeof(unsigned), cudaMemcpyDeviceToHost, ex->stream));
@@ -1961,7 +1963,7 @@ static int choose_join_form(const JoinCall& c, int requested, long long t_needed
   // it on joins of any size / never.
   if (!c.keep && !ex->split_ok && pairs > 0) {
     const bool want = c.knobs.tail >= 0 ? c.knobs.tail == 1 : pairs >= (1ull << 20);
-    if (want) CKS(tail_form_base(ex, c.us, c.paths0, c.paths1, c.ub, c.ue, &f->tail_base));
+    if (want) CKS(tail_form_base(ex, c.us, c.paths0, c.paths1, c.ub, c.ue, c.unit_lo, c.unit_hi, &f->tail_base));
     if (f->tail_base && (size_t)f->tail_base->size * ex->M * npb * 2048 > budget) f->tail_base = nullptr;
   }
   // A KEEP join whose partner set is a live selection of a base set (level 3: data1's gene rows) may score its partners through
@@ -2277,7 +2279,7 @@ static int join_impl(gcre_exec* ex, const gcre_uidset* us, const gcre_pathset* p
     } else {
       drop_view(paths_res);
     }
-    CKS(record_provenance(ex, us, paths0, paths1, paths_res, ub, ue, pair_lo, pair_hi));
+    CKS(record_provenance(ex, us, paths0, paths1, paths_res, ub, ue, pair_lo, pair_hi, unit_lo, unit_hi));
   }
 
   CKS(emit_topk(held, top_k, out_scores, n_scores));

@@ -14,7 +14,7 @@
 //           accumulated on top of the base (ballot-compacted into a shared-memory queue of row offsets, drained eight at a
 //           time); partners that add no carrier reuse the base evaluation
 //   score : counts -> anti-diagonal value-table look-ups (src/methods.h:96-103, 220-230) -> running per-permutation
-//           max kept in registers across all units of the warp, merged at the end with one atomicMax per permutation
+//           max kept in registers across all units of the warp, merged at the end with an atomicMax per permutation it raises
 //   true scores / top-K candidates / kept rows exactly as in the dense kernel.
 //
 // Kept rows carry their counts forward.  A KEEP join has the per-permutation counts of every row it writes in registers
@@ -339,12 +339,22 @@ __global__ void __launch_bounds__(sparse::THREADS, sparse::min_blocks(M, THR)) j
   float best[THR ? 1 : 32];
 #pragma unroll
   for (int b = 0; b < (THR ? 1 : 32); b++) best[b] = 0.0f;
+  // Only records go out: the lane reads its 32 current maxima (one 128-byte line) and raises those its own beat.  Every warp of
+  // the persistent grid flushes at the end of the launch, all at once and on the same lines of a.perm_max; issued
+  // unconditionally, those atomics serialised the tail of every small join.  Skipping one is safe: maxima only grow.
   auto flush_best = [&](int pb) {
     const int r0 = (pb * 32 + lane) * 32;
-    if (!THR && r0 < a.Ip) {
+    if constexpr (!THR) {
+      if (r0 >= a.Ip) return;
+      const int4* p = reinterpret_cast<const int4*>(a.perm_max + r0);
 #pragma unroll
-      for (int b = 0; b < (THR ? 1 : 32); b++)
-        if (best[b] > 0.0f) atomicMax(a.perm_max + r0 + b, __float_as_int(best[b]));
+      for (int q = 0; q < 8; q++) {
+        const int4 v = __ldcg(p + q);
+        const int cur[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+        for (int k = 0; k < 4; k++)
+          if (best[4 * q + k] > __int_as_float(cur[k])) atomicMax(a.perm_max + r0 + 4 * q + k, __float_as_int(best[4 * q + k]));
+      }
     }
   };
   // THR = true: thresholded look-ups.  The per-permutation maxima live in global memory only (a.perm_max, float bit patterns

@@ -235,22 +235,31 @@ __global__ void finish_uids_kernel(uint32_t n, const int32_t* __restrict__ count
 // Entries name a row of a base path set and its orientation: base row << 1 | 1 when the row's halves are swapped (method 2:
 // joined half h holds base half 1 - h).  A KEEP join whose partner set is a selection of the base set records, per result
 // row it writes, the partner's base row (`tail`) and - when every upstream row is exactly one oriented base row - the
-// upstream row's entry (`head`).  One thread per upstream row of [ub, ue).  `sel`: the selection's own entries (below).
+// upstream row's entry (`head`).  `sel`: the selection's own entries (below).
+// Both passes below run one thread per work unit of the join index (<= partners_per_unit partners of one upstream row; units
+// [unit_lo, unit_hi) are those of upstream rows [ub, ue)).  The networks are heavy-tailed: one row of the benchmark's network has
+// 4,622 partners, and a thread per upstream row left each launch as long as that row's serial loop.  A warp per unit idled
+// most lanes instead: the level-4 rows of the benchmark average 9 partners (BASELINE config 3, B200 at 1,000 W, eligibility pass
+// of methods 1 / 2: 0.37 / 0.39 ms with a thread per row, 0.21 / 0.25 with a warp per unit, 0.05 / 0.06 with a thread per unit).
 template <int M>
-__global__ void record_rows_kernel(uint32_t ub, uint32_t ue, const int32_t* __restrict__ count, const uint32_t* __restrict__ location,
-                                   const unsigned long long* __restrict__ res_idx, const int32_t* __restrict__ signs, int path_length,
-                                   const uint32_t* __restrict__ sel, const uint32_t* __restrict__ tail0, uint32_t* __restrict__ tail_res,
-                                   uint32_t* __restrict__ head_res) {
-  const uint32_t idx = ub + blockIdx.x * blockDim.x + threadIdx.x;
-  if (idx >= ue) return;
-  const int c = count[idx];
+__global__ void record_rows_kernel(unsigned long long unit_lo, unsigned long long unit_hi, const uint32_t* __restrict__ unit_idx,
+                                   const unsigned long long* __restrict__ unit_prefix, int partners_per_unit, const int32_t* __restrict__ count,
+                                   const uint32_t* __restrict__ location, const unsigned long long* __restrict__ res_idx,
+                                   const int32_t* __restrict__ signs, int path_length, const uint32_t* __restrict__ sel,
+                                   const uint32_t* __restrict__ tail0, uint32_t* __restrict__ tail_res, uint32_t* __restrict__ head_res) {
+  const unsigned long long q = unit_lo + (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (q >= unit_hi) return;
+  const uint32_t idx = unit_idx[q];
+  const uint32_t j0 = (uint32_t)(q - unit_prefix[idx]) * (uint32_t)partners_per_unit;
+  const uint32_t j1 = min((uint32_t)count[idx], j0 + (uint32_t)partners_per_unit);
+  const uint32_t loc0 = location[idx];
+  const unsigned long long r0 = res_idx[idx];
   const uint32_t head = head_res ? tail0[idx] : 0u;
-  for (int j = 0; j < c; j++) {
-    const uint32_t loc = location[idx] + (uint32_t)j;
-    const unsigned long long r = res_idx[idx] + (unsigned long long)j;
+  for (uint32_t j = j0; j < j1; j++) {
+    const uint32_t loc = loc0 + j;
     const bool swap = (M == 2) && !need_flip(path_length, signs, idx, loc);  // src/methods.h:137-145: partner half 1 - h joins half h
-    tail_res[r] = sel[loc] | (swap ? 1u : 0u);
-    if (head_res) head_res[r] = head;
+    tail_res[r0 + j] = sel[loc] | (swap ? 1u : 0u);
+    if (head_res) head_res[r0 + j] = head;
   }
 }
 
@@ -260,21 +269,25 @@ __global__ void selection_entries_kernel(const int32_t* __restrict__ idx, uint32
   if (k < n) sel[k] = (uint32_t)idx[k] << 1;
 }
 
-// Does every pair of upstream rows [ub, ue) meet the tail form's condition: the partner's head, oriented as the pair joins it,
+// Does every pair of units [unit_lo, unit_hi) meet the tail form's condition: the partner's head, oriented as the pair joins it,
 // is the upstream row's tail (same base row, same orientation)?  Partner rows outside [head_lo, head_hi) have no record.
-// Any pair that does not sets *bad.
+// Any pair that does not sets *bad.  One thread per unit, as record_rows_kernel.
 template <int M>
-__global__ void tail_eligible_kernel(uint32_t ub, uint32_t ue, const int32_t* __restrict__ count, const uint32_t* __restrict__ location,
-                                     const int32_t* __restrict__ signs, int path_length, const uint32_t* __restrict__ tail0,
-                                     const uint32_t* __restrict__ head1, unsigned long long head_lo, unsigned long long head_hi,
-                                     unsigned* __restrict__ bad) {
-  const uint32_t idx = ub + blockIdx.x * blockDim.x + threadIdx.x;
+__global__ void tail_eligible_kernel(unsigned long long unit_lo, unsigned long long unit_hi, const uint32_t* __restrict__ unit_idx,
+                                     const unsigned long long* __restrict__ unit_prefix, int partners_per_unit, const int32_t* __restrict__ count,
+                                     const uint32_t* __restrict__ location, const int32_t* __restrict__ signs, int path_length,
+                                     const uint32_t* __restrict__ tail0, const uint32_t* __restrict__ head1, unsigned long long head_lo,
+                                     unsigned long long head_hi, unsigned* __restrict__ bad) {
+  const unsigned long long q = unit_lo + (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
   bool ok = true;
-  if (idx < ue) {
-    const int c = count[idx];
-    const uint32_t t = c > 0 ? tail0[idx] : 0u;
-    for (int j = 0; j < c && ok; j++) {
-      const uint32_t loc = location[idx] + (uint32_t)j;
+  if (q < unit_hi) {
+    const uint32_t idx = unit_idx[q];
+    const uint32_t j0 = (uint32_t)(q - unit_prefix[idx]) * (uint32_t)partners_per_unit;
+    const uint32_t j1 = min((uint32_t)count[idx], j0 + (uint32_t)partners_per_unit);
+    const uint32_t loc0 = location[idx];
+    const uint32_t t = tail0[idx];
+    for (uint32_t j = j0; j < j1 && ok; j++) {
+      const uint32_t loc = loc0 + j;
       if (loc < head_lo || loc >= head_hi) {
         ok = false;
         break;
