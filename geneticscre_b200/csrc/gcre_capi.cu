@@ -360,6 +360,8 @@ struct gcre_exec {
   unsigned* d_scalars = nullptr;  // [0] candidate count, [1] max_total, [2..3] 64-bit work counter of the sparse kernel,
                                   // [4..5] 64-bit count of pairs that took the exact path of the thresholded look-ups (diagnostic)
   DevBuf cand, scratch, scan_tmp;
+  DevBuf ident;             // [ident_rows] entries k << 1: the row map of a pre-counted join whose partners are their own rows
+  uint32_t ident_rows = 0;
   unsigned* h_scalars = nullptr;  // pinned
   // page-locked landing area of a join's results: [kSpecCand candidates][Ip permutation maxima].  They are copied behind every
   // launch together with the scalars, so a join waits for the device once instead of three times.
@@ -557,7 +559,7 @@ extern "C" int gcre_exec_create(int method, int num_cases, int num_ctrls, int it
     CK(pool_stream(device, &ex->copy_stream));
     CK(pool_event(device, false, &ex->ev_copy));
     CK(pool_event(device, false, &ex->ev_order));
-    for (DevBuf* b : {&ex->cand, &ex->scratch, &ex->scan_tmp}) b->owner = ex;
+    for (DevBuf* b : {&ex->cand, &ex->scratch, &ex->scan_tmp, &ex->ident}) b->owner = ex;
     CK(dev_alloc(ex, (void**)&ex->d_masks, std::max<size_t>((size_t)iters * ex->W64, 1) * 8));
     CK(dev_alloc(ex, (void**)&ex->d_pm, (size_t)ex->Wp * ex->Ip * 8));
     CK(cudaMemsetAsync(ex->d_masks, 0, std::max<size_t>((size_t)iters * ex->W64, 1) * 8, ex->stream));
@@ -608,6 +610,7 @@ extern "C" int gcre_exec_destroy(gcre_exec* ex) {
   ex->cand.release();
   ex->scan_tmp.release();
   ex->scratch.release();
+  ex->ident.release();
   // streams (drained above), events and the page-locked words go back to the process-wide pools
   unpool_pinned(ex->h_scalars);
   pinned_big_release(ex->h_res);
@@ -1692,6 +1695,20 @@ static int tail_form_base(gcre_exec* ex, const gcre_uidset* us, const gcre_paths
   return GCRE_OK;
 }
 
+// The row map of a pre-counted join whose partner set of `rows` rows is scored through itself: entries k << 1 (precount_mode
+// refuses sets of 2^31 rows or more)
+static int identity_map(gcre_exec* ex, uint32_t rows, const uint32_t** out) {
+  if (rows > ex->ident_rows) {
+    CKS(ex->ident.ensure((size_t)rows * 4));
+    selection_entries_kernel<<<grid_for((long long)rows, 256), 256, 0, ex->stream>>>(nullptr, rows, (uint32_t*)ex->ident.p);
+    CK(cudaGetLastError());
+    LAUNCHED();
+    ex->ident_rows = rows;
+  }
+  *out = (const uint32_t*)ex->ident.p;
+  return GCRE_OK;
+}
+
 // ------------------------------------------------------------------------------------------------------------------
 // join
 // ------------------------------------------------------------------------------------------------------------------
@@ -1889,9 +1906,10 @@ struct JoinCall {
 struct JoinForm {
   int kernel = GCRE_KERNEL_DENSE;
   bool split = false;                        // the split-carrier kernels (join_sparse_sc.cuh)
-  bool precount = false;                     // pre-counted partners (PC kernels of join_sparse.cuh)
-  const gcre_pathset* tail_base = nullptr;   // partners scored through this set's rows (PC + TAIL kernels): the tail form, or ...
-  bool selected = false;                     // ... with `precount`, a KEEP join whose partners are a selection of this set
+  bool precount = false;                     // pre-counted partners: the partner set itself, or the base set of a selection partner
+  const gcre_pathset* pc_set = nullptr;      // PC kernels of join_sparse.cuh: partners are scored through this set's carrier lists
+                                             // and pre-counted table (with `precount` as above, else the base set of the tail form)
+  const uint32_t* map1 = nullptr;            // ... through these rows of it: per partner row, pc_set row << 1 | halves swapped
   bool emit = false;                         // kept rows take their counts along
   bool base_emitted = false;                 // the upstream rows carry counts and totals from the join that made them
   bool thr = false;                          // thresholded look-ups
@@ -1963,14 +1981,15 @@ static int choose_join_form(const JoinCall& c, int requested, long long t_needed
   // it on joins of any size / never.
   if (!c.keep && !ex->split_ok && pairs > 0) {
     const bool want = c.knobs.tail >= 0 ? c.knobs.tail == 1 : pairs >= (1ull << 20);
-    if (want) CKS(tail_form_base(ex, c.us, c.paths0, c.paths1, c.ub, c.ue, c.unit_lo, c.unit_hi, &f->tail_base));
-    if (f->tail_base && (size_t)f->tail_base->size * ex->M * npb * 2048 > budget) f->tail_base = nullptr;
+    if (want) CKS(tail_form_base(ex, c.us, c.paths0, c.paths1, c.ub, c.ue, c.unit_lo, c.unit_hi, &f->pc_set));
+    if (f->pc_set && (size_t)f->pc_set->size * ex->M * npb * 2048 > budget) f->pc_set = nullptr;
+    if (f->pc_set) f->map1 = c.paths1->prov.tail;
   }
   // A KEEP join whose partner set is a live selection of a base set (level 3: data1's gene rows) may score its partners through
   // the base set's rows and pre-counted table (join_sparse.cuh): a selected row is its base row, so no eligibility pass
   const Provenance& sel = c.paths1->prov;
   const gcre_pathset* sel_base = c.keep && !ex->split_ok && sel.sel && base_current(ex, sel) ? sel.base : nullptr;
-  int pc_mode = f->tail_base ? PRECOUNT_NO
+  int pc_mode = f->pc_set ? PRECOUNT_NO
                 : sel_base   ? precount_mode(pairs, sel_base->size, ex->M, npb, budget, c.knobs.precount, true)
                              : precount_mode(pairs, c.paths1->size, ex->M, npb, budget, c.knobs.precount, false);
   if (ex->split_ok && pc_mode == PRECOUNT_SAMPLE) pc_mode = PRECOUNT_NO;  // the split-carrier kernel is the better form there
@@ -1998,9 +2017,10 @@ static int choose_join_form(const JoinCall& c, int requested, long long t_needed
     pc_mode = (sums[0] * 10 < sums[1] * 6) ? PRECOUNT_YES : PRECOUNT_NO;
   }
   f->precount = pc_mode == PRECOUNT_YES;
-  if (f->precount && sel_base) {
-    f->tail_base = sel_base;
-    f->selected = true;
+  if (f->precount) {
+    f->pc_set = sel_base ? sel_base : c.paths1;
+    if (sel_base) f->map1 = sel.sel;
+    else CKS(identity_map(ex, c.paths1->size, &f->map1));
   }
   return GCRE_OK;
 }
@@ -2013,15 +2033,15 @@ static int prepare_join_operands(const JoinCall& c, const JoinForm& f, JoinParam
   if (f.kernel == GCRE_KERNEL_SPARSE) {
     CKS(ensure_patient_major(ex, f.split));
     gcre_pathset* p0 = const_cast<gcre_pathset*>(c.paths0);
-    gcre_pathset* p1 = const_cast<gcre_pathset*>(f.tail_base ? f.tail_base : c.paths1);
+    gcre_pathset* p1 = const_cast<gcre_pathset*>(f.pc_set ? f.pc_set : c.paths1);
     if (!f.base_emitted) CKS(ensure_view(ex, p0, c.knobs.view_exact));
     CKS(ensure_view(ex, p1, c.knobs.view_exact));
-    if (f.precount || f.tail_base) CKS(ensure_precount(ex, p1));
+    if (f.pc_set) CKS(ensure_precount(ex, p1));
     sp->off0 = p0->view.off; sp->len0 = p0->view.len; sp->car0 = p0->view.car; sp->ncase0 = p0->view.ncase;
     sp->pcnt0 = f.base_emitted ? p0->view.pcnt : nullptr;
     sp->off1 = p1->view.off; sp->len1 = p1->view.len; sp->car1 = p1->view.car; sp->ncase1 = p1->view.ncase;
-    sp->pcnt1 = (f.precount || f.tail_base) ? p1->view.pcnt : nullptr;
-    sp->tail1 = f.selected ? c.paths1->prov.sel : f.tail_base ? c.paths1->prov.tail : nullptr;
+    sp->pcnt1 = f.pc_set ? p1->view.pcnt : nullptr;
+    sp->map1 = f.map1;
     sp->n = ex->n;
     sp->unit_prefix = (const unsigned long long*)c.us->units.p;
     sp->unit_idx = (const uint32_t*)c.us->unit_idx.p;
@@ -2127,7 +2147,7 @@ static int run_launch_plan(const JoinCall& c, const JoinForm& f, JoinParams jp, 
       sp.n_units = pe - p;
       CK(cudaMemsetAsync(ex->d_scalars + 2, 0, 6 * sizeof(unsigned), ex->stream));
       if (f.split) CK(launch_join_sparse_sc(ex->stream, jp, sp, ex->M, c.keep, ex->sm_count, ex->wide, c.knobs.sc_pts, &st->shared_masks));
-      else CK(launch_join_sparse(ex->stream, jp, sp, ex->M, c.keep, ex->sm_count, f.precount, f.tail_base != nullptr, f.thr, ex->wide));
+      else CK(launch_join_sparse(ex->stream, jp, sp, ex->M, c.keep, ex->sm_count, f.pc_set != nullptr, f.thr, ex->wide));
       LAUNCHED();
       st->launches++;
     } else {
@@ -2299,7 +2319,7 @@ static int join_impl(gcre_exec* ex, const gcre_uidset* us, const gcre_pathset* p
     opts->kernel_used = form.kernel;
     opts->launches = st.launches;
     opts->precounted = form.precount;
-    opts->tail_form = form.tail_base != nullptr && !form.selected;
+    opts->tail_form = form.pc_set != nullptr && !form.precount;
     opts->split_carrier = form.split;
     opts->shared_masks = st.shared_masks;
     opts->thresholded = form.thr && st.launches > 0 ? 1 : 0;

@@ -263,10 +263,11 @@ __global__ void record_rows_kernel(unsigned long long unit_lo, unsigned long lon
   }
 }
 
-// The entries of a selection (gcre_pathset_select): row k is base row idx[k], halves as they are
+// The entries of a selection (gcre_pathset_select): row k is base row idx[k], halves as they are; with idx null row k is row k
+// (the map of a pre-counted join whose partners are scored through their own rows)
 __global__ void selection_entries_kernel(const int32_t* __restrict__ idx, uint32_t n, uint32_t* __restrict__ sel) {
   const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
-  if (k < n) sel[k] = (uint32_t)idx[k] << 1;
+  if (k < n) sel[k] = (idx ? (uint32_t)idx[k] : k) << 1;
 }
 
 // Does every pair of units [unit_lo, unit_hi) meet the tail form's condition: the partner's head, oriented as the pair joins it,
