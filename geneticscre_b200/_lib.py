@@ -86,6 +86,8 @@ SYMBOLS = {
     "gcre_pathset_debug_view_info": (_I, [_VP, C.POINTER(C.c_int64)]),
     "gcre_pathset_debug_counts": (_I, [_VP, C.POINTER(C.c_uint16), C.POINTER(_U32), C.POINTER(_U32)]),
     "gcre_pathset_debug_lists": (_I, [_VP, C.POINTER(C.c_uint64), C.POINTER(_U32), C.POINTER(_U32), C.POINTER(_U32)]),
+    "gcre_pathset_debug_bounds": (_I, [_VP, C.POINTER(C.c_int64)]),
+    "gcre_exec_debug_diag_cap": (_I, [_VP, C.POINTER(C.c_int64)]),
 }
 
 _lib = None

@@ -171,6 +171,13 @@ class PathSet:
                      "layout": int(info[4]), "current": bool(info[5])}
         return {"lists": lists, "table": table, "stats_valid": bool(info[2])}
 
+    def debug_bounds(self):
+        """``{"max_half_pop": the recorded bound on any half-row's carriers (-1 = unknown), "allocated": carrier-list entries
+        allocated (0 = no lists)}`` (include/gcre_b200.h, gcre_pathset_debug_bounds)."""
+        out = np.zeros(2, dtype=np.int64)
+        check(self.ex._lib.gcre_pathset_debug_bounds(self._h, _ptr(out, C.c_int64)))
+        return {"max_half_pop": int(out[0]), "allocated": int(out[1])}
+
 
 class JoinExec:
     """JoinExec (src/gcre.h:103-180).  ``nthreads`` is accepted and ignored (the join runs on the GPU)."""
@@ -303,6 +310,12 @@ class JoinExec:
         p, n = C.c_void_p(), C.c_int(0)
         check(self._lib.gcre_exec_device_perm_max(self._h, C.byref(p), C.byref(n)))
         return p.value, n.value
+
+    def debug_diag_cap(self):
+        """The largest joined half-row total the anti-diagonal value tables cover (-1: none built) - tests and diagnostics."""
+        out = C.c_int64(0)
+        check(self._lib.gcre_exec_debug_diag_cap(self._h, C.byref(out)))
+        return out.value
 
     def read_perm_max(self):
         out = np.zeros(max(self.iters_requested, 1), dtype=np.float64)

@@ -1441,6 +1441,20 @@ extern "C" int gcre_pathset_debug_lists(const gcre_pathset* ps, uint64_t* off, u
   return GCRE_OK;
 }
 
+extern "C" int gcre_pathset_debug_bounds(const gcre_pathset* ps, int64_t* out) {
+  if (!ps || !out) return fail(GCRE_ERR_ARG, "null argument");
+  LIVE(ps);
+  out[0] = ps->max_half_pop;  // as recorded, not recomputed
+  out[1] = ps->view.valid ? (int64_t)ps->view.total : 0;
+  return GCRE_OK;
+}
+
+extern "C" int gcre_exec_debug_diag_cap(const gcre_exec* ex, int64_t* out) {
+  if (!ex || !out) return fail(GCRE_ERR_ARG, "null argument");
+  *out = ex->diag_cap;
+  return GCRE_OK;
+}
+
 // ------------------------------------------------------------------------------------------------------------------
 // value-table re-layout
 // ------------------------------------------------------------------------------------------------------------------
@@ -2289,8 +2303,12 @@ static int join_impl(gcre_exec* ex, const gcre_uidset* us, const gcre_pathset* p
   CKS(run_launch_plan(c, form, jp, sp, tr, &held, &st));
   tr.mark("launches");
   if (keep) {
-    // (rows outside a shard of a fresh result set are zero: the kernel's maximum over the written rows is the set's)
-    paths_res->max_half_pop = ((pair_lo == 0 && pair_hi == total) || us->res_is_prefix) ? std::max<long long>(paths_res->max_half_pop, (long long)ex->h_scalars[1]) : -1;
+    // The kernel's maximum covers the rows it wrote.  A join that wrote every row (a full one with prefix result rows) sets the
+    // bound from them; after any other join the rows it did not write keep theirs, so an unknown bound (-1: the set was
+    // loaded or set since its last join) stays unknown and a known one (0 for a fresh set) grows to cover the new rows.
+    const long long prev = paths_res->max_half_pop;
+    const bool every_row = us->res_is_prefix && pair_lo == 0 && pair_hi == total;
+    paths_res->max_half_pop = (every_row || prev >= 0) ? std::max<long long>(prev, (long long)ex->h_scalars[1]) : -1;
     if (form.emit) {  // emitted with the rows
       paths_res->view.pcnt_gen = ex->mask_gen;
       paths_res->view.stats_valid = true;

@@ -260,10 +260,17 @@ int gcre_merge_topk(const gcre_score* lists, const int* list_sizes, int n_lists,
  * gcre_pathset_debug_lists: the carrier lists: off = uint64[size * method + 1] (list starts, in entries), len / ncase =
  *   uint32[size * method], car = uint32[off[size * method]] (patient indices, sentinel num_cases + num_ctrls as padding).
  *   GCRE_ERR_ASSERT when the lists are not built.
+ * gcre_pathset_debug_bounds: out = int64[2]: [0] the largest carrier count of any half-row as the set records it (not
+ *   recomputed; -1 = unknown, computed by the next join that reads the set), which sizes its carrier lists and the exec's
+ *   anti-diagonal tables and must never be below the true one; [1] the carrier-list entries allocated (0: no lists built).
+ * gcre_exec_debug_diag_cap: out = the largest joined half-row total the exec's anti-diagonal value tables cover (-1: none
+ *   built since the value table last changed).
  */
 int gcre_pathset_debug_view_info(const gcre_pathset* ps, int64_t* out);
 int gcre_pathset_debug_counts(const gcre_pathset* ps, uint16_t* counts, uint32_t* len, uint32_t* ncase);
 int gcre_pathset_debug_lists(const gcre_pathset* ps, uint64_t* off, uint32_t* len, uint32_t* ncase, uint32_t* car);
+int gcre_pathset_debug_bounds(const gcre_pathset* ps, int64_t* out);
+int gcre_exec_debug_diag_cap(const gcre_exec* ex, int64_t* out);
 
 #ifdef __cplusplus
 }
