@@ -34,7 +34,7 @@ class JoinOptsC(C.Structure):
     _fields_ = [("uid_begin", C.c_uint32), ("uid_end", C.c_uint32), ("kernel", C.c_int32), ("skip_host_perm", C.c_int32),
                 ("pairs_scored", C.c_uint64), ("kernel_ms", C.c_double), ("kernel_used", C.c_int32), ("launches", C.c_int32),
                 ("precounted", C.c_int32), ("split_carrier", C.c_int32), ("thresholded", C.c_int32), ("shared_masks", C.c_int32),
-                ("exact_pairs", C.c_uint64), ("tail_form", C.c_int32), ("reserved2", C.c_int32)]
+                ("exact_pairs", C.c_uint64), ("tail_form", C.c_int32), ("dedup_rows", C.c_uint32)]
 
 
 # every symbol include/gcre_b200.h declares: name -> (restype, argtypes)

@@ -302,7 +302,7 @@ class JoinExec:
         scores = [Score(s.score, s.src, s.trg, s.cases, s.ctrls) for s in sc[: n_sc.value]]
         info = {"pairs": int(opts.pairs_scored), "kernel_ms": float(opts.kernel_ms), "kernel": int(opts.kernel_used), "launches": int(opts.launches),
                 "precounted": bool(opts.precounted), "tail_form": bool(opts.tail_form), "split_carrier": bool(opts.split_carrier), "thresholded": bool(opts.thresholded), "shared_masks": bool(opts.shared_masks),
-                "exact_pairs": int(opts.exact_pairs)}
+                "exact_pairs": int(opts.exact_pairs), "dedup_rows": int(opts.dedup_rows)}
         return joined_res(scores, perm[: self.iters_requested].copy(), info)
 
     def device_perm_max(self):

@@ -20,6 +20,10 @@
 #include <thread>
 #include <vector>
 
+#include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_scan.cuh>
+#include <cub/device/device_select.cuh>
+
 #include "common.cuh"
 #include "setup_kernels.cuh"
 #include "join_dense.cuh"
@@ -410,6 +414,20 @@ struct gcre_uidset {
   unsigned long long total = 0, n_units_total = 0, max_loc_end = 0, max_res_end = 0;
   bool res_is_prefix = true;   // every path_idx equals the running sum of counts: a full join overwrites rows [0, total)
   DevBuf count, loc, prefix, res, units, unit_idx, signs;
+  // Equal upstream rows grouped for the score-only joins over this index (group_upstream_rows), for one version of one upstream
+  // set and one row range: rebuilt when any of them changes, reused by the joins of every permutation batch in between
+  struct Grouping {
+    bool built = false, collide = false;  // collide: built under the test hook that leaves the fingerprints out of the keys
+    unsigned long long set_uid = 0, set_ver = 0;
+    uint32_t ub = 0, ue = 0;
+    unsigned long long n_units = 0;  // the representatives' work units (unit_list)
+    uint32_t dedup_rows = 0;         // rows that are members of another row's group
+    bool pays = false;               // enough duplicates to pay for the indirection (GROUP_MAX_UNIT_SHARE)
+    DevBuf mem_rng, members, unit_list;  // per row the range of its members in `members`; the representatives' units
+    mutable std::vector<uint32_t> h_members;  // host copy of `members`, read back when a candidate first needs it (expand_members)
+    mutable bool h_members_valid = false;
+  };
+  mutable Grouping grp;
 };
 
 static int materialize_zero(gcre_pathset* ps) {
@@ -445,6 +463,7 @@ static void drop_view(gcre_pathset* ps) {
   dev_free(ps->ex, ps->view.ncase);
   dev_free(ps->ex, ps->view.car);
   dev_free(ps->ex, ps->view.pcnt);
+  dev_free(ps->ex, ps->view.fp);
   ps->view = SparseView();
 }
 
@@ -1556,11 +1575,14 @@ static int ensure_view(gcre_exec* ex, gcre_pathset* ps, bool view_exact) {
   CKS(materialize_zero(ps));
   {  // (re)build lists and stats; counts emitted with the rows stay - the rows have not changed
     uint32_t* pcnt = ps->view.pcnt;
+    unsigned long long* fp = ps->view.fp;
     const unsigned long long gen = ps->view.pcnt_gen, elo = ps->view.emit_lo, ehi = ps->view.emit_hi;
     const int layout = ps->view.pcnt_layout;
     ps->view.pcnt = nullptr;
+    ps->view.fp = nullptr;
     drop_view(ps);
     ps->view.pcnt = pcnt;
+    ps->view.fp = fp;
     ps->view.pcnt_gen = gen;
     ps->view.pcnt_layout = layout;
     ps->view.emit_lo = elo;
@@ -1629,6 +1651,8 @@ static int ensure_precount(gcre_exec* ex, gcre_pathset* ps) {
   dev_free(ex, ps->view.pcnt);
   ps->view.pcnt = nullptr;
   ps->view.pcnt_layout = 0;
+  dev_free(ex, ps->view.fp);  // emitted over the rows the table covered; the new table covers every row
+  ps->view.fp = nullptr;
   const long long items = (long long)ps->size * ex->M;
   const int nb = ex->Iw / 32;
   CK(dev_alloc(ex, (void**)&ps->view.pcnt, std::max<size_t>((size_t)items * nb, 1) * 2048));
@@ -1753,7 +1777,9 @@ static int build_uidset(gcre_exec* ex, int path_length, const gcre_uid_ref* uids
                         gcre_uidset* us) {
   static_assert(sizeof(UidRefPOD) == sizeof(gcre_uid_ref), "uid_ref layout");
   us->ex = ex;
-  for (DevBuf* b : {&us->count, &us->loc, &us->prefix, &us->res, &us->units, &us->unit_idx, &us->signs}) b->owner = ex;
+  for (DevBuf* b : {&us->count, &us->loc, &us->prefix, &us->res, &us->units, &us->unit_idx, &us->signs, &us->grp.mem_rng, &us->grp.members,
+                    &us->grp.unit_list})
+    b->owner = ex;
   us->path_length = path_length;
   us->n_uids = n_uids;
   us->n_signs = n_signs;
@@ -1834,6 +1860,10 @@ static void free_uidset_buffers(gcre_uidset* us) {
   us->units.release();
   us->unit_idx.release();
   us->signs.release();
+  us->grp.mem_rng.release();
+  us->grp.members.release();
+  us->grp.unit_list.release();
+  us->grp.built = false;
 }
 
 extern "C" int gcre_uidset_create(gcre_exec* ex, int path_length, const gcre_uid_ref* uids, uint32_t n_uids, const int32_t* signs,
@@ -1895,6 +1925,9 @@ struct JoinKnobs {
   int thr = env_01("GCRE_THR");            // 0 / 1: thresholded look-ups off / on for every join
   int precount = env_precount();           // PRECOUNT_NO / _YES / _SAMPLE for every join the budget allows (precount_mode)
   int tail = env_01("GCRE_TEST_TAIL");     // 0 / 1: the tail form never / on joins of any size
+  int dedup = env_01("GCRE_TEST_DEDUP");   // 0 / 1: grouping of equal upstream rows never / on joins of any size, however few duplicates
+  bool dedup_collide = env_01("GCRE_TEST_DEDUP_COLLIDE") == 1;  // grouping keys without the fingerprints: every row of a partner
+                                                                // range collides and only the word compare tells
   int sc_pts = env_01("GCRE_SC_PTS");      // 0 / 1: the shared-memory form of the split-carrier kernels off / on where it fits
   bool no_emit = env_01("GCRE_TEST_EMIT") == 0;  // kept rows do not take their counts along
   // every launch-plan size shrunk, so the prefix / budget-overflow / redo paths of run_launch_plan run on tiny joins
@@ -1929,6 +1962,7 @@ struct JoinForm {
   bool thr = false;                          // thresholded look-ups
   int layout = 0;                            // count-table layout: 0, or the split-carrier kernels' words per lane group
   size_t entry_bytes = 0;                    // bytes of one (row, half) entry of a count table in that layout
+  const gcre_uidset::Grouping* grp = nullptr;  // representatives of equal upstream rows only (group_upstream_rows)
 };
 
 // the kernel parameters that name a join's operands and its index: the pairs, whatever the form
@@ -1962,6 +1996,120 @@ static int sample_overlap(gcre_exec* ex, const gcre_uidset* us, const gcre_paths
   CK(cudaMemcpyAsync(ex->h_scalars + 8, d_sums, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ex->stream));
   CK(cudaStreamSynchronize(ex->stream));
   memcpy(sums, ex->h_scalars + 8, 2 * sizeof(unsigned long long));
+  return GCRE_OK;
+}
+
+// Grouping of equal upstream rows (setup_kernels.cuh: group_*).  A score-only join scores one representative of rows with equal
+// bits and equal index entries, and its candidates are taken in for the other rows too (expand_members).  Measured on B200 at
+// 1,000 W with the level-4 join of BASELINE config 3 (1.35 M upstream rows, 12 M pairs; profiles/r7_*): the set-up costs 0.95 /
+// 1.05 ms per join (methods 1 / 2; the word compare of the members 0.70 / 0.79 of it, the sort 0.17), the fingerprints 0.38 ms of
+// the level-3 join that emits them; 827 K / 766 K rows are members, and the join kernel falls from 5.9 / 11.3 to
+// 2.6 / 5.7 ms.  GROUP_MIN_PAIRS: smaller joins do not group (below ~1 M pairs the whole join takes about what the set-up
+// takes).  GROUP_MAX_UNIT_SHARE: the grouping is used when the representatives keep at most this share of the units - the
+// kernel time saved, (1 - share) x 5.9 ms for method 1, then still pays for the ~1 ms set-up (break-even ~0.83; method 2 ~0.91).
+constexpr unsigned long long GROUP_MIN_PAIRS = 1ull << 20;
+constexpr double GROUP_MAX_UNIT_SHARE = 0.8;
+
+struct MaxU32 {
+  __device__ __forceinline__ uint32_t operator()(uint32_t a, uint32_t b) const { return a > b ? a : b; }
+};
+
+// The grouping of upstream rows [ub, ue) of the join, built or found current on the join index.  One read-back.
+static int group_upstream_rows(const JoinCall& c, const gcre_uidset::Grouping** out) {
+  gcre_exec* ex = c.ex;
+  const gcre_uidset* us = c.us;
+  gcre_uidset::Grouping& g = us->grp;
+  const gcre_pathset* p0 = c.paths0;
+  const bool collide = c.knobs.dedup_collide;
+  *out = nullptr;
+  if (!(g.built && g.set_uid == p0->uid && g.set_ver == p0->ver && g.ub == c.ub && g.ue == c.ue && g.collide == collide)) {
+    g.built = false;
+    const uint32_t n = c.ue - c.ub;
+    const unsigned long long n_units = c.unit_hi - c.unit_lo;
+    const int32_t* signs = ex->M == 2 && us->path_length >= 3 ? (const int32_t*)us->signs.p : nullptr;  // need_flip reads signs[idx]
+    unsigned long long *keys = nullptr, *keys_s = nullptr;
+    uint32_t *rows = nullptr, *rows_s = nullptr, *head = nullptr, *member = nullptr, *slot = nullptr, *unit_ids = nullptr;
+    unsigned long long* d_out = nullptr;  // [0] representatives' units, [1] members
+    uint8_t *is_rep = nullptr, *flags = nullptr;
+    int rc = [&]() -> int {
+      CK(dev_alloc(ex, (void**)&keys, (size_t)n * 8));
+      CK(dev_alloc(ex, (void**)&keys_s, (size_t)n * 8));
+      CK(dev_alloc(ex, (void**)&rows, (size_t)n * 4));
+      CK(dev_alloc(ex, (void**)&rows_s, (size_t)n * 4));
+      CK(dev_alloc(ex, (void**)&head, (size_t)n * 4));
+      CK(dev_alloc(ex, (void**)&member, ((size_t)n + 1) * 4));
+      CK(dev_alloc(ex, (void**)&slot, ((size_t)n + 1) * 4));
+      CK(dev_alloc(ex, (void**)&is_rep, std::max<size_t>(us->n_uids, 1)));
+      CK(dev_alloc(ex, (void**)&unit_ids, std::max<size_t>(n_units, 1) * 4));
+      CK(dev_alloc(ex, (void**)&flags, std::max<size_t>(n_units, 1)));
+      CK(dev_alloc(ex, (void**)&d_out, 2 * sizeof(unsigned long long)));
+      CK(cudaMemsetAsync(d_out, 0, 2 * sizeof(unsigned long long), ex->stream));
+      CKS(g.mem_rng.ensure(std::max<size_t>(us->n_uids, 1) * sizeof(uint2)));
+      CKS(g.members.ensure(std::max<size_t>(n, 1) * 4));
+      CKS(g.unit_list.ensure(std::max<size_t>(n_units, 1) * 4));
+      size_t b_sort = 0, b_max = 0, b_sum = 0, b_sel = 0;
+      CK(cub::DeviceRadixSort::SortPairs(nullptr, b_sort, keys, keys_s, rows, rows_s, (int)n, 0, 64, ex->stream));
+      CK(cub::DeviceScan::InclusiveScan(nullptr, b_max, head, head, MaxU32(), (int)n, ex->stream));
+      CK(cub::DeviceScan::ExclusiveSum(nullptr, b_sum, member, slot, (int)n + 1, ex->stream));
+      CK(cub::DeviceSelect::Flagged(nullptr, b_sel, unit_ids, flags, (uint32_t*)g.unit_list.p, d_out, (long long)n_units, ex->stream));
+      const size_t tmp_bytes = std::max(std::max(b_sort, b_max), std::max(b_sum, b_sel));
+      CKS(ex->scan_tmp.ensure(tmp_bytes));
+      void* tmp = ex->scan_tmp.p;
+      size_t tb = tmp_bytes;
+      group_keys_kernel<<<grid_for(n, 256), 256, 0, ex->stream>>>(c.ub, n, collide ? nullptr : p0->view.fp, (const int32_t*)us->count.p,
+                                                                  (const uint32_t*)us->loc.p, signs, keys, rows);
+      CK(cudaGetLastError());
+      LAUNCHED();
+      CK(cub::DeviceRadixSort::SortPairs(tmp, tb, keys, keys_s, rows, rows_s, (int)n, 0, 64, ex->stream));
+      LAUNCHED();
+      group_heads_kernel<<<grid_for(n, 256), 256, 0, ex->stream>>>(n, keys_s, head);
+      CK(cudaGetLastError());
+      LAUNCHED();
+      tb = tmp_bytes;
+      CK(cub::DeviceScan::InclusiveScan(tmp, tb, head, head, MaxU32(), (int)n, ex->stream));
+      LAUNCHED();
+      group_verify_kernel<<<grid_for((long long)n * 32, 256), 256, 0, ex->stream>>>(n, rows_s, head, p0->d_rows, (int)row_words(ex),
+                                                                                   (const int32_t*)us->count.p, (const uint32_t*)us->loc.p, signs, member);
+      CK(cudaGetLastError());
+      LAUNCHED();
+      CK(cudaMemsetAsync(member + n, 0, 4, ex->stream));
+      tb = tmp_bytes;
+      CK(cub::DeviceScan::ExclusiveSum(tmp, tb, member, slot, (int)n + 1, ex->stream));
+      LAUNCHED();
+      CK(cudaMemsetAsync(g.mem_rng.p, 0, (size_t)us->n_uids * sizeof(uint2), ex->stream));
+      group_finish_kernel<<<grid_for(n, 256), 256, 0, ex->stream>>>(n, rows_s, head, member, slot, (uint32_t*)g.members.p, (uint2*)g.mem_rng.p, is_rep);
+      CK(cudaGetLastError());
+      LAUNCHED();
+      group_unit_flags_kernel<<<grid_for((long long)n_units, 256), 256, 0, ex->stream>>>(c.unit_lo, n_units, (const uint32_t*)us->unit_idx.p, is_rep,
+                                                                                        unit_ids, flags);
+      CK(cudaGetLastError());
+      LAUNCHED();
+      tb = tmp_bytes;
+      CK(cub::DeviceSelect::Flagged(tmp, tb, unit_ids, flags, (uint32_t*)g.unit_list.p, d_out, (long long)n_units, ex->stream));
+      LAUNCHED();
+      CK(cudaMemcpyAsync(d_out + 1, slot + n, 4, cudaMemcpyDeviceToDevice, ex->stream));
+      CK(cudaMemcpyAsync(ex->h_scalars + 8, d_out, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ex->stream));
+      CK(cudaStreamSynchronize(ex->stream));
+      unsigned long long h[2];
+      memcpy(h, ex->h_scalars + 8, sizeof h);
+      g.n_units = h[0];
+      g.dedup_rows = (uint32_t)h[1];
+      g.pays = (double)g.n_units <= GROUP_MAX_UNIT_SHARE * (double)n_units;
+      g.set_uid = p0->uid;
+      g.set_ver = p0->ver;
+      g.ub = c.ub;
+      g.ue = c.ue;
+      g.collide = collide;
+      g.h_members_valid = false;
+      g.built = true;
+      return GCRE_OK;
+    }();
+    for (void* p : {(void*)keys, (void*)keys_s, (void*)rows, (void*)rows_s, (void*)head, (void*)member, (void*)slot, (void*)is_rep, (void*)unit_ids,
+                    (void*)flags, (void*)d_out})
+      dev_free(ex, p);
+    CKS(rc);
+  }
+  if (g.pays || c.knobs.dedup == 1) *out = &g;
   return GCRE_OK;
 }
 
@@ -2036,6 +2184,12 @@ static int choose_join_form(const JoinCall& c, int requested, long long t_needed
     if (sel_base) f->map1 = sel.sel;
     else CKS(identity_map(ex, c.paths1->size, &f->map1));
   }
+  // score-only joins whose upstream rows carry fingerprints score each group of equal rows once; GCRE_TEST_DEDUP=1 / 0 (test
+  // hook) groups on joins of any size / never
+  if (!c.keep && pairs > 0 && v0.fp && c.ub >= v0.emit_lo && c.ue <= v0.emit_hi && c.ue > c.ub) {
+    const bool want = c.knobs.dedup >= 0 ? c.knobs.dedup == 1 : pairs >= GROUP_MIN_PAIRS;
+    if (want) CKS(group_upstream_rows(c, &f->grp));
+  }
   return GCRE_OK;
 }
 
@@ -2070,6 +2224,8 @@ static int prepare_join_operands(const JoinCall& c, const JoinForm& f, JoinParam
       res->view.pcnt_layout = f.layout;
       CK(dev_alloc(ex, (void**)&res->view.len, items * 4));
       CK(dev_alloc(ex, (void**)&res->view.ncase, items * 4));
+      CK(dev_alloc(ex, (void**)&res->view.fp, std::max<size_t>(res->size, 1) * 8));
+      sp->fp_res = res->view.fp;
       sp->pcnt_res = res->view.pcnt;
       sp->len_res = res->view.len;
       sp->ncase_res = res->view.ncase;
@@ -2098,6 +2254,9 @@ static int prepare_join_operands(const JoinCall& c, const JoinForm& f, JoinParam
     jp->slots = ex->d_topk + 1;
     jp->n_slots = c.top_k;
   }
+  if (f.grp) {
+    sp->unit_list = (const uint32_t*)f.grp->unit_list.p;
+  }
   return GCRE_OK;
 }
 
@@ -2108,6 +2267,47 @@ struct LaunchStats {  // of one join's launch plan (gcre_join_opts)
   bool shared_masks = false;
 };
 
+// Grouped upstream rows: the candidates `cand` of representatives, taken in by the host, are also candidates of the member rows
+// of their rows - the same pair but for the row, so the same score and counts.  Of a group only the first top_k - 1 members can
+// be among the K best with a given partner (ties go to the smaller row), so no more are taken in.  One small gather of the
+// candidates' member ranges on the device; the members themselves are read back once per grouping, when first needed.
+static int expand_members(gcre_exec* ex, const gcre_uidset::Grouping& g, const std::vector<Cand>& cand, int top_k, std::vector<gcre_score>* held) {
+  const unsigned n = (unsigned)cand.size();
+  if (n == 0 || g.dedup_rows == 0 || top_k < 2) return GCRE_OK;
+  CKS(ex->scratch.ensure((size_t)n * (sizeof(uint32_t) + sizeof(uint2)) + 8));
+  uint32_t* d_rows = (uint32_t*)ex->scratch.p;
+  uint2* d_rng = (uint2*)(d_rows + n + (n & 1));
+  std::vector<uint32_t> rows(n);
+  for (unsigned k = 0; k < n; k++) rows[k] = cand[k].idx;
+  std::vector<uint2> rng(n);
+  CK(cudaMemcpyAsync(d_rows, rows.data(), (size_t)n * 4, cudaMemcpyHostToDevice, ex->stream));
+  group_ranges_kernel<<<grid_for(n, 256), 256, 0, ex->stream>>>(n, d_rows, (const uint2*)g.mem_rng.p, d_rng);
+  CK(cudaGetLastError());
+  LAUNCHED();
+  CK(cudaMemcpyAsync(rng.data(), d_rng, (size_t)n * sizeof(uint2), cudaMemcpyDeviceToHost, ex->stream));
+  CK(cudaStreamSynchronize(ex->stream));
+  for (unsigned k = 0; k < n; k++) {
+    if (rng[k].y <= rng[k].x) continue;
+    if (!g.h_members_valid) {
+      g.h_members.resize(g.dedup_rows);
+      CK(cudaMemcpyAsync(g.h_members.data(), g.members.p, (size_t)g.dedup_rows * 4, cudaMemcpyDeviceToHost, ex->stream));
+      CK(cudaStreamSynchronize(ex->stream));
+      g.h_members_valid = true;
+    }
+    const uint32_t e = std::min<uint32_t>(rng[k].y, rng[k].x + (uint32_t)(top_k - 1));
+    for (uint32_t m = rng[k].x; m < e; m++) {
+      gcre_score sc;
+      sc.score = key_score(cand[k].key);
+      sc.src = (int32_t)g.h_members[m];
+      sc.trg = (int32_t)cand[k].loc;
+      sc.cases = cand[k].cases;
+      sc.ctrls = cand[k].ctrls;
+      held->push_back(sc);
+    }
+  }
+  return GCRE_OK;
+}
+
 // The join's launches; their candidates are merged on the host into the top-K `held`.
 static int run_launch_plan(const JoinCall& c, const JoinForm& f, JoinParams jp, SparseParams sp, PhaseTrace& tr, std::vector<gcre_score>* held,
                            LaunchStats* st) {
@@ -2115,7 +2315,8 @@ static int run_launch_plan(const JoinCall& c, const JoinForm& f, JoinParams jp, 
   // dense kernel: chunks are ranges of flattened pairs; sparse kernel: ranges of units (<= PB pairs each)
   const bool sparse_k = f.kernel == GCRE_KERNEL_SPARSE;
   const unsigned long long per_item = sparse_k ? sparse::PB : 1;
-  const unsigned long long item_lo = sparse_k ? c.unit_lo : c.pair_lo, item_hi = sparse_k ? c.unit_hi : c.pair_hi;
+  // (grouped upstream rows: items index the representatives' units, in ascending order)
+  const unsigned long long item_lo = f.grp ? 0 : sparse_k ? c.unit_lo : c.pair_lo, item_hi = f.grp ? f.grp->n_units : sparse_k ? c.unit_hi : c.pair_hi;
   // Launch plan.  Top-K candidates are appended by the kernels only when their score beats the K-th best known so far,
   // and a launch must be able to hold every candidate it may produce:
   //   * small joins (<= 64K pairs): one launch with room for every pair;
@@ -2126,6 +2327,9 @@ static int run_launch_plan(const JoinCall& c, const JoinForm& f, JoinParams jp, 
   //     across launches, so later pairs only displace on a strictly greater score.  If the budget overflows (scores that
   //     keep rising), that launch's candidates are dropped and the range is redone in safe chunks (cap = chunk size);
   //     permutation maxima are max-merged, so re-scoring a pair is harmless.
+  // With grouped upstream rows the kernels append the representatives' candidates only; each is then also a candidate of the
+  // first top_k - 1 members of its row (expand_members).  The K-th score no longer rules out a tie in later launches (a member
+  // taken in early has a larger row than a representative of a later launch), so ties with it stay candidates.
   struct Seg { unsigned long long b, e; bool safe; };
   std::vector<Seg> plan;
   const bool tiny_plan = c.knobs.small_plan;
@@ -2219,12 +2423,14 @@ static int run_launch_plan(const JoinCall& c, const JoinForm& f, JoinParams jp, 
         sc.ctrls = h_cand[k].ctrls;
         held->push_back(sc);
       }
+      if (f.grp) CKS(expand_members(ex, *f.grp, h_cand, c.top_k, held));
       trim_topk(*held, c.top_k);
       if ((int)held->size() == c.top_k) {
         double kth = (*held)[0].score;
         for (const auto& sc : *held) kth = std::min(kth, sc.score);
-        // later launches hold larger (src, trg) only, so a tie with the K-th score can no longer win a place
-        thr_key = score_key(kth);
+        // later launches hold larger (src, trg) only, so a tie with the K-th score can no longer win a place (with grouped rows
+        // it can: ties stay candidates)
+        thr_key = score_key(kth) - (f.grp ? 1 : 0);
       }
     }
     tr.mark("cands");
@@ -2338,6 +2544,7 @@ static int join_impl(gcre_exec* ex, const gcre_uidset* us, const gcre_pathset* p
     opts->launches = st.launches;
     opts->precounted = form.precount;
     opts->tail_form = form.pc_set != nullptr && !form.precount;
+    opts->dedup_rows = form.grp ? form.grp->dedup_rows : 0;
     opts->split_carrier = form.split;
     opts->shared_masks = st.shared_masks;
     opts->thresholded = form.thr && st.launches > 0 ? 1 : 0;

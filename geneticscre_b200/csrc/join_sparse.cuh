@@ -98,6 +98,9 @@ struct SparseView {
   // rows whose counts / ranges / len / ncase were emitted: a KEEP join over a shard of its upstream rows (multi-GPU: each
   // rank builds only the rows its shard of the next level consumes) fills [emit_lo, emit_hi) only
   unsigned long long emit_lo = 0, emit_hi = 0;
+  // per row, a 64-bit hash of its words (row_fingerprint), emitted with the counts over the same [emit_lo, emit_hi): what the
+  // grouping of equal upstream rows (gcre_capi.cu: group_upstream_rows) sorts by.  Null for rows no join wrote.
+  unsigned long long* fp = nullptr;
 };
 
 struct SparseParams {
@@ -116,6 +119,8 @@ struct SparseParams {
   uint32_t* ncase_res;
   unsigned long long* exact_pairs;        // diagnostic (thresholded look-ups): pairs whose exact permutation scores had to be looked up
   const uint32_t* map1;                   // PC kernels: per partner row, the row of the pre-counted set it is scored through << 1 | halves swapped
+  const uint32_t* unit_list;              // grouped upstream rows: the representatives' units; launch item k is unit unit_list[k], else unit k
+  unsigned long long* fp_res;             // KEEP: where to emit the kept rows' fingerprints, else null
 };
 
 // ---- view construction ----------------------------------------------------------------------------------------------
@@ -310,6 +315,16 @@ __device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefe
 __device__ __forceinline__ void prefetch_l1(const void* p) { asm volatile("prefetch.global.L1 [%0];" ::"l"(p)); }
 
 // ---- per pair, shared with join_sparse_sc.cuh ----
+// 64-bit hash of 16 bytes of a row at 16-byte position pos (SparseView::fp sums it over the row)
+__device__ __forceinline__ unsigned long long row_fp_part(unsigned long long w0, unsigned long long w1, unsigned pos) {
+  unsigned long long h = (w0 ^ (((w1 << 31) | (w1 >> 33)) * 0x9E3779B97F4A7C15ull)) + (pos + 1ull) * 0xD6E8FEB86659FD93ull;
+  h ^= h >> 33;
+  h *= 0xFF51AFD7ED558CCDull;
+  h ^= h >> 33;
+  h *= 0xC4CEB9FE1A85EC53ull;
+  return h ^ (h >> 33);
+}
+
 // the kept joined row (src/join_base.cpp:246-249) = upstream row | partner row, written to result row r.  16-byte accesses (Wp is
 // even, rows are 16-byte aligned), streaming stores: the row is next read by the following level's join.  At 100,000 patients a
 // row is 12.5 KB per half and this copy is most of a KEEP join.  Wp: the caller's copy of a.Wp (re-read from the parameters here,
@@ -331,6 +346,22 @@ __device__ __forceinline__ void store_kept_row(const JoinParams& a, int Wp, cons
       __stcs(out + Wv + k, make_ulonglong2(xn.x | yn.x, xn.y | yn.y));
     }
   }
+}
+
+// The fingerprint of kept row r (SparseView::fp): a function of the row's words alone, whichever kernel wrote it - read back
+// from L2 right behind store_kept_row.  Out of line: formed in the store loop it cost every KEEP instance registers and spills.
+// Warp-uniform call.
+__device__ __noinline__ void store_kept_fp(const SparseParams& s, const JoinParams& a, int row_words, size_t r, int lane) {
+  __syncwarp();
+  const ulonglong2* row = reinterpret_cast<const ulonglong2*>(a.pres + r * row_words);
+  unsigned long long fp = 0;
+  for (int k = lane; k < row_words / 2; k += 32) {
+    const ulonglong2 x = __ldcg(row + k);
+    fp += row_fp_part(x.x, x.y, (unsigned)k);
+  }
+#pragma unroll
+  for (int d = 16; d > 0; d >>= 1) fp += __shfl_xor_sync(0xffffffffu, fp, d);
+  if (lane == 0) s.fp_res[r] = fp;
 }
 
 // the carrier totals of half h of kept row r, beside its emitted counts (t0 / nc0: the upstream half's, nd / ncn: what the
@@ -493,7 +524,7 @@ __global__ void __launch_bounds__(sparse::THREADS, sparse::min_blocks(M, THR)) j
     g = __shfl_sync(0xffffffffu, g, 0);
     if (g >= n_work) break;
     const int pb = (int)(g / s.n_units);
-    const unsigned long long unit = s.unit_begin + (g % s.n_units);
+    const unsigned long long unit = s.unit_list ? s.unit_list[s.unit_begin + (g % s.n_units)] : s.unit_begin + (g % s.n_units);
     if (THR) {
       if (pb != pb_cur || (++since_refresh & 7u) == 0u) {  // other warps keep raising the maxima: re-read every 8th unit
         thr = load_thr(pb);
@@ -856,7 +887,11 @@ __global__ void __launch_bounds__(sparse::THREADS, sparse::min_blocks(M, THR)) j
 
       // on the first permutation block only: the kept row, the true score and the candidate
       if (first_pb) {
-        if (KEEP) store_kept_row<M>(a, Wp, p0row, loc, (size_t)(a.res_idx[idx] + j), flip, lane);
+        if (KEEP) {
+          const size_t r = (size_t)(a.res_idx[idx] + j);
+          store_kept_row<M>(a, Wp, p0row, loc, r, flip, lane);
+          if (s.fp_res) store_kept_fp(s, a, row_words, r, lane);
+        }
         const uint32_t park = (j - j0) & 31u;
         if (lane == 0) park_totals<M>(s_park[warp][park], t0, nd, nc0, ncn);
         if (park == 31u || j + 1 == j1) score_parked<M, KEEP>(a, s_park[warp], park, idx, loc, lane);

@@ -214,7 +214,7 @@ __global__ void __launch_bounds__(PTS ? sparse_sc::PTS_THREADS : sparse_sc::THRE
     if (lane == 0) g = atomicAdd(s.work_counter, 1ull);
     g = __shfl_sync(0xffffffffu, g, 0);
     if (g >= s.n_units) break;
-    const unsigned long long unit = s.unit_begin + g;
+    const unsigned long long unit = s.unit_list ? s.unit_list[s.unit_begin + g] : s.unit_begin + g;
     const uint32_t idx = s.unit_idx[unit];
     const uint32_t subu = (uint32_t)(unit - s.unit_prefix[idx]);
     const uint32_t cnt_idx = (uint32_t)a.count[idx];
@@ -485,6 +485,7 @@ __global__ void __launch_bounds__(PTS ? sparse_sc::PTS_THREADS : sparse_sc::THRE
           }
         }
         store_kept_row<M>(a, Wp, p0row, loc, r, flip, lane);
+        if (s.fp_res) store_kept_fp(s, a, row_words, r, lane);
       }
       if (lane == 0) park_totals<M>(s_park[warp][park], t0, nd, nc0, ncn);
       if (park == 31u || j + 1 == j1) score_parked<M, KEEP>(a, s_park[warp], park, idx, loc, lane);

@@ -301,4 +301,94 @@ __global__ void tail_eligible_kernel(unsigned long long unit_lo, unsigned long l
   if (__any_sync(0xffffffffu, !ok) && (threadIdx.x & 31) == 0) atomicOr(bad, 1u);
 }
 
+// ---- grouping of equal upstream rows (score-only sparse joins, gcre_capi.cu: group_upstream_rows) ---------------------
+// Two upstream rows with equal bits, equal partner range (location, count) and - method 2 - equal sign have pairwise equal pairs.
+// Rows are sorted by a key of their fingerprint and those index entries; each row of a run of equal keys is then compared with
+// the run's first row (its smallest) word for word, and becomes its member only if everything is equal.
+__device__ __forceinline__ unsigned long long group_mix(unsigned long long h, unsigned long long v) {
+  h ^= v + 0x9E3779B97F4A7C15ull + (h << 6) + (h >> 2);
+  h ^= h >> 31;
+  h *= 0xBF58476D1CE4E5B9ull;
+  return h ^ (h >> 29);
+}
+
+// key and value of sort position i: upstream row ub + i.  signs: null unless the pairs' orientation depends on the upstream row;
+// fp: null for the test hook that makes every row of a partner range collide
+__global__ void group_keys_kernel(uint32_t ub, uint32_t n, const unsigned long long* __restrict__ fp, const int32_t* __restrict__ count,
+                                  const uint32_t* __restrict__ location, const int32_t* __restrict__ signs, unsigned long long* __restrict__ keys,
+                                  uint32_t* __restrict__ rows) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const uint32_t u = ub + i;
+  unsigned long long h = group_mix(fp ? fp[u] : 0ull, ((unsigned long long)location[u] << 32) | (uint32_t)count[u]);
+  if (signs) h = group_mix(h, (uint32_t)signs[u]);
+  keys[i] = h;
+  rows[i] = u;
+}
+
+// run starts: position i when its key differs from the previous one, else 0 (a max-scan turns this into each position's run start)
+__global__ void group_heads_kernel(uint32_t n, const unsigned long long* __restrict__ keys, uint32_t* __restrict__ head) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) head[i] = (i == 0 || keys[i] != keys[i - 1]) ? i : 0u;
+}
+
+// one warp per sort position: member[i] = 1 when the row equals its run's first row in every word and index entry
+__global__ void group_verify_kernel(uint32_t n, const uint32_t* __restrict__ rows, const uint32_t* __restrict__ head, const uint64_t* __restrict__ p0,
+                                    int row_words, const int32_t* __restrict__ count, const uint32_t* __restrict__ location,
+                                    const int32_t* __restrict__ signs, uint32_t* __restrict__ member) {
+  const int lane = threadIdx.x & 31;
+  const unsigned long long i = ((unsigned long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  if (i >= n) return;
+  const uint32_t h = head[i];
+  bool eq = h != (uint32_t)i;
+  if (eq) {
+    const uint32_t a = rows[h], b = rows[i];
+    eq = count[a] == count[b] && location[a] == location[b] && (!signs || signs[a] == signs[b]);
+    if (eq) {
+      const ulonglong2* x = reinterpret_cast<const ulonglong2*>(p0 + (size_t)a * row_words);
+      const ulonglong2* y = reinterpret_cast<const ulonglong2*>(p0 + (size_t)b * row_words);
+      bool same = true;
+      for (int k = lane; k < row_words / 2; k += 32) {
+        const ulonglong2 u = __ldg(x + k), v = __ldg(y + k);
+        same &= u.x == v.x && u.y == v.y;
+      }
+      eq = __all_sync(0xffffffffu, same);
+    }
+  }
+  if (lane == 0) member[i] = eq ? 1u : 0u;
+}
+
+// slot[i]: exclusive running count of members.  A member's row goes to members[slot[i]]; a run's first row gets the range of its
+// members (the verified rows of its run, ascending: the sort is stable over ascending rows); every row is marked representative
+// or not.  mem_rng must be zero beforehand (rows without members).
+__global__ void group_finish_kernel(uint32_t n, const uint32_t* __restrict__ rows, const uint32_t* __restrict__ head, const uint32_t* __restrict__ member,
+                                    const uint32_t* __restrict__ slot, uint32_t* __restrict__ members, uint2* __restrict__ mem_rng,
+                                    uint8_t* __restrict__ is_rep) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const uint32_t u = rows[i];
+  is_rep[u] = member[i] ? 0 : 1;
+  if (member[i]) members[slot[i]] = u;
+  if (head[i] == i) {
+    mem_rng[u].x = slot[i];
+    if (i > 0) mem_rng[rows[head[i - 1]]].y = slot[i];
+  }
+  if (i == n - 1) mem_rng[rows[head[i]]].y = slot[n];
+}
+
+// the member range of each of n candidate rows (gcre_capi.cu: expand_members)
+__global__ void group_ranges_kernel(uint32_t n, const uint32_t* __restrict__ rows, const uint2* __restrict__ mem_rng, uint2* __restrict__ out) {
+  const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
+  if (k < n) out[k] = mem_rng[rows[k]];
+}
+
+// the representatives' units of [unit_lo, unit_hi), flagged for compaction
+__global__ void group_unit_flags_kernel(unsigned long long unit_lo, unsigned long long n_units, const uint32_t* __restrict__ unit_idx,
+                                        const uint8_t* __restrict__ is_rep, uint32_t* __restrict__ unit_ids, uint8_t* __restrict__ flags) {
+  const unsigned long long q = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (q >= n_units) return;
+  unit_ids[q] = (uint32_t)(unit_lo + q);
+  flags[q] = is_rep[unit_idx[unit_lo + q]];
+}
+
 }  // namespace gcre

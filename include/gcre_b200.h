@@ -91,7 +91,8 @@ typedef struct {
                                had to be looked up; every other pair was ruled out by one compare per look-up */
   int32_t tail_form;        /* out: 1 when the pre-counted form ran against the gene rows of the base set the partner rows were
                                selected from (join_sparse.cuh, tail form: every partner adds one gene to its upstream path) */
-  int32_t reserved2;
+  uint32_t dedup_rows;      /* out: upstream rows not scored because they equal a smaller row of the join in every word and index
+                               entry (score-only sparse joins): that row's candidates were appended for them too */
 } gcre_join_opts;
 
 /* One split of a reported path for the decorated p-value (R/DecoratedPvalue.R:198-304). */
