@@ -49,6 +49,8 @@ SYMBOLS = {
     "gcre_exec_destroy": (_I, [_VP]),
     "gcre_exec_get_info": (_I, [_VP, C.POINTER(ExecInfoC)]),
     "gcre_exec_decorated_exact": (_I, [_VP, C.POINTER(C.c_uint64), _U32, C.POINTER(DecoratedC)]),
+    "gcre_exec_decorated_paths": (_I, [_VP, _VP, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_int32), _U32, _I,
+                                       C.POINTER(DecoratedC)]),
     "gcre_exec_set_stream": (_I, [_VP, _VP]),
     "gcre_exec_set_value_table": (_I, [_VP, C.POINTER(C.c_double), _I, _I]),
     "gcre_exec_generate_value_table": (_I, [_VP]),

@@ -830,6 +830,24 @@ extern "C" int gcre_exec_get_value_table(const gcre_exec* ex, double* out, int r
   return GCRE_OK;
 }
 
+// Scratch budget of the decorated p-value calls: splits run in chunks whose scratch fits it (one larger split runs alone).
+// GCRE_TEST_DECORATED_SCRATCH (test hook, bytes; read per call) shrinks it so that a short list spans several chunks.
+static size_t decorated_scratch_budget() {
+  if (const char* e = std::getenv("GCRE_TEST_DECORATED_SCRATCH")) return std::max<size_t>(1, std::strtoull(e, nullptr, 10));
+  return (size_t)256 << 20;
+}
+
+// decorated_exact_kernel over ni packed splits (d_rows [ni][4][W64]); d_scr: ni * 2 * (n + 1) doubles
+static int launch_decorated_exact(gcre_exec* ex, const uint64_t* d_rows, uint32_t ni, double* d_scr, DecoratedOut* d_out) {
+  if (ex->M == 1)
+    decorated_exact_kernel<1><<<ni, DEC_THREADS, 0, ex->stream>>>(d_rows, ni, ex->W64, ex->n_cases, ex->n_ctrls, ex->d_vt, ex->vt_rows, ex->vt_cols, d_scr, d_out);
+  else
+    decorated_exact_kernel<2><<<ni, DEC_THREADS, 0, ex->stream>>>(d_rows, ni, ex->W64, ex->n_cases, ex->n_ctrls, ex->d_vt, ex->vt_rows, ex->vt_cols, d_scr, d_out);
+  CK(cudaGetLastError());
+  LAUNCHED();
+  return GCRE_OK;
+}
+
 // computeDecoratedPvalue (R/DecoratedPvalue.R:198-304) in its exact limit for n_items splits; see decorated.cuh.
 extern "C" int gcre_exec_decorated_exact(gcre_exec* ex, const uint64_t* rows, uint32_t n_items, gcre_decorated* out) {
   static_assert(sizeof(gcre_decorated) == sizeof(DecoratedOut), "gcre_decorated layout");
@@ -838,7 +856,7 @@ extern "C" int gcre_exec_decorated_exact(gcre_exec* ex, const uint64_t* rows, ui
   if (!ex->d_vt) return fail(GCRE_ERR_ASSERT, "assertion");  // no value table set
   if (!n_items) return GCRE_OK;
   const size_t per_item = 2 * ((size_t)ex->n + 1) * 8;                                  // scratch: two probability vectors
-  const uint32_t chunk = (uint32_t)std::max<size_t>(1, std::min<size_t>(n_items, ((size_t)256 << 20) / per_item));
+  const uint32_t chunk = (uint32_t)std::max<size_t>(1, std::min<size_t>(n_items, decorated_scratch_budget() / per_item));
   void *d_rows = nullptr, *d_scr = nullptr, *d_out = nullptr;
   int rc = [&]() -> int {
     CK(dev_alloc(ex, &d_rows, (size_t)chunk * 4 * ex->W64 * 8));
@@ -847,14 +865,7 @@ extern "C" int gcre_exec_decorated_exact(gcre_exec* ex, const uint64_t* rows, ui
     for (uint32_t i0 = 0; i0 < n_items; i0 += chunk) {
       const uint32_t ni = std::min(chunk, n_items - i0);
       CK(cudaMemcpyAsync(d_rows, rows + (size_t)i0 * 4 * ex->W64, (size_t)ni * 4 * ex->W64 * 8, cudaMemcpyHostToDevice, ex->stream));
-      if (ex->M == 1)
-        decorated_exact_kernel<1><<<ni, DEC_THREADS, 0, ex->stream>>>((const uint64_t*)d_rows, ni, ex->W64, ex->n_cases, ex->n_ctrls, ex->d_vt, ex->vt_rows,
-                                                                      ex->vt_cols, (double*)d_scr, (DecoratedOut*)d_out);
-      else
-        decorated_exact_kernel<2><<<ni, DEC_THREADS, 0, ex->stream>>>((const uint64_t*)d_rows, ni, ex->W64, ex->n_cases, ex->n_ctrls, ex->d_vt, ex->vt_rows,
-                                                                      ex->vt_cols, (double*)d_scr, (DecoratedOut*)d_out);
-      CK(cudaGetLastError());
-      LAUNCHED();
+      CKS(launch_decorated_exact(ex, (const uint64_t*)d_rows, ni, (double*)d_scr, (DecoratedOut*)d_out));
       CK(cudaMemcpyAsync(out + i0, d_out, (size_t)ni * sizeof(DecoratedOut), cudaMemcpyDeviceToHost, ex->stream));
       CK(cudaStreamSynchronize(ex->stream));
     }
@@ -864,6 +875,152 @@ extern "C" int gcre_exec_decorated_exact(gcre_exec* ex, const uint64_t* rows, ui
   dev_free(ex, d_scr);
   dev_free(ex, d_out);
   return rc;
+}
+
+// Decorated p-values of whole paths given as gene rows of a path set; see gcre_b200.h and decorated.cuh.
+extern "C" int gcre_exec_decorated_paths(gcre_exec* ex, const gcre_pathset* genes, const int32_t* gene_idx, const int32_t* signs,
+                                         const int32_t* lengths, uint32_t n_paths, int stratified, gcre_decorated* out) {
+  if (!ex || !genes) return fail(GCRE_ERR_ARG, "null argument");
+  if (n_paths && (!gene_idx || !lengths || !out || (ex->M == 2 && !signs))) return fail(GCRE_ERR_ARG, "null argument");
+  if (genes->ex != ex) return fail(GCRE_ERR_ARG, "the gene rows belong to another exec");
+  if (stratified != 0 && stratified != 1) return fail(GCRE_ERR_ARG, "stratified must be 0 or 1");
+  if (!n_paths) return GCRE_OK;
+  CKS(use_device(ex));
+  if (!ex->d_vt) return fail(GCRE_ERR_ASSERT, "assertion");  // no value table set
+  // splits in the order of decorated_pvalues_for_path: forward j = 1 .. L-1 (genes 0 .. j-1, then gene j), backward j = L-1 .. 1
+  // (genes L-1 .. j, then gene j-1); slot[i] = path * 8 + split
+  std::vector<DecSplit> splits;
+  std::vector<uint32_t> slot;
+  splits.reserve((size_t)n_paths * 4);
+  for (uint32_t p = 0; p < n_paths; p++) {
+    const int L = lengths[p];
+    if (L < 1 || L > 5) return fail(GCRE_ERR_RANGE, "path %u: length %d is outside 1..5", p, L);
+    const int32_t* g = gene_idx + (size_t)p * 5;
+    int neg = 0;
+    for (int j = 0; j < L; j++) {
+      if (g[j] < 0 || (uint32_t)g[j] >= genes->size) return fail(GCRE_ERR_RANGE, "path %u: gene index %d is outside the gene rows", p, g[j]);
+      if (ex->M == 2) {
+        const int sg = signs[(size_t)p * 5 + j];
+        if (sg != 1 && sg != -1) return fail(GCRE_ERR_ARG, "path %u: sign %d is not +1 / -1", p, sg);
+        if (sg == -1) neg |= 1 << j;
+      }
+    }
+    uint32_t k = 0;
+    for (int j = 1; j < L; j++, k++) {
+      DecSplit s{};
+      for (int i = 0; i <= j; i++) s.gene[i] = g[i];
+      s.n_sub = j;
+      s.neg = neg & ((1 << (j + 1)) - 1);
+      splits.push_back(s);
+      slot.push_back(p * 8 + k);
+    }
+    for (int j = L - 1; j >= 1; j--, k++) {
+      DecSplit s{};
+      for (int i = L - 1; i >= j - 1; i--) {  // genes L-1 .. j, then gene j-1
+        const int at = L - 1 - i;
+        s.gene[at] = g[i];
+        s.neg |= ((neg >> i) & 1) << at;
+      }
+      s.n_sub = L - j;
+      splits.push_back(s);
+      slot.push_back(p * 8 + k);
+    }
+  }
+  CKS(materialize_zero(const_cast<gcre_pathset*>(genes)));
+  std::memset(out, 0, (size_t)n_paths * 8 * sizeof(gcre_decorated));
+  const uint32_t n_items = (uint32_t)splits.size();
+  if (!n_items) return GCRE_OK;
+  const uint64_t* d_genes = genes->d_rows;
+  const size_t stride = (size_t)ex->Wp * ex->M;  // row_words: gene rows are read in place
+  std::vector<DecoratedOut> res(n_items);
+  void *d_splits = nullptr, *d_a = nullptr, *d_b = nullptr, *d_out = nullptr, *d_tot = nullptr, *d_sizes = nullptr, *d_off = nullptr;
+  int rc = [&]() -> int {
+    CK(dev_alloc(ex, &d_splits, (size_t)n_items * sizeof(DecSplit)));
+    CK(cudaMemcpyAsync(d_splits, splits.data(), (size_t)n_items * sizeof(DecSplit), cudaMemcpyHostToDevice, ex->stream));
+    const DecSplit* sp = (const DecSplit*)d_splits;
+    if (!stratified) {  // form the packed splits on the device, then the kernel of gcre_exec_decorated_exact unchanged
+      const size_t per_item = 4 * (size_t)ex->W64 * 8 + 2 * ((size_t)ex->n + 1) * 8;
+      const uint32_t chunk = (uint32_t)std::max<size_t>(1, std::min<size_t>(n_items, decorated_scratch_budget() / per_item));
+      CK(dev_alloc(ex, &d_a, (size_t)chunk * 4 * ex->W64 * 8));
+      CK(dev_alloc(ex, &d_b, (size_t)chunk * 2 * ((size_t)ex->n + 1) * 8));
+      CK(dev_alloc(ex, &d_out, (size_t)chunk * sizeof(DecoratedOut)));
+      for (uint32_t i0 = 0; i0 < n_items; i0 += chunk) {
+        const uint32_t ni = std::min(chunk, n_items - i0);
+        decorated_form_kernel<<<ni, DEC_THREADS, 0, ex->stream>>>(d_genes, stride, sp + i0, ni, ex->W64, (uint64_t*)d_a);
+        CK(cudaGetLastError());
+        LAUNCHED();
+        CKS(launch_decorated_exact(ex, (const uint64_t*)d_a, ni, (double*)d_b, (DecoratedOut*)d_out));
+        CK(cudaMemcpyAsync(res.data() + i0, d_out, (size_t)ni * sizeof(DecoratedOut), cudaMemcpyDeviceToHost, ex->stream));
+      }
+      CK(cudaStreamSynchronize(ex->stream));
+      return GCRE_OK;
+    }
+    // stratified: one stratum when none is set; the per-patient dense indices of gcre_exec_set_permutation_strata otherwise
+    const int S = ex->n_strata > 1 ? ex->n_strata : 1;
+    const int32_t* d_strata = ex->n_strata > 1 ? ex->d_strata_idx : nullptr;
+    CK(dev_alloc(ex, &d_tot, (size_t)S * 2 * 4));
+    if (d_strata) {
+      CK(cudaMemsetAsync(d_tot, 0, (size_t)S * 2 * 4, ex->stream));
+      strata_totals_kernel<<<grid_for(ex->n, 256), 256, 0, ex->stream>>>(d_strata, ex->n, ex->n_cases, (int*)d_tot);
+      CK(cudaGetLastError());
+      LAUNCHED();
+    } else {
+      const int one[2] = {ex->n_cases, ex->n_ctrls};
+      CK(cudaMemcpyAsync(d_tot, one, sizeof(one), cudaMemcpyHostToDevice, ex->stream));
+    }
+    std::vector<int4> sizes(n_items);
+    CK(dev_alloc(ex, &d_sizes, (size_t)n_items * sizeof(int4)));
+    decorated_strata_count_kernel<<<n_items, DEC_THREADS, (size_t)4 * S * 4, ex->stream>>>(d_genes, stride, sp, n_items, ex->W64, ex->n_cases, ex->n, d_strata, S,
+                                                                                          (const int*)d_tot, (int4*)d_sizes);
+    CK(cudaGetLastError());
+    LAUNCHED();
+    CK(cudaMemcpyAsync(sizes.data(), d_sizes, (size_t)n_items * sizeof(int4), cudaMemcpyDeviceToHost, ex->stream));
+    CK(cudaStreamSynchronize(ex->stream));
+    for (uint32_t i = 0; i < n_items; i++)
+      if (sizes[i].w >= 0)  // R's sample() stops here ("cannot take a sample larger than the population")
+        return fail(GCRE_ERR_RANGE, "path %u split %u: stratum %d has fewer free patients than carriers to redraw", slot[i] / 8, slot[i] % 8, sizes[i].w);
+    // chunks whose joint-distribution scratch fits the budget; off[i] = split i's scratch offset (doubles) inside its chunk
+    std::vector<unsigned long long> off(n_items);
+    std::vector<uint32_t> cuts{0};
+    const size_t budget = decorated_scratch_budget();
+    size_t used = 0, most = 0;
+    for (uint32_t i = 0; i < n_items; i++) {
+      const size_t need = dec_joint_scratch(sizes[i].x, sizes[i].y);
+      if (i > cuts.back() && (used + need) * 8 > budget) {
+        cuts.push_back(i);
+        used = 0;
+      }
+      off[i] = used;
+      used += need;
+      most = std::max(most, used);
+    }
+    cuts.push_back(n_items);
+    CK(dev_alloc(ex, &d_off, (size_t)n_items * 8));
+    CK(cudaMemcpyAsync(d_off, off.data(), (size_t)n_items * 8, cudaMemcpyHostToDevice, ex->stream));
+    CK(dev_alloc(ex, &d_b, most * 8));
+    CK(dev_alloc(ex, &d_out, (size_t)n_items * sizeof(DecoratedOut)));
+    const size_t smem = (size_t)5 * S * 4;
+    for (size_t c = 0; c + 1 < cuts.size(); c++) {
+      const uint32_t i0 = cuts[c], ni = cuts[c + 1] - cuts[c];
+      if (ex->M == 1)
+        decorated_strata_joint_kernel<1><<<ni, DEC_THREADS, smem, ex->stream>>>(d_genes, stride, sp + i0, ni, ex->W64, ex->n_cases, ex->n_ctrls, d_strata, S,
+                                                                                (const int*)d_tot, ex->d_vt, ex->vt_rows, ex->vt_cols,
+                                                                                (const unsigned long long*)d_off + i0, (double*)d_b, (DecoratedOut*)d_out + i0);
+      else
+        decorated_strata_joint_kernel<2><<<ni, DEC_THREADS, smem, ex->stream>>>(d_genes, stride, sp + i0, ni, ex->W64, ex->n_cases, ex->n_ctrls, d_strata, S,
+                                                                                (const int*)d_tot, ex->d_vt, ex->vt_rows, ex->vt_cols,
+                                                                                (const unsigned long long*)d_off + i0, (double*)d_b, (DecoratedOut*)d_out + i0);
+      CK(cudaGetLastError());
+      LAUNCHED();
+    }
+    CK(cudaMemcpyAsync(res.data(), d_out, (size_t)n_items * sizeof(DecoratedOut), cudaMemcpyDeviceToHost, ex->stream));
+    CK(cudaStreamSynchronize(ex->stream));
+    return GCRE_OK;
+  }();
+  for (void* p : {d_splits, d_a, d_b, d_out, d_tot, d_sizes, d_off}) dev_free(ex, p);
+  if (rc != GCRE_OK) return rc;
+  for (uint32_t i = 0; i < n_items; i++) std::memcpy(&out[slot[i]], &res[i], sizeof(gcre_decorated));
+  return GCRE_OK;
 }
 
 static int rebuild_mask_layouts(gcre_exec* ex) {

@@ -6,9 +6,11 @@ without replacement among the patients the sub-path does not cover, the path is 
 decorated p-value is the share of redraws scoring at least as high as the real path (computeDecoratedPvalue,
 R/DecoratedPvalue.R:198-304).
 
-The exact, non-stratified limit also runs on the GPU (`decorated_exact_device`, csrc/decorated.cuh: one CTA per split, AND +
-popcount for the eight counts, hypergeometric weights by the ratio recurrence, value-table look-ups over the support); the
-Monte-Carlo and stratified modes are host utilities.  Only
+The exact limit also runs on the GPU (csrc/decorated.cuh: one CTA per split, AND + popcount for the eight counts,
+hypergeometric weights by the ratio recurrence, value-table look-ups over the support): `decorated_exact_device` for splits
+packed on the host, and `decorated_pvalues_device` for whole top-K lists whose splits are formed on the device from the gene
+rows already there (`synth.path_genes` maps a level's scores to genes and signs), non-stratified or stratified under the
+exec's permutation strata.  The Monte-Carlo mode is a host utility.  Only
 the number of redrawn carriers that fall among the cases matters, and that number is hypergeometric, so besides the
 reference's Monte-Carlo estimate (`n_permutations` redraws; R's `sample()` stream cannot be reproduced, a seeded numpy
 generator is used) the exact limit of that estimate is available (`n_permutations=None`): the tail probability is summed
@@ -174,6 +176,45 @@ def decorated_exact_device(ex, splits) -> list[DecoratedResult]:
     return [DecoratedResult(o.pvalue, o.cases1, o.ctrls1, o.cases2, o.ctrls2, o.score) for o in out]
 
 
+def _split_labels(L: int) -> list[dict]:
+    """direction / subpath1 / subpath2 of a path's splits (R/DecoratedPvalue.R:123-180): forward, then backward."""
+    labels = [{"direction": "Forward", "subpath1": list(range(j)), "subpath2": j} for j in range(1, L)]
+    labels += [{"direction": "Backward", "subpath1": list(range(L - 1, j - 1, -1)), "subpath2": j - 1} for j in range(L - 1, 0, -1)]
+    return labels
+
+
+def decorated_pvalues_device(ex, gene_set, genes, signs, lengths, stratified: bool = False) -> list[list[dict]]:
+    """Exact decorated p-values of many paths in one device call (gcre_exec_decorated_paths, csrc/decorated.cuh).
+
+    ex: a JoinExec holding the value table; gene_set: a PathSet of ``ex`` whose rows are the genes (data1);
+    genes / signs: int [k][<= 5] per path (gene rows in path order, +1 / -1 cumulative signs as :func:`synth.path_genes` gives);
+    lengths: int [k].  stratified: redraw inside the strata set by ``ex.setPermutationStrata`` (one stratum when none is set).
+    Returns per path what :func:`decorated_pvalues_for_path` returns for it (same labels, order and fields)."""
+    import ctypes as C
+
+    from . import _lib
+
+    lengths = np.ascontiguousarray(np.atleast_1d(lengths), dtype=np.int32)
+    k = lengths.shape[0]
+    g = np.zeros((k, 5), dtype=np.int32)
+    sg = np.zeros((k, 5), dtype=np.int32)
+    gin, sin = (np.asarray(v, dtype=np.int32).reshape(k, -1) if k else np.zeros((0, 5), np.int32) for v in (genes, signs))
+    if gin.shape[1] > 5 or sin.shape[1] > 5:
+        raise ValueError("paths have at most 5 genes")
+    g[:, :gin.shape[1]] = gin
+    sg[:, :sin.shape[1]] = sin
+    out = (_lib.DecoratedC * (8 * max(k, 1)))()
+    i32 = C.POINTER(C.c_int32)
+    _lib.check(ex._lib.gcre_exec_decorated_paths(ex._h, gene_set._h, g.ctypes.data_as(i32), sg.ctypes.data_as(i32), lengths.ctypes.data_as(i32),
+                                                 k, 1 if stratified else 0, out))
+    res = []
+    for i in range(k):
+        labels = _split_labels(int(lengths[i]))
+        res.append([{**lab, **DecoratedResult(o.pvalue, o.cases1, o.ctrls1, o.cases2, o.ctrls2, o.score).__dict__}
+                    for lab, o in zip(labels, out[8 * i:8 * i + len(labels)])])
+    return res
+
+
 def decorated_pvalues_for_path(gene_rows: np.ndarray, signs, n_cases: int, n_ctrls: int, method: int, value_table: np.ndarray,
                                n_permutations: int | None = None, rng: np.random.Generator | None = None, strata=None,
                                device_exec=None) -> list[dict]:
@@ -190,13 +231,9 @@ def decorated_pvalues_for_path(gene_rows: np.ndarray, signs, n_cases: int, n_ctr
     if method == 2:
         neg[signs == -1] = rows[signs == -1]
         pos[signs == -1] = False
-    splits, labels = [], []
-    for j in range(1, L):  # forward: genes 1..j, then gene j+1
-        splits.append((pos[:j].any(0), neg[:j].any(0), pos[j], neg[j]))
-        labels.append({"direction": "Forward", "subpath1": list(range(j)), "subpath2": j})
-    for j in range(L - 1, 0, -1):  # backward: genes L..j+1, then gene j
-        splits.append((pos[j:].any(0), neg[j:].any(0), pos[j - 1], neg[j - 1]))
-        labels.append({"direction": "Backward", "subpath1": list(range(L - 1, j - 1, -1)), "subpath2": j - 1})
+    splits = [(pos[:j].any(0), neg[:j].any(0), pos[j], neg[j]) for j in range(1, L)]  # forward: genes 1..j, then gene j+1
+    splits += [(pos[j:].any(0), neg[j:].any(0), pos[j - 1], neg[j - 1]) for j in range(L - 1, 0, -1)]  # backward: genes L..j+1, then gene j
+    labels = _split_labels(L)
     if device_exec is not None:  # all splits of the path in one kernel launch (exact mode, no strata)
         if n_permutations is not None or strata is not None:
             raise ValueError("the device path computes the exact, non-stratified limit")

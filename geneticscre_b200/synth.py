@@ -363,6 +363,49 @@ def _derive_levels(net: Network, max_path_length: int) -> None:
     net.levels["5"] = Level("5", 5, g1.copy(), g3.copy(), p3_from[g3].copy(), loc3[g3].copy(), third_sign.copy(), keep=False)
 
 
+def path_genes(net: Network, level: str, src, trg):
+    """Genes and cumulative signs of a level's top-K paths: the inverse of the row layouts `_derive_levels` sets up.
+
+    src / trg: the ``Score.src`` / ``Score.trg`` of a join of ``level`` ('1a', '1b', '2' .. '5').  Returns int32 ``genes[k][5]``
+    (rows of data1 in path order), ``signs[k][5]`` (cumulative products of the edge signs, +1 for the first gene) and
+    ``lengths[k]``; unused slots are 0.  A sentinel entry (src < 0) raises ValueError."""
+    src = np.atleast_1d(np.asarray(src, dtype=np.int64))
+    trg = np.atleast_1d(np.asarray(trg, dtype=np.int64))
+    if src.shape != trg.shape:
+        raise ValueError("src and trg must have the same length")
+    if (src < 0).any() or (trg < 0).any():
+        raise ValueError("a sentinel entry (src < 0) names no path")
+    k = src.shape[0]
+    es, et, s = net.edges_src, net.edges_trg, net.edges_sign
+    one = np.ones(k, dtype=np.int64)
+    if level == "1a":
+        cols = [src], [one]
+    elif level == "1b":
+        cols = [net.ents2[trg]], [one]
+    elif level == "2":
+        cols = [src, et[trg]], [one, s[trg]]
+    elif level == "3":
+        cols = [es[src], et[src], et[trg]], [one, s[src], s[src] * s[trg]]
+    elif level in ("4", "5"):
+        r = net.rels3
+        tp = r["sign"][src]
+        if level == "4":
+            cols = [r["g1"][src], r["g2"][src], r["g3"][src], et[trg]], [one, s[r["e_i"][src]], tp, tp * s[trg]]
+        else:
+            tq = r["sign"][trg]
+            cols = ([r["g1"][src], r["g2"][src], r["g3"][src], r["g2"][trg], r["g3"][trg]],
+                    [one, s[r["e_i"][src]], tp, tp * s[r["e_i"][trg]], tp * tq])
+    else:
+        raise ValueError(f"unknown level {level!r}")
+    genes = np.zeros((k, 5), dtype=np.int32)
+    signs = np.zeros((k, 5), dtype=np.int32)
+    L = len(cols[0])
+    for j in range(L):
+        genes[:, j] = cols[0][j]
+        signs[:, j] = cols[1][j]
+    return genes, signs, np.full(k, L, dtype=np.int32)
+
+
 @dataclass
 class Workload:
     """Everything one GWASPA run hands to the join path."""

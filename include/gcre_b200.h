@@ -120,6 +120,23 @@ int gcre_exec_get_info(const gcre_exec* ex, gcre_exec_info* out);
  * n_items splits at once against this exec's value table and method.  rows: uint64[n_items][4][ceil(n/64)] packed carrier
  * vectors pos1, neg1 (sub-path), pos2, neg2 (added gene), patient c -> word c/64 bit c%64, cases first. */
 int gcre_exec_decorated_exact(gcre_exec* ex, const uint64_t* rows, uint32_t n_items, gcre_decorated* out);
+/* Decorated p-values of n_paths whole paths whose genes are rows of `genes` (a path set of this exec; only the first, positive
+ * half of each row is read), every split formed on the device.  gene_idx / signs: int32[n_paths][5], lengths[i] in 1..5 (slots
+ * past a path's length are not read); signs +1 / -1 (method 2; ignored, and may be NULL, for method 1).
+ * out: gcre_decorated[n_paths][8]: path i's 2(L-1) splits in the order of decorated_pvalues_for_path (forward j = 1 .. L-1:
+ * genes 0 .. j-1 + gene j; then backward j = L-1 .. 1: genes L-1 .. j + gene j-1), the remaining slots zeroed.
+ * stratified = 0: exactly gcre_exec_decorated_exact on those splits.  stratified = 1: the exact limit of stratified resampling
+ * (the reference's strataF, R/DecoratedPvalue.R:236-268) under the strata set by gcre_exec_set_permutation_strata (none set: one
+ * stratum), so one setting serves the permutations and the decorated p-values.  Per stratum g, with free = ~(pos1 | neg1):
+ * c_g / d_g the free cases / controls, kp_g = |pos2 & ~pos1 & free & g|, kn_g = |neg2 & ~neg1 & free & g|,
+ *   joint_g[x][y] = Hyp(c_g, d_g, kp_g)(x) * Hyp(d_g - (kp_g - x), c_g - x, kn_g)(y),
+ * J = the 2-D convolution of the joint_g in dense-stratum order, p = sum J[cp][cn] * [score_of(cp, sum kp, cn, sum kn) >= score]
+ * (score and the counts as in the non-stratified mode).
+ * Errors: `genes` of another exec, a method-2 sign not +-1: GCRE_ERR_ARG; a gene index outside [0, size of genes) or a length
+ * outside 1..5: GCRE_ERR_RANGE; no value table: GCRE_ERR_ASSERT; a stratum with fewer free patients than carriers to redraw:
+ * GCRE_ERR_RANGE naming the path and split (R's sample() stops there).  n_paths = 0: GCRE_OK. */
+int gcre_exec_decorated_paths(gcre_exec* ex, const gcre_pathset* genes, const int32_t* gene_idx, const int32_t* signs,
+                              const int32_t* lengths, uint32_t n_paths, int stratified, gcre_decorated* out);
 /* Run this exec's work on a caller-owned CUDA stream (cudaStream_t passed as void*); NULL restores the internal one. */
 int gcre_exec_set_stream(gcre_exec* ex, void* cuda_stream);
 
